@@ -21,6 +21,9 @@ Own arm, three measurements in one run:
              bounded sample of the same workload (rank 0, N=1 only).
 
 Reference arm (`--impl reference`): the oracle on all host cores, bounded sample per step.
+
+`--dump-outputs DIR` writes what the last timed step of the device-resident arm computed (rank 0) as float64 .npy
+files, so that two builds run with the same arguments (hence the same seeded inputs) can be compared output for output.
 """
 from __future__ import annotations
 
@@ -35,6 +38,7 @@ import time
 import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree it runs from
 sys.path.insert(0, ROOT)
 
 M, N = 64, 4
@@ -57,6 +61,26 @@ def algorithmic_flops(stats, m=M, n=N):
 
 
 ALGO_BYTES_PER_FIT = M * 8 + N * 8 + N * 8 + 32      # samples + guess + solution + Result = 608 B (shared grid/bounds)
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(out_dir, x, results):
+    """Writes x.npy (batch x n parameters), one file per Result field and rows.npy (the row numbers written), all float64.
+    When every row does not fit in DUMP_BYTES, the rows are a fixed seeded sample, the same in every run of one batch size.
+    +-inf is written as the largest finite double of that sign: a fit that stops because lambda exceeded maxLambda
+    (furtherImprovement) returns lambda = +inf whenever the last increase overflowed, as the reference does, and every lambda
+    above maxLambda is the same state of the algorithm.  NaN is written as NaN."""
+    arrays = {"x": x, **{f: results[f] for f in results.dtype.names}}
+    row_bytes = 8 * (1 + sum(a[0].size for a in arrays.values()))
+    batch = len(x)
+    keep = min(batch, (DUMP_BYTES - 4096) // row_bytes)          # (4096: room for the .npy headers)
+    rows = np.arange(batch) if keep == batch else np.sort(np.random.default_rng(0).choice(batch, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "rows.npy"), rows.astype(np.float64))
+    big = np.finfo(np.float64).max
+    for name, a in arrays.items():
+        a = np.nan_to_num(np.asarray(a[rows], dtype=np.float64), nan=np.nan, posinf=big, neginf=-big)
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a))
 
 
 class ClockSampler:
@@ -380,7 +404,10 @@ def main():
     ap.add_argument("--ref-step-seconds", type=float, default=3.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the configs[2]/[3]/[4] measurements")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the parameters and Result fields of the last timed step to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 0)
 
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -458,6 +485,8 @@ def main():
                       "qp_iterations"), (int(v) for v in stats_d.cpu().tolist())))
     value = world * B * args.steps / (elapsed_ms * 1e-3)
     res_host = eng.results_from_bytes(res_d, np.float64)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, x_d.cpu().numpy(), res_host)
     assert np.all(res_host["status"] >= 0), "a fit failed"
 
     # ---------------- end-to-end arm: pinned host buffers through the host-pointer C ABI ----------------
