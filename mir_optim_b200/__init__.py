@@ -16,7 +16,7 @@ from ._abi import (BoxQPStatus, LeastSquaresStatus, ModelDesc, ModelId, BatchSta
                    MODEL_FD_JACOBIAN, MODEL_GRID_PER_PROBLEM)
 
 _HERE = _os.path.dirname(_os.path.abspath(__file__))
-LIB_PATH = _os.environ.get("MIR_B200_LIB") or _os.path.join(_HERE, "libmir_optim_b200.so")   # env override: kernel-variant experiments
+LIB_PATH = _os.environ.get("MIR_B200_LIB") or _os.path.join(_HERE, "libmir_optim_b200.so")   # env override: load the library from another path
 
 
 class LibraryMissing(ImportError):

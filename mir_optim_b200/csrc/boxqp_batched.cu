@@ -2,9 +2,6 @@
 // factor in shared memory, P read in place); 64 < n <= 128: one CTA per QP, P's lower triangle, the factor and all vectors in
 // shared memory.  Persistent warps / CTAs pull QP indices from an atomic counter.
 // C ABI: mir_solve_box_qp_{d,s}, mir_solve_box_qp_batched[_dev]_{d,s}  (solveBoxQP, boxcqp.d:85-102 / 122-379).
-#include <cstdlib>
-#include <cstring>
-
 #include "boxqp_cta.cuh"
 #include "boxqp_warp.cuh"
 #include "runtime.cuh"
@@ -16,7 +13,6 @@ template <class T> struct QPBatchArgs {
     int32_t* status; uint32_t* iterations;
     unsigned int* counter;
     unsigned int batch; int n;
-    int tma;                   // warp kernel: stage P's lower triangle into the factor buffer by TMA (unconstrained solve)
     typename Num<T>::QPSettings st;
 };
 
@@ -67,16 +63,12 @@ __global__ void __launch_bounds__(NT) boxqp_cta_kernel(const QPBatchArgs<T> a)
 }
 
 // One warp (= one CTA) per QP, n <= 64.
-template <class T, bool PAD>
+template <class T>
 __global__ void __launch_bounds__(32) boxqp_warp_kernel(const QPBatchArgs<T> a)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     WarpQPSmem<T>& sm = *reinterpret_cast<WarpQPSmem<T>*>(smem_raw);
     const int n = a.n, lane = threadIdx.x;
-    unsigned tmaParity = 0;
-    if (lane == 0) wqp_mbar_init(&sm.bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    __syncwarp();
     for (;;) {
         unsigned int prob = 0;
         if (lane == 0) prob = atomicAdd(a.counter, 1u);
@@ -90,7 +82,7 @@ __global__ void __launch_bounds__(32) boxqp_warp_kernel(const QPBatchArgs<T> a)
         }
         __syncwarp();
         unsigned iters = 0, solves = 0;
-        const int st = boxqp_warp<T, PAD>(a.st, n, Pg, sm, lane, iters, solves, PAD ? &tmaParity : nullptr);
+        const int st = boxqp_warp<T>(a.st, n, Pg, sm, lane, iters, solves);
         __syncwarp();
         for (int i = lane; i < n; i += 32) a.x[(size_t)prob * n + i] = sm.x[i];
         if (lane == 0) { a.status[prob] = st; if (a.iterations) a.iterations[prob] = iters; }
@@ -123,16 +115,11 @@ static int qp_batched_dev(const typename Num<T>::QPSettings* settings, size_t ba
     QPBatchArgs<T> a;
     a.P = P; a.q = q; a.l = l; a.u = u; a.x = x; a.status = status; a.iterations = iterations;
     a.batch = (unsigned)batch; a.n = (int)n; a.st = settings ? *settings : def;
-    // TMA staging of P into a 16-byte-aligned (padded) packed layout (boxqp_warp.cuh): measured on B200 at n = 64, 36.6 ms per
-    // 100,000 QPs against 34.6 ms for the dense layout filled by the element loop -- so it is opt-in (MIRB200_QP_TMA=1)
-    static const bool useTma = [] { const char* e = std::getenv("MIRB200_QP_TMA"); return e && *e == '1'; }();
-    a.tma = useTma ? 1 : 0;
     MIRB200_CUDA(cudaMallocAsync((void**)&a.counter, sizeof(unsigned int), stream));
     MIRB200_CUDA(cudaMemsetAsync(a.counter, 0, sizeof(unsigned int), stream));
 
-    static const bool ctaOnly = [] { const char* e = std::getenv("MIRB200_QP_KERNEL"); return e && !std::strcmp(e, "cta"); }();   // experiments / tests
-    if (n <= (size_t)WQP_NMAX && !ctaOnly) {
-        auto wk = (a.tma && sizeof(T) == 8) ? boxqp_warp_kernel<T, true> : boxqp_warp_kernel<T, false>;
+    if (n <= (size_t)WQP_NMAX) {
+        auto wk = boxqp_warp_kernel<T>;
         const size_t wsmem = sizeof(WarpQPSmem<T>);
         MIRB200_CUDA(cudaFuncSetAttribute(wk, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)wsmem));
         MIRB200_CUDA(cudaFuncSetAttribute(wk, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));

@@ -15,10 +15,7 @@
 //   * the triangular solves keep the right-hand side in registers (two entries per lane) and broadcast one solved entry per
 //     column with a shuffle;
 //   * P itself is never copied: only its lower triangle is read (boxcqp.d:288-302, 335), a lane's own row through L1
-//     (sequential), the rest of a symmetric row as column entries, which are coalesced across the lanes;
-//   * the unconstrained solve, which factors all of P, has its lower triangle staged straight into the factor buffer by
-//     TMA: one cp.async.bulk per row (rows of the packed layout are padded to 16-byte boundaries for that), completion
-//     on an mbarrier -- 64 asynchronous copies in flight instead of 2,080 dependent load / store pairs.
+//     (sequential), the rest of a symmetric row as column entries, which are coalesced across the lanes.
 #pragma once
 #include "boxqp_small.cuh"   // KBN
 #include "repro_math.cuh"
@@ -28,52 +25,17 @@ namespace mirb200 {
 constexpr int WQP_NMAX = 64;
 constexpr unsigned WQP_FULL = 0xffffffffu;
 
-// Packed lower triangle, row i begins at wtri<PAD>(i).  PAD = false: dense, i (i + 1) / 2.  PAD = true: every row padded to
-// an even number of entries, so that (in double) each row starts on a 16-byte boundary and can be the destination of a
-// TMA bulk copy.  Measured on B200 (100,000 QPs, n = 64, double): dense + element loop 34.6 ms; padded + element loop
-// 37.4 ms (the regular row starts collide in the banks more often); padded + TMA staging 36.6 ms.  Dense is the default.
-template <bool PAD> __host__ __device__ constexpr int wtri(int i)
-{
-    return PAD ? ((i & 1) ? 2 * ((i >> 1) + 1) * ((i >> 1) + 1) : 2 * (i >> 1) * ((i >> 1) + 1)) : i * (i + 1) / 2;
-}
+// Packed lower triangle, row i begins at wtri(i).
+__host__ __device__ constexpr int wtri(int i) { return i * (i + 1) / 2; }
 
 template <class T> struct WarpQPSmem {
-    T F[2 * (WQP_NMAX / 2) * (WQP_NMAX / 2 + 1)];   // packed lower factor of the current (sub-)system (sized for the padded layout)
-    unsigned long long bar;                // mbarrier of the TMA staging
+    T F[WQP_NMAX * (WQP_NMAX + 1) / 2];    // packed lower factor of the current (sub-)system
     T q[WQP_NMAX], l[WQP_NMAX], u[WQP_NMAX], x[WQP_NMAX];   // by variable
     T b[WQP_NMAX], sx[WQP_NMAX];           // right-hand side / solution of the current (sub-)system, by compact index
     T col[WQP_NMAX], rdiag[WQP_NMAX], sc[WQP_NMAX];
     int idx[WQP_NMAX];                     // compact index -> variable, ascending
     signed char flag[WQP_NMAX];            // -1 lower, 0 free, +1 upper (boxcqp.d:153-158)
 };
-
-// ---- TMA (cp.async.bulk) + mbarrier, as in syrk_dmma.cuh ---------------------------------------------------------------
-__device__ __forceinline__ unsigned wqp_smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void wqp_mbar_init(unsigned long long* bar, unsigned count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(wqp_smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void wqp_mbar_expect_tx(unsigned long long* bar, unsigned bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(wqp_smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void wqp_mbar_wait(unsigned long long* bar, unsigned parity)
-{
-    asm volatile(
-        "{\n"
-        ".reg .pred p;\n"
-        "WAIT_%=:\n"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n"
-        "@p bra DONE_%=;\n"
-        "bra WAIT_%=;\n"
-        "DONE_%=:\n"
-        "}\n" ::"r"(wqp_smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void wqp_tma_g2s(void* dst, const void* src, unsigned bytes, unsigned long long* bar)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(wqp_smem_u32(dst)), "l"(src), "r"(bytes), "r"(wqp_smem_u32(bar)) : "memory");
-}
 
 template <class T> __device__ __forceinline__ T warp_max(T v)
 {
@@ -90,12 +52,8 @@ template <class T> __device__ __forceinline__ T warp_min(T v)
 
 // A(a, c) for a >= c: the (unscaled) lower triangle of the s x s system.  b: sm.b (overwritten by its scaled copy),
 // solution in sm.sx.  Returns LAPACK info (0, or k > 0: breakdown at pivot k), uniform over the warp.
-// tmaSrc / tmaLd (optional, double only): the system IS the leading s x s block of the row-major matrix at tmaSrc with row
-// pitch tmaLd (even): its lower triangle is staged into the factor buffer by TMA bulk copies, one per row, instead of the
-// element loop; tmaParity is the phase bit of sm.bar (flipped here).
-template <class T, bool PAD, class AGet>
-__device__ int posvx_warp(int s, AGet A, WarpQPSmem<T>& sm, int lane, int* equed_out = nullptr,
-                          const T* tmaSrc = nullptr, int tmaLd = 0, unsigned* tmaParity = nullptr)
+template <class T, class AGet>
+__device__ int posvx_warp(int s, AGet A, WarpQPSmem<T>& sm, int lane, int* equed_out = nullptr)
 {
     const int nh = (s + 1) >> 1;
     const int r0 = lane, r1 = s - 1 - lane;
@@ -139,7 +97,7 @@ __device__ int posvx_warp(int s, AGet A, WarpQPSmem<T>& sm, int lane, int* equed
     // ---- the lower triangle of the (equilibrated) system, packed, and the scaled right-hand side
     // (four independent loads in flight per row: the loop is latency-bound on L1 / L2 otherwise)
     auto fill_row = [&](int r, T scr) {
-        T* Fr = sm.F + wtri<PAD>(r);
+        T* Fr = sm.F + wtri(r);
         int c = 0;
         for (; c + 3 <= r; c += 4) {
             const T a0 = A(r, c), a1 = A(r, c + 1), a2 = A(r, c + 2), a3 = A(r, c + 3);
@@ -148,46 +106,25 @@ __device__ int posvx_warp(int s, AGet A, WarpQPSmem<T>& sm, int lane, int* equed
         }
         for (; c <= r; ++c) Fr[c] = Asc(r, scr, c);
     };
-    bool staged = false;
-    if constexpr (sizeof(T) == 8 && PAD) {
-        if (tmaSrc != nullptr && (tmaLd & 1) == 0 && (reinterpret_cast<uintptr_t>(tmaSrc) & 15) == 0) {
-            staged = true;
-            // one bulk copy per row, rounded up to an even number of entries (the extra entry of an odd row lands in the
-            // row's padding slot and is never read); every lane issues its own two rows
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // earlier generic accesses to F before the async-proxy writes
-            __syncwarp();
-            if (lane == 0) wqp_mbar_expect_tx(&sm.bar, (unsigned)(wtri<PAD>(s) * sizeof(T)));
-            if (v0) wqp_tma_g2s(sm.F + wtri<PAD>(r0), tmaSrc + (size_t)r0 * tmaLd, (unsigned)(((r0 + 2) & ~1) * sizeof(T)), &sm.bar);
-            if (v1) wqp_tma_g2s(sm.F + wtri<PAD>(r1), tmaSrc + (size_t)r1 * tmaLd, (unsigned)(((r1 + 2) & ~1) * sizeof(T)), &sm.bar);
-            wqp_mbar_wait(&sm.bar, *tmaParity);
-            *tmaParity ^= 1u;
-            if (equil) {
-                if (v0) { T* Fr = sm.F + wtri<PAD>(r0); for (int c = 0; c <= r0; ++c) Fr[c] = (sm.sc[c] * sc0) * Fr[c]; }
-                if (v1) { T* Fr = sm.F + wtri<PAD>(r1); for (int c = 0; c <= r1; ++c) Fr[c] = (sm.sc[c] * sc1) * Fr[c]; }
-            }
-        }
-    }
-    if (!staged) {
-        if (v0) fill_row(r0, sc0);
-        if (v1) fill_row(r1, sc1);
-    }
+    if (v0) fill_row(r0, sc0);
+    if (v1) fill_row(r1, sc1);
     T b0 = v0 ? sm.b[r0] * sc0 : (T)0, b1 = v1 ? sm.b[r1] * sc1 : (T)0;         // dposvx: B := diag(S) B
     __syncwarp();
 
     // ---- ?potrf, right-looking.  The diagonal entry of L is kept as its reciprocal (rdiag), F keeps the pivot.
     for (int j = 0; j < s; ++j) {
-        const T d = sm.F[wtri<PAD>(j) + j];
+        const T d = sm.F[wtri(j) + j];
         if (d <= (T)0) return j + 1;           // breakdown (uniform; a NaN pivot passes, as in OpenBLAS' potf2)
         T ljj, rinv;
         mux_sqrt_rcp(d, ljj, rinv);
         T l0 = (T)0, l1 = (T)0;
-        if (v0 && r0 > j) { T* p = sm.F + wtri<PAD>(r0) + j; l0 = *p * rinv; *p = l0; sm.col[r0] = l0; }
-        if (v1 && r1 > j) { T* p = sm.F + wtri<PAD>(r1) + j; l1 = *p * rinv; *p = l1; sm.col[r1] = l1; }
+        if (v0 && r0 > j) { T* p = sm.F + wtri(r0) + j; l0 = *p * rinv; *p = l0; sm.col[r0] = l0; }
+        if (v1 && r1 > j) { T* p = sm.F + wtri(r1) + j; l1 = *p * rinv; *p = l1; sm.col[r1] = l1; }
         if (lane == 0) sm.rdiag[j] = rinv;
         __syncwarp();
         {
             // both rows of the lane in one sweep over k (r0 <= r1: the pivot-column entry is loaded once for the two)
-            T* F0 = sm.F + wtri<PAD>(r0); T* F1 = sm.F + wtri<PAD>(r1);
+            T* F0 = sm.F + wtri(r0); T* F1 = sm.F + wtri(r1);
             const int e0 = (v0 && r0 > j) ? r0 : j, e1 = (v1 && r1 > j) ? r1 : ((v0 && r0 > j) ? r0 : j);
             int k = j + 1;
             for (; k + 1 <= e0; k += 2) {
@@ -211,14 +148,14 @@ __device__ int posvx_warp(int s, AGet A, WarpQPSmem<T>& sm, int lane, int* equed
             const bool lowHalf = j < nh;
             const T zj = __shfl_sync(WQP_FULL, lowHalf ? z0 : z1, lowHalf ? j : s - 1 - j) * sm.rdiag[j];
             if (lowHalf) { if (lane == j) z0 = zj; } else { if (lane == s - 1 - j) z1 = zj; }
-            if (v0 && r0 > j) z0 = fma(-sm.F[wtri<PAD>(r0) + j], zj, z0);
-            if (v1 && r1 > j) z1 = fma(-sm.F[wtri<PAD>(r1) + j], zj, z1);
+            if (v0 && r0 > j) z0 = fma(-sm.F[wtri(r0) + j], zj, z0);
+            if (v1 && r1 > j) z1 = fma(-sm.F[wtri(r1) + j], zj, z1);
         }
         for (int j = s - 1; j >= 0; --j) {                             // backward, row j of L (= column j of L^T)
             const bool lowHalf = j < nh;
             const T xj = __shfl_sync(WQP_FULL, lowHalf ? z0 : z1, lowHalf ? j : s - 1 - j) * sm.rdiag[j];
             if (lowHalf) { if (lane == j) z0 = xj; } else { if (lane == s - 1 - j) z1 = xj; }
-            const T* Fj = sm.F + wtri<PAD>(j);
+            const T* Fj = sm.F + wtri(j);
             if (v0 && r0 < j) z0 = fma(-Fj[r0], xj, z0);
             if (v1 && r1 < j) z1 = fma(-Fj[r1], xj, z1);
         }
@@ -273,9 +210,9 @@ __device__ int posvx_warp(int s, AGet A, WarpQPSmem<T>& sm, int lane, int* equed
 
 // solveBoxQP for one QP by one warp.  P: n x n row-major in global memory (lower triangle read); sm.q / l / u hold the
 // problem vectors; the solution is left in sm.x.  Returns mir_box_qp_status (uniform).
-template <class T, bool PAD>
+template <class T>
 __device__ int boxqp_warp(const typename Num<T>::QPSettings& st, int n, const T* __restrict__ P, WarpQPSmem<T>& sm, int lane,
-                          unsigned& iterations, unsigned& solves, unsigned* tmaParity = nullptr)
+                          unsigned& iterations, unsigned& solves)
 {
     iterations = 0; solves = 0;
     if (n == 0) return mir_qp_solved;                                          // boxcqp.d:162-163
@@ -289,7 +226,7 @@ __device__ int boxqp_warp(const typename Num<T>::QPSettings& st, int n, const T*
     if (v1) sm.b[i1] = -sm.q[i1];
     __syncwarp();
     ++solves;
-    if (posvx_warp<T, PAD>(n, Pl, sm, lane, nullptr, tmaParity ? P : nullptr, n, tmaParity) != 0) return mir_qp_numericError;   // boxcqp.d:194-213
+    if (posvx_warp<T>(n, Pl, sm, lane) != 0) return mir_qp_numericError;   // boxcqp.d:194-213
     T x0 = v0 ? sm.sx[i0] : (T)0, x1 = v1 ? sm.sx[i1] : (T)0;
     const T l0 = v0 ? sm.l[i0] : (T)0, u0 = v0 ? sm.u[i0] : (T)0, l1 = v1 ? sm.l[i1] : (T)0, u1 = v1 ? sm.u[i1] : (T)0;
     const T q0 = v0 ? sm.q[i0] : (T)0, q1 = v1 ? sm.q[i1] : (T)0;
@@ -345,7 +282,7 @@ __device__ int boxqp_warp(const typename Num<T>::QPSettings& st, int n, const T*
             ++solves;
             const int* idx = sm.idx;
             auto Asub = [&](int a, int c) -> T { return Pl(idx[a], idx[c]); };   // idx ascending: a >= c => idx[a] >= idx[c]
-            if (posvx_warp<T, PAD>(s, Asub, sm, lane) != 0) return mir_qp_numericError;   // boxcqp.d:310-324
+            if (posvx_warp<T>(s, Asub, sm, lane) != 0) return mir_qp_numericError;   // boxcqp.d:310-324
             if (w0) sm.x[c0] = sm.sx[a0];                                      // boxcqp.d:327-329
             if (w1) sm.x[c1] = sm.sx[a1];
             __syncwarp();

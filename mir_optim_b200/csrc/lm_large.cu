@@ -212,9 +212,8 @@ static int large_solve(const typename Num<T>::Settings& st, unsigned model, unsi
     MIRB200_CUDA(cudaStreamWaitEvent(work.s, work.e, 0));
     stream = work.s;
 
-    // double: the Broyden update runs inside the SYRK ring (syrk_dmma.cuh); MIRB200_NO_BROYDEN_FUSE=1 keeps the separate kernel (experiments)
-    static const bool noFuse = [] { const char* e = std::getenv("MIRB200_NO_BROYDEN_FUSE"); return e && *e == '1'; }();
-    const bool fuseBroyden = kDouble && !noFuse;
+    // double: the Broyden update runs inside the SYRK ring (syrk_dmma.cuh); float keeps the separate kernel
+    const bool fuseBroyden = kDouble;
     static const bool trace = [] { const char* e = std::getenv("MIRB200_TRACE"); return e && *e == '1'; }();
     const auto tr0 = std::chrono::steady_clock::now();
     auto TR = [&](const char* what) { if (trace) { cudaStreamSynchronize(stream); fprintf(stderr, "[trace] %-28s %8.3f ms\n", what, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - tr0).count()); } };

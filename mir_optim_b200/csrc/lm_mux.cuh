@@ -49,7 +49,7 @@ constexpr unsigned MUX_FULL = 0xffffffffu;
 // as shared memory holds) step through the phases of the pass loop TOGETHER (a CTA barrier after every phase): they
 // share nothing but the instruction cache, which then holds one phase's code for all of them instead of thrashing
 // between five warps in five different phases.
-// (template parameters MUX_WARPS / TEAM0 of the kernel)
+// (template parameter MUX_WARPS of the kernel)
 enum { MUX_EVAL_INIT = 1, MUX_EVAL_TRIAL = 2, MUX_JAC_FRESH = 4, MUX_JAC_BROYDEN = 8 };
 
 // Everything a problem ("slot") keeps between phases, in shared memory of its CTA.
@@ -68,12 +68,12 @@ template <class T> struct MuxSlot {
 };
 struct MuxQueue {
     int qn[2], qhead[2];                // row-task queues of the two halves of the pass loop: length, next task
-    int retired;                        // warps of the team that have run out of problems (exit consensus)
+    int retired;                        // warps of the CTA that have run out of problems (exit consensus)
     unsigned char qtask[2][MUX_SLOTS * 16];
 };
 template <class T, int W> struct MuxCtaSmem {
     MuxSlot<T> slot[MUX_SLOTS * W];
-    MuxQueue team[2];                   // the CTA's warps form one or two teams, each stepping through the phases on its own
+    MuxQueue q;
 };
 
 // ---- group (8-lane) collectives, executed by the whole warp; every lane of a group receives the same bits -----------
@@ -335,11 +335,9 @@ __device__ __forceinline__ int boxqp_dist(bool act, int gl, int gshift, const ty
 template <class Model, class T, bool ON> struct SharedFD { struct State {}; static constexpr int CPI = 1; };
 template <class Model, class T> struct SharedFD<Model, T, true> { using State = typename Model::template FDState<MUX_R>; static constexpr int CPI = Model::CPI; };
 
-// MUX_WARPS warps per CTA, the first TEAM0 of them form team 0, the rest team 1 (TEAM0 == MUX_WARPS: one team).  A team
-// walks the phases of the pass loop together (named barrier over its own warps) and pools its row work; two teams on one
-// SM drift out of phase, so the latency-bound n-sized phase of one overlaps with the FP-heavy row phase of the other
-// (measured: float 2 x 5 warps 4.78 M fits/s against 4.50 M for 10 in step).
-template <class Model, class T, bool FD, int MUX_WARPS, int TEAM0 = MUX_WARPS>
+// MUX_WARPS warps per CTA walk the phases of the pass loop together (a CTA barrier after every phase) and pool their row
+// work in one queue.
+template <class Model, class T, bool FD, int MUX_WARPS>
 __global__ void __launch_bounds__(32 * MUX_WARPS)
 lm_mux_kernel(const typename Num<T>::Settings st, const SmallBatchArgs args)
 {
@@ -365,15 +363,11 @@ lm_mux_kernel(const typename Num<T>::Settings st, const SmallBatchArgs args)
     MuxSlot<T>& my = cta.slot[myslot];                                       // the slot of this lane's group
     for (int e = threadIdx.x; e < (int)(sizeof(Cta) / 4); e += 32 * MUX_WARPS) reinterpret_cast<unsigned*>(&cta)[e] = 0u;
     if constexpr (MUX_WARPS > 1) __syncthreads(); else __syncwarp();
-    // my team: its queue, its named barrier (id 1 / 2) over its own threads, the slots it serves
     const int warpId = threadIdx.x >> 5;
-    const int teamId = (warpId < TEAM0) ? 0 : 1;
-    const int teamWarps = teamId == 0 ? TEAM0 : MUX_WARPS - TEAM0;
-    MuxQueue& tq = cta.team[teamId];
-    auto team_sync = [&]() {
+    MuxQueue& tq = cta.q;
+    auto cta_sync = [&]() {
         if constexpr (MUX_WARPS == 1) __syncwarp();
-        else if constexpr (TEAM0 == MUX_WARPS) __syncthreads();
-        else asm volatile("bar.sync %0, %1;" ::"r"(teamId + 1), "r"(teamWarps * 32) : "memory");
+        else __syncthreads();
     };
 
     // ---- warp-role state: the shared abscissa of my rows (lane + 32 k)
@@ -654,13 +648,13 @@ lm_mux_kernel(const typename Num<T>::Settings st, const SmallBatchArgs args)
                 }
                 evalPending = (rf & (MUX_EVAL_INIT | MUX_EVAL_TRIAL)) != 0;
             }
-            // exit consensus of the team: every warp that has run out of problems is counted once
+            // exit consensus of the CTA: every warp that has run out of problems is counted once
             const bool warpRetired = __all_sync(MUX_FULL, retired);
             if (half == 0 && warpRetired && lane == 0 && !countedRetired) atomicAdd(&tq.retired, 1);
             if (half == 0 && warpRetired) countedRetired = true;
-            team_sync();
-            if (half == 0 && *(volatile int*)&tq.retired == teamWarps) goto done;
-            if (lane == 0 && (warpId == 0 || warpId == TEAM0)) { tq.qn[half ^ 1] = 0; tq.qhead[half ^ 1] = 0; }     // the other half's queue is idle now
+            cta_sync();
+            if (half == 0 && *(volatile int*)&tq.retired == MUX_WARPS) goto done;
+            if (lane == 0 && warpId == 0) { tq.qn[half ^ 1] = 0; tq.qhead[half ^ 1] = 0; }     // the other half's queue is idle now
             const int nTasks = tq.qn[half];
 #pragma unroll 1
             for (;;) {
@@ -830,7 +824,7 @@ lm_mux_kernel(const typename Num<T>::Settings st, const SmallBatchArgs args)
                 }
                 __syncwarp();
             }
-            team_sync();
+            cta_sync();
             if (evalPending) trial = my.result;
         }
     }

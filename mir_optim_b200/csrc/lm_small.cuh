@@ -79,10 +79,6 @@ template <class T> __device__ __forceinline__ T warm_lambda(const SmallBatchArgs
     return (v > (T)0 && v < Num<T>::inf()) ? v : (T)0;
 }
 
-#ifndef MIRB200_MINBLOCKS
-#define MIRB200_MINBLOCKS 1
-#endif
-
 // Lambda-overflow tail.  State: J is current (needJacobian == false), age == 0, the last pass was a rejection.
 // The step solves min 1/2 d'Pd + q'd over a box that contains d = 0, with P = J'J + lambda I >= lambda I and
 // q = J'r.  The minimiser has objective <= 0, hence lambda/2 |d|^2 <= -q'd <= |q| |d| and |d|_2 <= 2 |q|_2 / lambda.
@@ -165,7 +161,7 @@ __device__ __forceinline__ bool tail_is_inert(const T (&x)[N], const T (&Jy)[N],
 }
 
 template <class Model, class T, int LANES, int R, bool FD>
-__global__ void __launch_bounds__(128, MIRB200_MINBLOCKS)
+__global__ void __launch_bounds__(128, 1)
 lm_small_kernel(const typename Num<T>::Settings st, const SmallBatchArgs args)
 {
     constexpr int N = Model::N;

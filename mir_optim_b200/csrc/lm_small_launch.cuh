@@ -41,8 +41,7 @@ int launch_tpp_cfg(const typename Num<T>::Settings& st, const SmallBatchArgs& ar
     int blocksPerSM = 0;
     const size_t mPad = ((size_t)args.m + 1) & ~(size_t)1;
     // shared abscissa (+ observations) (+ the accepted steps of the v-list)
-    const size_t smem = sizeof(T) * (mPad + (YOS ? (size_t)args.m * TPP_THREADS : 0) + (VL ? (size_t)TPP_VLN * Model::N * TPP_THREADS : 0)
-                                     + ((VL && TPP_CPA) ? (size_t)TppPrefetch<Model>::ELEMS * TPP_THREADS : 0));
+    const size_t smem = sizeof(T) * (mPad + (YOS ? (size_t)args.m * TPP_THREADS : 0) + (VL ? (size_t)TPP_VLN * Model::N * TPP_THREADS : 0));
     if (smem > 200 * 1024) { set_error("mir_optim_b200: m too large for the thread-per-problem kernel"); return MIR_B200_EUNSUPPORTED; }
     if (smem > 48 * 1024) MIRB200_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     MIRB200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocksPerSM, kern, TPP_THREADS, smem));
@@ -50,7 +49,7 @@ int launch_tpp_cfg(const typename Num<T>::Settings& st, const SmallBatchArgs& ar
     unsigned long long blocksWanted = (args.batch + TPP_THREADS - 1) / TPP_THREADS;
     unsigned long long grid = (unsigned long long)sm_count() * blocksPerSM;
     if (blocksWanted < grid) grid = blocksWanted ? blocksWanted : 1;
-    const size_t perThread = (size_t)args.m * TppSlabOf<Model, YOS, VL>::ELEMS;
+    const size_t perThread = (size_t)args.m * TppSlab<Model::N, YOS, VL>::ELEMS;
     T* slab = nullptr;
     MIRB200_CUDA(cudaMallocAsync((void**)&slab, sizeof(T) * (perThread ? perThread : 1) * TPP_THREADS * grid, stream));
     kern<<<(unsigned)grid, TPP_THREADS, smem, stream>>>(st, args, slab);
@@ -63,12 +62,10 @@ template <class Model, class T, bool FD>
 int launch_tpp_fd(const typename Num<T>::Settings& st, const SmallBatchArgs& args, cudaStream_t stream)
 {
     // observations in shared memory while two CTAs per SM still fit (m * 128 threads * sizeof(T) <= ~100 KB)
-    static const bool noYOS = [] { const char* e = std::getenv("MIRB200_TPP_YOS"); return e && *e == '0'; }();      // experiments
-    const bool yos = Model::kHasData && !noYOS && sizeof(T) * ((size_t)args.m + TPP_VLN * Model::N) * TPP_THREADS <= 100 * 1024;
+    const bool yos = Model::kHasData && sizeof(T) * ((size_t)args.m + TPP_VLN * Model::N) * TPP_THREADS <= 100 * 1024;
     if constexpr (!FD) {
         // analytic Jacobian with the default maxAge (3, LS:945) or a smaller one: the v-list scheme (no stored Jacobian)
-        static const bool noVL = [] { const char* e = std::getenv("MIRB200_TPP_STORED_J"); return e && *e == '1'; }();
-        if ((st.maxAge ? st.maxAge : 3u) <= (unsigned)TPP_VLN && !noVL)
+        if ((st.maxAge ? st.maxAge : 3u) <= (unsigned)TPP_VLN)
             return yos ? launch_tpp_cfg<Model, T, FD, true, true>(st, args, stream) : launch_tpp_cfg<Model, T, FD, false, true>(st, args, stream);
     }
     return yos ? launch_tpp_cfg<Model, T, FD, true, false>(st, args, stream) : launch_tpp_cfg<Model, T, FD, false, false>(st, args, stream);
@@ -80,10 +77,10 @@ int launch_tpp(const typename Num<T>::Settings& st, const SmallBatchArgs& args, 
 }
 
 // Four problems per warp (lm_mux.cuh): n <= 8, m <= 128.  One warp per CTA; the warp's four problems live in its shared memory.
-template <class Model, class T, bool FD, int MUX_WARPS, int TEAM0 = MUX_WARPS>
+template <class Model, class T, bool FD, int MUX_WARPS>
 int launch_mux_w(const typename Num<T>::Settings& st, const SmallBatchArgs& args, cudaStream_t stream)
 {
-    auto kern = lm_mux_kernel<Model, T, FD, MUX_WARPS, TEAM0>;
+    auto kern = lm_mux_kernel<Model, T, FD, MUX_WARPS>;
     const size_t smem = sizeof(MuxCtaSmem<T, MUX_WARPS>);
     static bool attrSet = false;       // (per instantiation)
     if (!attrSet) {
@@ -103,24 +100,18 @@ int launch_mux_w(const typename Num<T>::Settings& st, const SmallBatchArgs& args
     return check_cuda(cudaGetLastError(), "lm_mux_kernel launch");
 }
 // Warps per CTA: as many as the shared memory of one SM holds (5 in double, 10 in float), stepping through the phases
-// together (lm_mux.cuh); MIRB200_MUX_LOCKSTEP=0 launches free-running single-warp CTAs instead (experiments).
+// together (lm_mux.cuh); batches too small to fill those CTAs run in single-warp CTAs.
 template <class Model, class T, bool FD>
 int launch_mux_fd(const typename Num<T>::Settings& st, const SmallBatchArgs& args, cudaStream_t stream)
 {
-    static const bool lockstep = [] { const char* e = std::getenv("MIRB200_MUX_LOCKSTEP"); return !(e && *e == '0'); }();
-    static const int wEnv = [] { const char* e = std::getenv("MIRB200_MUX_W"); return e ? std::atoi(e) : 0; }();      // experiments: warps per CTA
     constexpr int W = sizeof(T) == 8 ? 5 : 10;          // as many warps as the shared memory of one SM holds, in ONE CTA
     constexpr int WH = sizeof(T) == 8 ? 2 : 5;          // two CTAs per SM (they drift out of phase: one in the n-sized phase, one on rows)
-    if (lockstep && args.batch >= (unsigned long long)MUX_SLOTS * W * 2) {
+    if (args.batch >= (unsigned long long)MUX_SLOTS * W * 2) {
         // float: two CTAs of 5 warps per SM measured 4.78 M fits/s against 4.50 M for one CTA of 10 (the two drift out of
         // phase and overlap the latency-bound n-sized phase of one with the FP-heavy row phase of the other); double has 5
         // warps per SM, which do not split: 2 x 2 warps measured 0.99 M against 1.10 M for one CTA of 5
-        const bool split = wEnv ? (wEnv == WH) : (sizeof(T) == 4);
-        if (split) return launch_mux_w<Model, T, FD, WH>(st, args, stream);
-        // double: one CTA of 5 warps in one team.  Two teams of 3 and 2 warps in the CTA (MIRB200_MUX_W=3; named barriers per team)
-        // measured 1.18 M against 1.21 M fits/s back to back: no gain, the teams' queues are too short to balance
-        if (sizeof(T) == 8 && wEnv == 3) return launch_mux_w<Model, T, FD, W, 3>(st, args, stream);
-        return launch_mux_w<Model, T, FD, W>(st, args, stream);
+        if constexpr (sizeof(T) == 4) return launch_mux_w<Model, T, FD, WH>(st, args, stream);
+        else return launch_mux_w<Model, T, FD, W>(st, args, stream);
     }
     return launch_mux_w<Model, T, FD, 1>(st, args, stream);
 }
@@ -131,11 +122,9 @@ int launch_mux(const typename Num<T>::Settings& st, const SmallBatchArgs& args, 
 }
 
 // Kernel choice: one thread per problem once the batch can fill the GPU with threads, else one lane group per
-// problem (more parallelism inside each problem).  MIRB200_BATCH_KERNEL=group|thread overrides (experiments).
+// problem (more parallelism inside each problem).
 inline bool use_thread_per_problem(unsigned long long batch)
 {
-    static const int forced = [] { const char* e = std::getenv("MIRB200_BATCH_KERNEL"); return !e ? 0 : (!std::strcmp(e, "thread") ? 1 : (!std::strcmp(e, "group") ? 2 : 0)); }();
-    if (forced) return forced == 1;
     return batch >= 16384ull;
 }
 

@@ -43,74 +43,14 @@
 
 namespace mirb200 {
 
-#ifndef MIRB200_TPP_THREADS
-#define MIRB200_TPP_THREADS 128
-#endif
-constexpr int TPP_THREADS = MIRB200_TPP_THREADS;
+constexpr int TPP_THREADS = 128;
 enum { JAC_NONE_ = 0, JAC_BROYDEN_ = 1, JAC_FRESH_ = 2 };
 enum { ROW_NONE_ = 0, ROW_EVAL_ = 1, ROW_INSTALL_ = 2 };
-
-// Experimental (off): warp-cooperative, coalesced refill of the observations through an out-of-line helper.  The inline
-// form was parity-green on B200 but 20 % slower (it disturbed the register allocation of the row loop); see DESIGN 7.
-#ifndef MIRB200_TPP_COOP_REFILL
-#define MIRB200_TPP_COOP_REFILL 0
-#endif
-#ifndef MIRB200_TPP_MINBLOCKS
-#define MIRB200_TPP_MINBLOCKS 1
-#endif
-// v-list scheme: keep the exps of every row at the anchor point in the slab (written by the row pass that builds a fresh
-// Jacobian, whose trial-point exps ARE the anchor's once it is installed) instead of re-evaluating them in every Broyden
-// row pass.  Same values, hence the same bits; one exp per row instead of two, one more slab vector per exp.
-#ifndef MIRB200_TPP_ANCHOR_EXP
-#define MIRB200_TPP_ANCHOR_EXP 0
-#endif
-constexpr bool TPP_AE = MIRB200_TPP_ANCHOR_EXP != 0;
-// v-list scheme: the slab values of the next MIRB200_TPP_CPASYNC pairs of rows travel to shared memory with cp.async
-// (depth + 1 slots per thread) instead of sitting in prefetch registers while the current pair is computed.
-#ifndef MIRB200_TPP_CPASYNC
-#define MIRB200_TPP_CPASYNC 0
-#endif
-constexpr bool TPP_CPA = MIRB200_TPP_CPASYNC != 0;
-// v-list scheme: slab loads bypass the L1 (ld.global.cg) so that it keeps the bounds, settings and spill lines
-#ifndef MIRB200_TPP_SLAB_CG
-#define MIRB200_TPP_SLAB_CG 0
-#endif
-template <class T> __device__ __forceinline__ T tpp_slab_ld(const T* p) { if constexpr (MIRB200_TPP_SLAB_CG != 0) return __ldcg(p); else return *p; }
-// fields per row of the cp.async prefetch: f_old, v_0, v_1 (+ the anchor exps)
-constexpr int TPP_CPA_DEPTH = MIRB200_TPP_CPASYNC;
-template <class Model> struct TppPrefetch { static constexpr int F = 3 + (TPP_AE ? Model::NE : 0); static constexpr int ELEMS = (TPP_CPA_DEPTH + 1) * 2 * F; };
-template <class T> __device__ __forceinline__ void tpp_cp_async(T* smemDst, const T* gsrc)
-{
-    const unsigned d = (unsigned)__cvta_generic_to_shared(smemDst);
-    if constexpr (sizeof(T) == 8) asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"(d), "l"(gsrc) : "memory");
-    else asm volatile("cp.async.ca.shared.global [%0], [%1], 4;" ::"r"(d), "l"(gsrc) : "memory");
-}
-
 
 // number of slab vectors of length m per thread besides the m x N Jacobian
 // (stored-J scheme: [yobs] buf0 buf1 v + m x N Jacobian;  v-list scheme: [yobs] buf0 buf1 v0 v1 v2, no Jacobian)
 constexpr int TPP_VLN = 3;          // Broyden terms the v-list scheme can hold = largest maxAge it serves
 template <int N, bool YOS, bool VL> struct TppSlab { static constexpr int ELEMS = (YOS ? 2 : 3) + (VL ? TPP_VLN : 1 + N); };
-// slab vectors per thread of a model: the above + (v-list, anchor-exp cache) one vector per exp of a row
-template <class Model, bool YOS, bool VL> struct TppSlabOf { static constexpr int ELEMS = TppSlab<Model::N, YOS, VL>::ELEMS + ((VL && TPP_AE) ? Model::NE : 0); };
-
-#if MIRB200_TPP_COOP_REFILL
-// Every lane whose bit is set in `need` started problem `prob` (its own value) in this pass: the whole warp copies that
-// problem's m samples (coalesced reads) into the lane's column `col0 + lane'` ([row][thread] layout, pitch NT).
-template <class T>
-__device__ __noinline__ void tpp_refill_observations(unsigned need, unsigned long long prob, const T* yptr, int m, T* col0, int lane)
-{
-    while (need) {
-        const int src = __ffs(need) - 1;
-        need &= need - 1;
-        const unsigned long long p = __shfl_sync(0xffffffffu, prob, src);
-        const T* yp = yptr + p * (unsigned long long)m;
-        T* const col = col0 + src;
-        for (int row = lane; row < m; row += 32) col[row * TPP_THREADS] = yp[row];
-    }
-    __syncwarp();
-}
-#endif
 
 // YOS: the observations of the thread's current problem live in shared memory ([row][thread], conflict-free)
 // instead of the slab -- they are read by every model evaluation, the most frequent phase.
@@ -122,7 +62,7 @@ __device__ __noinline__ void tpp_refill_observations(unsigned need, unsigned lon
 // a 3x smaller memory stream (ncu, round 1: the stored-J row loop moved 233 KB per fit and ran at 44 % of HBM
 // bandwidth with 12 % occupancy) and a slab that fits the L2.
 template <class Model, class T, bool FD, bool YOS, bool VL>
-__global__ void __launch_bounds__(TPP_THREADS, MIRB200_TPP_MINBLOCKS)
+__global__ void __launch_bounds__(TPP_THREADS, 1)
 lm_tpp_kernel(const typename Num<T>::Settings st, const SmallBatchArgs args, T* __restrict__ slabBase)
 {
     constexpr int N = Model::N;
@@ -142,17 +82,15 @@ lm_tpp_kernel(const typename Num<T>::Settings st, const SmallBatchArgs args, T* 
 
     static_assert(!(VL && FD), "the v-list scheme needs an analytic Jacobian");
     // slab of this CTA: [yobs m (only !YOS)][buf0 m][buf1 m][v m (x TPP_VLN if VL)][J m*N (not VL)], each element strided by NT
-    T* const slab = slabBase + (size_t)blockIdx.x * ((size_t)m * TppSlabOf<Model, YOS, VL>::ELEMS) * NT + tid;
+    T* const slab = slabBase + (size_t)blockIdx.x * ((size_t)m * TppSlab<N, YOS, VL>::ELEMS) * NT + tid;
     const int mPad = (m + 1) & ~1;
     T* const pYO = YOS ? st_ + mPad + tid : slab;
     T* const pB0 = slab + (size_t)(YOS ? 0 : 1) * m * NT;
     T* const pB1 = pB0 + (size_t)m * NT;
     T* const pV = pB1 + (size_t)m * NT;
     T* const pJ = pV + (size_t)m * NT;                                         // (stored-J scheme only)
-    T* const pE = pV + (size_t)TPP_VLN * m * NT;                               // (v-list with the anchor-exp cache only) [exp][row]
     // accepted steps d_k of the v-list, [k][i][thread] in shared memory
     T* const pDL = st_ + mPad + (YOS ? (size_t)m * NT : 0) + tid;
-    T* const pPF = pDL + (size_t)TPP_VLN * N * NT;                              // (cp.async prefetch only) [slot][row of the pair][field][thread]
     auto DL = [&](int k, int i) -> T& { return pDL[(k * N + i) * NT]; };
     auto YO = [&](int row) -> T& { return pYO[row * NT]; };
     auto JE = [&](int row, int i) -> T& { return pJ[(row * N + i) * NT]; };
@@ -189,9 +127,6 @@ lm_tpp_kernel(const typename Num<T>::Settings st, const SmallBatchArgs args, T* 
 
     for (;;) {
         // ------------------------------------------------------------------ fetch
-#if MIRB200_TPP_COOP_REFILL
-        bool started = false;
-#endif
         if (!active && !retired) {
             const unsigned int idx = atomicAdd(args.counter, 1u);
             if (idx >= args.batch) retired = true;
@@ -230,15 +165,11 @@ lm_tpp_kernel(const typename Num<T>::Settings st, const SmallBatchArgs args, T* 
                 } else {
                     active = true; init = true; resume = false; specOK = false; pend = false; nterm = 0; specKind = JAC_NONE_;
                     tp = gridPerProblem ? tptr + prob * (unsigned long long)m : st_;
-#if MIRB200_TPP_COOP_REFILL
-                    started = true;
-#else
                     if (Model::kHasData) {
                         const T* yp = yptr + prob * (unsigned long long)m;
 #pragma unroll 8
                         for (int row = 0; row < m; ++row) YO(row) = yp[row];
                     }
-#endif
 #pragma unroll
                     for (int i = 0; i < N; ++i) { xt[i] = x[i]; Jy[i] = (T)0; dX[i] = (T)0; }
                     maxAge = st.maxAge ? st.maxAge : (FD ? 2u * N : 3u);                             // LS:945
@@ -248,12 +179,6 @@ lm_tpp_kernel(const typename Num<T>::Settings st, const SmallBatchArgs args, T* 
                 }
             }
         }
-#if MIRB200_TPP_COOP_REFILL
-        if (Model::kHasData) {
-            const unsigned need = __ballot_sync(0xffffffffu, started);
-            if (need) tpp_refill_observations<T>(need, prob, yptr, m, pYO - (tid & 31), tid & 31);
-        }
-#endif
         if (__all_sync(0xffffffffu, retired)) break;
 
         // ------------------------------------------------------------------ guards of this pass, LS:974-995, and the Jacobian decision, LS:996-1015
@@ -456,16 +381,11 @@ lm_tpp_kernel(const typename Num<T>::Settings st, const SmallBatchArgs args, T* 
                 const typename Model::Pre preA = Model::prepare(anchor);
                 // slab values are loaded a pair of rows ahead (global-memory latency); abscissa and observation come from
                 // shared memory at compute time
-                constexpr int NEA = (TPP_AE && NE > 0) ? NE : 1;
-                struct RowIn { T fo, v0, v1; T ea[NEA]; };
+                struct RowIn { T fo, v0, v1; };
                 auto rowLoad = [&](int row, RowIn& in, bool on) {
-                    if constexpr (TPP_AE) {
-#pragma unroll
-                        for (int q = 0; q < NE; ++q) in.ea[q] = (kB && on) ? pE[((size_t)q * m + row) * NT] : (T)0;
-                    }
-                    in.fo = (kB && on) ? tpp_slab_ld(fold + row * NT) : (T)0;
-                    in.v0 = (kB && k > 0 && on) ? tpp_slab_ld(pV + row * NT) : (T)0;
-                    in.v1 = (kB && k > 1 && on) ? tpp_slab_ld(pV + (size_t)m * NT + row * NT) : (T)0;
+                    in.fo = (kB && on) ? fold[row * NT] : (T)0;
+                    in.v0 = (kB && k > 0 && on) ? pV[row * NT] : (T)0;
+                    in.v1 = (kB && k > 1 && on) ? *(pV + (size_t)m * NT + row * NT) : (T)0;
                 };
                 // Branch-free: every lane runs the Broyden arithmetic (selects pick the result, loads and stores are
                 // predicated).  eT / eA: the exps of this row at the trial point and at the anchor.
@@ -490,12 +410,6 @@ lm_tpp_kernel(const typename Num<T>::Settings st, const SmallBatchArgs args, T* 
 #pragma unroll
                     for (int i = 0; i < N; ++i) Jn[i] = kB ? fma(v, dX[i], Jr[i]) : Jf[i];
                     if (kB && on) pVk[row * NT] = v;
-                    if constexpr (TPP_AE) {
-                        if (kF && on) {                          // if this Jacobian is installed, xt is the next anchor
-#pragma unroll
-                            for (int q = 0; q < NE; ++q) pE[((size_t)q * m + row) * NT] = eT[q];
-                        }
-                    }
                     if (isEval && on) out[row * NT] = r;
                     if (on) {
                         acc2 = fma(r, r, acc2);
@@ -512,80 +426,23 @@ lm_tpp_kernel(const typename Num<T>::Settings st, const SmallBatchArgs args, T* 
                     const int rowB = two ? row + 1 : row;
                     const T ta = Model::kHasData ? tp[row] : (T)0, ya = Model::kHasData ? YO(row) : (T)0;
                     const T tb = Model::kHasData ? tp[rowB] : (T)0, yb = Model::kHasData ? YO(rowB) : (T)0;
-                    if constexpr (TPP_AE) {
-                        T ea[2 * NE + 1], ee[2 * NE + 1];
-                        Model::exp_args(pre, xt, ta, ea); Model::exp_args(pre, xt, tb, ea + NE);
-                        exp_repro_many<2 * NE>(ea, ee);
-                        rowFinish(row, A, ta, ya, ee, A.ea, true);
-                        rowFinish(row + 1, B, tb, yb, ee + NE, B.ea, two);
-                        return;
-                    }
                     T ea[4 * NE], ee[4 * NE];
                     Model::exp_args(pre, xt, ta, ea); Model::exp_args(pre, xt, tb, ea + NE);
                     Model::exp_args(preA, anchor, ta, ea + 2 * NE); Model::exp_args(preA, anchor, tb, ea + 3 * NE);
-#ifdef MIRB200_TPP_EXP_CONV
-                    exp_repro_many_conv<4 * NE>(ea, ee, __activemask());
-#else
                     exp_repro_many<4 * NE>(ea, ee);
-#endif
                     rowFinish(row, A, ta, ya, ee, ee + 2 * NE, true);
                     rowFinish(row + 1, B, tb, yb, ee + NE, ee + 3 * NE, two);
                 };
                 int row = 0;
                 RowIn ra, rb;
-                if constexpr (TPP_CPA) {
-                    constexpr int F = TppPrefetch<Model>::F;
-                    // issue: the fields a Broyden row needs, into slot `slot`, half `h` (0 / 1 = first / second row of the pair)
-                    auto issue = [&](int r, int slot, int h) {
-                        T* const dst = pPF + (size_t)((slot * 2 + h) * F) * NT;
-                        if (kB) {
-                            tpp_cp_async(dst, fold + (size_t)r * NT);
-                            if (k > 0) tpp_cp_async(dst + NT, pV + (size_t)r * NT);
-                            if (k > 1) tpp_cp_async(dst + 2 * NT, pV + (size_t)m * NT + (size_t)r * NT);
-                            if constexpr (TPP_AE) {
-#pragma unroll
-                                for (int q = 0; q < NE; ++q) tpp_cp_async(dst + (3 + q) * NT, pE + ((size_t)q * m + r) * NT);
-                            }
-                        }
-                    };
-                    auto take = [&](RowIn& in, int slot, int h) {
-                        const T* const src = pPF + (size_t)((slot * 2 + h) * F) * NT;
-                        in.fo = kB ? src[0] : (T)0;
-                        in.v0 = (kB && k > 0) ? src[NT] : (T)0;
-                        in.v1 = (kB && k > 1) ? src[2 * NT] : (T)0;
-                        if constexpr (TPP_AE) {
-#pragma unroll
-                            for (int q = 0; q < NE; ++q) in.ea[q] = kB ? src[(3 + q) * NT] : (T)0;
-                        }
-                    };
-                    constexpr int D = TPP_CPA_DEPTH, S = D + 1;
-                    int slot = 0, ahead = D % S;            // slot of the pair being computed / of the pair being fetched
-#pragma unroll
-                    for (int d = 0; d < D; ++d) {
-                        if (2 * d + 2 <= m) { issue(2 * d, d, 0); issue(2 * d + 1, d, 1); }
-                        asm volatile("cp.async.commit_group;" ::: "memory");
-                    }
+                rowLoad(0, ra, m >= 2); rowLoad(1, rb, m >= 2);
 #pragma unroll 1
-                    for (; row + 2 <= m; row += 2) {
-                        if (row + 2 * D + 2 <= m) { issue(row + 2 * D, ahead, 0); issue(row + 2 * D + 1, ahead, 1); }
-                        asm volatile("cp.async.commit_group;" ::: "memory");
-                        asm volatile("cp.async.wait_group %0;" ::"n"(D) : "memory");
-                        take(ra, slot, 0); take(rb, slot, 1);
-                        pairCompute(row, ra, rb, true);
-                        slot = (slot + 1 == S) ? 0 : slot + 1;
-                        ahead = (ahead + 1 == S) ? 0 : ahead + 1;
-                    }
-                    asm volatile("cp.async.wait_group 0;" ::: "memory");
-                } else {
-                    rowLoad(0, ra, m >= 2); rowLoad(1, rb, m >= 2);
-#pragma unroll 1
-                    for (; row + 2 <= m; row += 2) {
-                        RowIn na, nb;
-                        const bool more = row + 4 <= m;
-                        rowLoad(row + 2, na, more); rowLoad(row + 3, nb, more);
-                        pairCompute(row, ra, rb, true);
-                        ra = na; rb = nb;
-                    }
+                for (; row + 2 <= m; row += 2) {
+                    RowIn na, nb;
+                    const bool more = row + 4 <= m;
+                    rowLoad(row + 2, na, more); rowLoad(row + 3, nb, more);
+                    pairCompute(row, ra, rb, true);
+                    ra = na; rb = nb;
                 }
                 if (row < m) { rowLoad(row, ra, true); pairCompute(row, ra, ra, false); }
             } else {
@@ -644,11 +501,7 @@ lm_tpp_kernel(const typename Num<T>::Settings st, const SmallBatchArgs args, T* 
                     const T tb = Model::kHasData ? tp[rowB] : (T)0, yb = Model::kHasData ? YO(rowB) : (T)0;
                     T ea[2 * NE], ee[2 * NE];
                     Model::exp_args(pre, xt, ta, ea); Model::exp_args(pre, xt, tb, ea + NE);
-#ifdef MIRB200_TPP_EXP_CONV
-                    exp_repro_many_conv<2 * NE>(ea, ee, __activemask());
-#else
                     exp_repro_many<2 * NE>(ea, ee);
-#endif
                     rowFinish(row, A, ta, ya, ee, true);
                     rowFinish(row + 1, B, tb, yb, ee + NE, two);
                 };

@@ -77,7 +77,7 @@ __global__ void __launch_bounds__(32) posvx_warp_kernel(const PosvxArgs<T> a)
         if (lane == 0) s_eq = 0;
         __syncwarp();
         auto A = [&](int i, int j) -> T { return Ag[(size_t)i * n + j]; };
-        const int info = posvx_warp<T, false>(n, A, sm, lane, &s_eq);
+        const int info = posvx_warp<T>(n, A, sm, lane, &s_eq);
         __syncwarp();
         for (int i = lane; i < n; i += 32) a.x[(size_t)p * n + i] = info ? (T)0 : sm.sx[i];
         if (lane == 0) { a.info[p] = info; a.equed[p] = s_eq; }

@@ -65,11 +65,11 @@ def test_tma_fed_kernels_contain_bulk_copies_and_mbarriers():
     assert ops.get("UBLKCP", 0) > 0 and ops.get("SYNCS", 0) > 0, ops
 
 
-def test_headline_kernel_experiments_are_off_by_default():
-    # the structural variants of DESIGN.md section 7 measured slower: the shipped kernel carries neither cp.async
-    # prefetch (LDGSTS) nor cache-global slab loads
+def test_headline_kernel_loads_slab_into_registers_and_evaluates_both_exp_pairs():
+    # DESIGN.md section 7: the row loop of the thread-per-problem kernel keeps its slab prefetch in registers (no cp.async,
+    # LDGSTS) and evaluates the exps of a row pair at the trial point and at the anchor
     names, _ = kernel_names()
     tpp = next(m for m, d in names.items() if "lm_tpp_kernel<mirb200::ModelGauss4<double, true>, double, false, true, true>" in d)
     ops = opcode_counts(tpp)
     assert ops.get("LDGSTS", 0) == 0, ops
-    assert ops.get("DFMA", 0) > 300, ops          # two interleaved exp pairs per row pair (anchor-exp cache off)
+    assert ops.get("DFMA", 0) > 300, ops          # two interleaved exp pairs per row pair
