@@ -346,6 +346,60 @@ int mir_optimize_least_squares_batched_dev_s(
     mir_least_squares_result_s* results, mir_batch_stats* stats, void* cuda_stream);
 
 /*
+ * Batched parameter covariance and standard errors at a given point (normally the x of a fit).  The reference has no
+ * covariance; this is an extension.  For one problem, with x the given parameters, r = f(x) (m rows) and J = dr/dx at x:
+ *
+ *   Free set   F = { i : l_i < x_i < u_i }.  A parameter exactly on a bound is fixed (the fit clamps its trial point with
+ *              max(min(., u), l), LS:1108-1110, so an active bound holds exactly).  n_F = |F|.
+ *   Jacobian   the model's analytic Jacobian, or the reference's central difference when MIR_MODEL_FD_JACOBIAN is set or
+ *              the model has none: settings->jacobianEpsilon and the bound clamp of LS:1030-1047, so a free parameter
+ *              within h of a bound gets the same one-sided difference the fit used.
+ *   Normal     A = J_F^T J_F and ||r||^2, accumulated in double also for float problems (float times float is exact in
+ *   matrix     double).
+ *   Inverse    S = D^-1/2 A D^-1/2 with D = diag(A); the Cholesky factor of S is inverted (LAPACK ?potrf + ?potri
+ *              semantics) and unscaled.  A zero diagonal entry of A, or a pivot <= 0 or NaN, stops the factorisation.
+ *   Scale      s^2 = ||r||^2 / (m - n_F); with MIR_COV_UNSCALED (residuals already divided by sigma; scipy's
+ *              absolute_sigma=True) s^2 = 1.
+ *   Outputs    cov = s^2 A^-1 on F x F; rows and columns of fixed parameters are exactly 0.  Both triangles are written
+ *              and are exactly symmetric (the lower triangle is computed and mirrored).  stddev_i = sqrt(cov_ii).
+ *              Everything is computed in double and rounded once to T.
+ *   info[b]    0   OK, including n_F = 0 (cov all zeros)
+ *              k>0 the factorisation broke down at the pivot of parameter k-1 (1-based, original numbering); free block NaN
+ *              -1  m <= n_F and scaled; free block +inf, as in scipy
+ *              -2  a residual, a Jacobian entry or an x_i is not finite; free block NaN
+ *              (checked in the order -2, -1, k).
+ *
+ * Model data as in the batched LM entries: t shared or MIR_MODEL_GRID_PER_PROBLEM, y, aux shared or
+ * MIR_MODEL_AUX_PER_PROBLEM, param, l / u shared (bound_stride == 0) or T[batch*bound_stride], MIR_MODEL_FD_JACOBIAN;
+ * MIR_MODEL_WARM_START and MIR_MODEL_NO_TAIL_SHORTCUT are ignored.  settings may be NULL (defaults); only
+ * jacobianEpsilon is read.  User models (mir_b200_model_compile) are compiled for the covariance at their first
+ * covariance call per precision.
+ *   x        T[batch*n]
+ *   cov      T[batch*n*n] or NULL;  stddev  T[batch*n] or NULL (not both NULL);  info  int32[batch]
+ * Returns MIR_B200_EINVAL for a NULL model, x, l, u or info, cov and stddev both NULL, n == 0 or m == 0, a data model
+ * with NULL t / y, or an n the model rejects; MIR_B200_EUNSUPPORTED for n > 128 and for LINEAR2, ROSENBROCK and
+ * SQRTCIRCLE.  batch == 0 does nothing.  A problem's output bits depend only on its own inputs (not on the batch size,
+ * its position or the run).
+ * Host-pointer form: stages the inputs to `device` (-1 = current), runs, copies cov / stddev / info back.  Device form:
+ * every pointer (model->t, model->y, model->aux, x, l, u, cov, stddev, info) is a device pointer on the current device;
+ * asynchronous on `cuda_stream`.
+ */
+enum { MIR_COV_UNSCALED = 1u };
+
+int mir_b200_covariance_batched_d(const mir_least_squares_settings_d* settings, const mir_model_desc* model,
+    size_t batch, size_t m, size_t n, const double* x, const double* l, const double* u, size_t bound_stride,
+    unsigned cov_flags, double* cov, double* stddev, int32_t* info, int device);
+int mir_b200_covariance_batched_s(const mir_least_squares_settings_s* settings, const mir_model_desc* model,
+    size_t batch, size_t m, size_t n, const float* x, const float* l, const float* u, size_t bound_stride,
+    unsigned cov_flags, float* cov, float* stddev, int32_t* info, int device);
+int mir_b200_covariance_batched_dev_d(const mir_least_squares_settings_d* settings, const mir_model_desc* model,
+    size_t batch, size_t m, size_t n, const double* x, const double* l, const double* u, size_t bound_stride,
+    unsigned cov_flags, double* cov, double* stddev, int32_t* info, void* cuda_stream);
+int mir_b200_covariance_batched_dev_s(const mir_least_squares_settings_s* settings, const mir_model_desc* model,
+    size_t batch, size_t m, size_t n, const float* x, const float* l, const float* u, size_t bound_stride,
+    unsigned cov_flags, float* cov, float* stddev, int32_t* info, void* cuda_stream);
+
+/*
  * fitSpline (fit_splie.d:26-85): least-squares fit of a C2 cubic spline (mir.interpolate.spline with the default
  * SplineConfiguration: not-a-knot ends) with FIXED knots x[n] to `points` data points; the unknowns are the spline
  * values at the knots, bounded by l[n] <= spline(x) <= u[n]; lambda >= 0 weighs the smoothing term

@@ -54,6 +54,7 @@ MODEL_GRID_PER_PROBLEM = 2
 MODEL_NO_TAIL_SHORTCUT = 4
 MODEL_AUX_PER_PROBLEM = 8
 MODEL_WARM_START = 16
+COV_UNSCALED = 1
 
 
 def _settings_types(real):
@@ -144,6 +145,8 @@ B200_SYMBOLS = [
     "mir_b200_nccl_unique_id", "mir_b200_nccl_comm_init", "mir_b200_nccl_comm_destroy",
     "mir_fit_spline_d", "mir_fit_spline_s", "mir_fit_spline_batched_d", "mir_fit_spline_batched_s",
     "mir_b200_model_compile", "mir_b200_model_release",
+    "mir_b200_covariance_batched_d", "mir_b200_covariance_batched_s",
+    "mir_b200_covariance_batched_dev_d", "mir_b200_covariance_batched_dev_s",
 ]
 
 
@@ -188,6 +191,11 @@ def bind_b200_abi(lib):
         fn = getattr(lib, f"mir_solve_box_qp_{sfx}")
         fn.argtypes = [C.POINTER(Q), C.c_size_t, vp, vp, vp, vp, vp]
         fn.restype = C.c_int
+        for dev in ("", "_dev"):
+            fn = getattr(lib, f"mir_b200_covariance_batched{dev}_{sfx}")
+            fn.argtypes = [C.POINTER(S), C.POINTER(ModelDesc), C.c_size_t, C.c_size_t, C.c_size_t,
+                           vp, vp, vp, C.c_size_t, C.c_uint, vp, vp, vp, vp if dev else C.c_int]
+            fn.restype = C.c_int
     fn = lib.mir_optimize_least_squares_sharded_d
     fn.argtypes = [C.POINTER(LeastSquaresSettingsD), C.POINTER(ModelDesc), C.c_size_t, C.c_size_t, vp, vp, vp,
                    vp, vp, C.POINTER(LeastSquaresResultD), C.POINTER(BatchStats)]

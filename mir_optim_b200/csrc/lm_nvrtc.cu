@@ -2,7 +2,9 @@
 // f / g, least_squares.d:78-80, 803-867).  mir_b200_model_compile registers the source; the first launch per precision
 // compiles `lm_cta_kernel<CtaUser<UserModel<T>, T>, T, FD>` (the general batched LM kernel, lm_cta.cuh, whose sources
 // are embedded in the library by embed_headers.py) with NVRTC for sm_100a, loads the cubin with the driver API and
-// caches the functions.  libnvrtc and libcuda are bound with dlopen: the library has no link-time dependency on them.
+// caches the functions.  The covariance kernel (`lm_cov_cta_kernel`, lm_cov.cuh) is a separate program, compiled at
+// the first covariance call per precision, so registration does no extra work for it.  libnvrtc and libcuda are bound
+// with dlopen: the library has no link-time dependency on them.
 #include <dlfcn.h>
 
 #include <cstring>
@@ -12,7 +14,7 @@
 #include <string>
 #include <vector>
 
-#include "lm_cta.cuh"
+#include "lm_cov.cuh"
 #include "runtime.cuh"
 
 namespace mirb200 {
@@ -80,25 +82,30 @@ Rtc& rtc()
 }
 
 struct Compiled { void* module = nullptr; void* fn[2] = {nullptr, nullptr}; };   // fn[FD]
+// the two programs compiled per user model: the LM kernel (at registration for double) and the covariance kernel (lazily)
+enum Program { kProgLM = 0, kProgCov = 1 };
 struct UserModelEntry {
     std::string source;
     std::mutex mu;                                  // compilation / loading of THIS model (others are not held up)
-    std::map<int, std::unique_ptr<Compiled>> loaded;    // key = device ordinal * 2 + (float ? 1 : 0): a module belongs to one context
-    std::vector<char> cubin[2]; std::string names[2][2];   // compiled code per precision (double: made at registration), kept for other devices
+    // key = (device ordinal * 2 + (float ? 1 : 0)) * 2 + program: a module belongs to one context
+    std::map<int, std::unique_ptr<Compiled>> loaded;
+    std::vector<char> cubin[2][2]; std::string names[2][2][2];   // [program][precision], kept for other devices
 };
 std::mutex g_mu;
 std::map<uint32_t, std::shared_ptr<UserModelEntry>> g_models;
 uint32_t g_next = (uint32_t)MIR_MODEL_USER_BASE;
 
 // NVRTC compile (no device needed); cubin returned in `cubin`, lowered kernel names in names[FD]
-int compile_source(const std::string& user, bool isFloat, std::vector<char>& cubin, std::string names[2])
+int compile_source(const std::string& user, bool isFloat, Program which, std::vector<char>& cubin, std::string names[2])
 {
     Rtc& r = rtc();
     if (!r.ok) { set_error("mir_optim_b200: run-time compilation unavailable: " + r.why); return MIR_B200_EUNSUPPORTED; }
     const char* T = isFloat ? "float" : "double";
-    std::string src = "#include \"lm_cta.cuh\"\n#line 1 \"user_model.cu\"\n" + user + "\n";
-    const std::string e0 = std::string("mirb200::lm_cta_kernel<mirb200::CtaUser<UserModel<") + T + ">, " + T + ">, " + T + ", false>";
-    const std::string e1 = std::string("mirb200::lm_cta_kernel<mirb200::CtaUser<UserModel<") + T + ">, " + T + ">, " + T + ", true>";
+    const std::string header = which == kProgLM ? "lm_cta.cuh" : "lm_cov.cuh";
+    const std::string kernel = which == kProgLM ? "mirb200::lm_cta_kernel" : "mirb200::lm_cov_cta_kernel";
+    std::string src = "#include \"" + header + "\"\n#line 1 \"user_model.cu\"\n" + user + "\n";
+    const std::string e0 = kernel + "<mirb200::CtaUser<UserModel<" + T + ">, " + T + ">, " + T + ", false>";
+    const std::string e1 = kernel + "<mirb200::CtaUser<UserModel<" + T + ">, " + T + ">, " + T + ", true>";
     nvrtcProgram prog = nullptr;
     int rc = r.createProgram(&prog, src.c_str(), "mir_user_model.cu", kEmbeddedCount, kEmbeddedSources, kEmbeddedNames);
     if (rc) { set_error(std::string("mir_optim_b200: nvrtcCreateProgram: ") + (r.getErrorString ? r.getErrorString(rc) : "?")); return MIR_B200_ECUDA; }
@@ -120,7 +127,7 @@ int compile_source(const std::string& user, bool isFloat, std::vector<char>& cub
     cubin.resize(sz);
     if (sz) r.getCUBIN(prog, cubin.data());
     r.destroyProgram(&prog);
-    if (!sz || names[0].empty() || names[1].empty()) { set_error("mir_optim_b200: NVRTC produced no code for the LM kernel"); return MIR_B200_ECUDA; }
+    if (!sz || names[0].empty() || names[1].empty()) { set_error("mir_optim_b200: NVRTC produced no code for the kernel"); return MIR_B200_ECUDA; }
     return MIR_B200_OK;
 }
 
@@ -132,7 +139,7 @@ int cu_fail(const char* what, int rc)
     return MIR_B200_ECUDA;
 }
 
-int get_compiled(uint32_t id, bool isFloat, Compiled** out)
+int get_compiled(uint32_t id, bool isFloat, Program prog, Compiled** out)
 {
     std::shared_ptr<UserModelEntry> e;
     {
@@ -144,17 +151,17 @@ int get_compiled(uint32_t id, bool isFloat, Compiled** out)
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) dev = 0;
     std::lock_guard<std::mutex> g(e->mu);
-    std::unique_ptr<Compiled>& c = e->loaded[dev * 2 + (isFloat ? 1 : 0)];
+    std::unique_ptr<Compiled>& c = e->loaded[(dev * 2 + (isFloat ? 1 : 0)) * 2 + prog];
     if (!c) {
         const int pi = isFloat ? 1 : 0;
-        if (e->cubin[pi].empty()) { const int rc = compile_source(e->source, isFloat, e->cubin[pi], e->names[pi]); if (rc) return rc; }
+        if (e->cubin[prog][pi].empty()) { const int rc = compile_source(e->source, isFloat, prog, e->cubin[prog][pi], e->names[prog][pi]); if (rc) return rc; }
         Rtc& r = rtc();
         if (!r.okCu) { set_error("mir_optim_b200: cannot load a compiled model: " + r.whyCu); return MIR_B200_ENODEVICE; }
         auto cc = std::make_unique<Compiled>();
-        int cr = r.cuModuleLoadData(&cc->module, e->cubin[pi].data());
+        int cr = r.cuModuleLoadData(&cc->module, e->cubin[prog][pi].data());
         if (cr) return cu_fail("cuModuleLoadData (user model)", cr);
         for (int fd = 0; fd < 2; ++fd) {
-            cr = r.cuModuleGetFunction(&cc->fn[fd], cc->module, e->names[pi][fd].c_str());
+            cr = r.cuModuleGetFunction(&cc->fn[fd], cc->module, e->names[prog][pi][fd].c_str());
             if (cr) return cu_fail("cuModuleGetFunction (user model)", cr);
         }
         c = std::move(cc);
@@ -170,7 +177,7 @@ int launch_user_model(const mir_model_desc& model, size_t n, const typename Num<
 {
     if (n > 128) { set_error("mir_optim_b200: the batched path supports n <= 128"); return MIR_B200_EUNSUPPORTED; }
     Compiled* c = nullptr;
-    int rc = get_compiled(model.model, sizeof(T) == 4, &c);
+    int rc = get_compiled(model.model, sizeof(T) == 4, kProgLM, &c);
     if (rc) return rc;
     Rtc& r = rtc();
     void* fn = c->fn[(args.flags & MIR_MODEL_FD_JACOBIAN) ? 1 : 0];      // (a model without jacobian() runs finite differences either way)
@@ -205,6 +212,40 @@ int launch_user_model(const mir_model_desc& model, size_t n, const typename Num<
 template int launch_user_model<double>(const mir_model_desc&, size_t, const Num<double>::Settings&, const SmallBatchArgs&, cudaStream_t);
 template int launch_user_model<float>(const mir_model_desc&, size_t, const Num<float>::Settings&, const SmallBatchArgs&, cudaStream_t);
 
+template <class T>
+int launch_user_cov(const mir_model_desc& model, T jacEps, CovArgs ca, cudaStream_t stream)
+{
+    Compiled* c = nullptr;
+    int rc = get_compiled(model.model, sizeof(T) == 4, kProgCov, &c);
+    if (rc) return rc;
+    Rtc& r = rtc();
+    void* fn = c->fn[(model.flags & MIR_MODEL_FD_JACOBIAN) ? 1 : 0];      // (a model without jacobian() runs finite differences either way)
+    const size_t smem = cov_smem_bytes<T>((int)ca.n, 1);
+    if (smem > kCovSmemLimit) { set_error("mir_optim_b200: n too large for the shared memory of the covariance kernel"); return MIR_B200_EUNSUPPORTED; }
+    int cr = r.cuFuncSetAttribute(fn, 8 /* CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES */, (int)smem);
+    if (cr) return cu_fail("cuFuncSetAttribute", cr);
+    int blocksPerSM = 0;
+    cr = r.cuOccupancy(&blocksPerSM, fn, CTA_NT, smem);
+    if (cr) return cu_fail("cuOccupancyMaxActiveBlocksPerMultiprocessor", cr);
+    if (blocksPerSM < 1) blocksPerSM = 1;
+    if (blocksPerSM > 8) blocksPerSM = 8;
+    unsigned long long grid = (unsigned long long)sm_count() * blocksPerSM;
+    if (ca.batch < grid) grid = ca.batch;
+    ca.scratch_stride = (unsigned long long)ca.m * ca.n + ca.m + 2;
+    grid = cta_cap_grid(grid, ca.scratch_stride * sizeof(T));
+    T* scratch = nullptr;
+    MIRB200_CUDA(cudaMallocAsync((void**)&scratch, sizeof(T) * ca.scratch_stride * grid, stream));
+    ca.scratch = scratch;
+    void* params[] = {&jacEps, &ca};
+    cr = r.cuLaunchKernel(fn, (unsigned)grid, 1, 1, CTA_NT, 1, 1, (unsigned)smem, stream, params, nullptr);
+    count_launch();
+    cudaFreeAsync(scratch, stream);
+    if (cr) return cu_fail("cuLaunchKernel (user model covariance)", cr);
+    return MIR_B200_OK;
+}
+template int launch_user_cov<double>(const mir_model_desc&, double, CovArgs, cudaStream_t);
+template int launch_user_cov<float>(const mir_model_desc&, float, CovArgs, cudaStream_t);
+
 }  // namespace mirb200
 
 using namespace mirb200;
@@ -218,7 +259,7 @@ int mir_b200_model_compile(const char* source, uint32_t* model_id)
     // validate now (double precision; NVRTC needs no device), so that syntax errors surface at registration
     auto e = std::make_shared<UserModelEntry>();
     e->source = source;
-    const int rc = compile_source(e->source, false, e->cubin[0], e->names[0]);
+    const int rc = compile_source(e->source, false, kProgLM, e->cubin[kProgLM][0], e->names[kProgLM][0]);
     if (rc) return rc;
     std::lock_guard<std::mutex> g(g_mu);
     *model_id = g_next++;
@@ -235,7 +276,7 @@ int mir_b200_model_release(uint32_t model_id)
     int cur = 0; cudaGetDevice(&cur);
     for (auto& kv : it->second->loaded) {
         if (!kv.second || !kv.second->module || !rtc().cuModuleUnload) continue;
-        if (cudaSetDevice(kv.first / 2) == cudaSuccess) { cudaDeviceSynchronize(); rtc().cuModuleUnload(kv.second->module); }
+        if (cudaSetDevice(kv.first / 4) == cudaSuccess) { cudaDeviceSynchronize(); rtc().cuModuleUnload(kv.second->module); }
     }
     cudaSetDevice(cur);
     g_models.erase(it);

@@ -97,9 +97,12 @@ class Engine(ReferenceAPI):
 
     # -- batched LM, device-resident torch tensors ----------------------------------------
     def optimize_batched_device(self, settings, model: ModelId, x, l, u, t=None, y=None, m: int | None = None,
-                                fd_jacobian: bool = False, results=None, stats=None, stream=None, tail_shortcut: bool = True):
+                                fd_jacobian: bool = False, results=None, stats=None, stream=None, tail_shortcut: bool = True,
+                                aux=None, param: float = 0.0, warm_start: bool = False):
         """All tensors are CUDA tensors on the current device; asynchronous on `stream` (default:
-        torch's current stream).  `results` : uint8 tensor (batch * sizeof(Result)); `stats`: int64[8] tensor."""
+        torch's current stream).  `results` : uint8 tensor (batch * sizeof(Result)); `stats`: int64[8] tensor.
+        aux: (n,) shared or (batch, n) model constants (the knots of ModelId.SPLINE); param: the model constant;
+        warm_start: results holds a previous call's Result PODs and their lambda is the initial damping."""
         import torch
         dt = np.dtype({torch.float64: np.float64, torch.float32: np.float32}[x.dtype])
         sfx, real, S, R, *_ = _types(dt)
@@ -111,9 +114,14 @@ class Engine(ReferenceAPI):
             m = y.shape[1] if m is None else m
         if t is not None and t.dim() == 2:
             flags |= MODEL_GRID_PER_PROBLEM
+        if aux is not None and aux.dim() == 2:
+            flags |= _abi.MODEL_AUX_PER_PROBLEM
+        if warm_start:
+            assert results is not None, "warm_start reads the lambda of a previous call's results"
+            flags |= _abi.MODEL_WARM_START
         if results is None:
             results = torch.empty(batch * RESULT_DTYPES[dt].itemsize, dtype=torch.uint8, device=x.device)
-        desc = ModelDesc(int(model), flags, _vp(t), _vp(y))
+        desc = ModelDesc(int(model), flags, _vp(t), _vp(y), _vp(aux), float(param))
         if stream is None:
             stream = torch.cuda.current_stream(x.device).cuda_stream
         fn = getattr(self.lib, f"mir_optimize_least_squares_batched_dev_{sfx}")
@@ -121,6 +129,80 @@ class Engine(ReferenceAPI):
                 _vp(results), _vp(stats), C.c_void_p(stream))
         self._check(rc)
         return results
+
+    # -- parameter covariance at a given point -------------------------------------------------
+    def covariance_batched(self, settings, model: ModelId, x: np.ndarray, l: np.ndarray, u: np.ndarray,
+                           t: np.ndarray | None = None, y: np.ndarray | None = None, m: int | None = None,
+                           fd_jacobian: bool = False, aux: np.ndarray | None = None, param: float = 0.0,
+                           scaled: bool = True, want_cov: bool = True, device: int = -1):
+        """Covariance and standard errors of the parameters x (batch, n) -- normally a fit's output -- with the model data
+        of :meth:`optimize_batched`.  settings may be None (only jacobianEpsilon is read).  scaled=False: residuals are
+        already divided by sigma (s^2 = 1, scipy's absolute_sigma=True).  Returns (cov (batch, n, n) or None,
+        stddev (batch, n), info int32[batch]); info: 0 OK, k > 0 breakdown at parameter k-1, -1 m <= number of free
+        parameters, -2 non-finite values (see mir_b200_covariance_batched_d in the header)."""
+        x = np.ascontiguousarray(x)
+        sfx, real, S, R, *_ = _types(x.dtype)
+        assert settings is None or isinstance(settings, S)
+        assert x.ndim == 2
+        batch, n = x.shape
+        l = np.ascontiguousarray(l, dtype=x.dtype); u = np.ascontiguousarray(u, dtype=x.dtype)
+        bound_stride = 0 if l.ndim == 1 else n
+        flags = MODEL_FD_JACOBIAN if fd_jacobian else 0
+        if y is not None:
+            y = np.ascontiguousarray(y, dtype=x.dtype); assert y.shape[0] == batch
+            m = y.shape[1] if m is None else m
+        if t is not None:
+            t = np.ascontiguousarray(t, dtype=x.dtype)
+            if t.ndim == 2:
+                flags |= MODEL_GRID_PER_PROBLEM
+        assert m is not None, "m is required for models without samples"
+        if aux is not None:
+            aux = np.ascontiguousarray(aux, dtype=x.dtype)
+            if aux.ndim == 2:
+                flags |= _abi.MODEL_AUX_PER_PROBLEM
+        desc = ModelDesc(int(model), flags, _vp(t), _vp(y), _vp(aux), float(param))
+        cov = np.empty((batch, n, n), dtype=x.dtype) if want_cov else None
+        stddev = np.empty((batch, n), dtype=x.dtype)
+        info = np.empty(batch, dtype=np.int32)
+        fn = getattr(self.lib, f"mir_b200_covariance_batched_{sfx}")
+        rc = fn(C.byref(settings) if settings is not None else None, C.byref(desc), batch, m, n, _vp(x), _vp(l), _vp(u),
+                bound_stride, 0 if scaled else _abi.COV_UNSCALED, _vp(cov), _vp(stddev), _vp(info), device)
+        self._check(rc)
+        return cov, stddev, info
+
+    def covariance_batched_device(self, settings, model: ModelId, x, l, u, t=None, y=None, m: int | None = None,
+                                  fd_jacobian: bool = False, aux=None, param: float = 0.0, scaled: bool = True,
+                                  want_cov: bool = True, cov=None, stddev=None, info=None, stream=None):
+        """:meth:`covariance_batched` on CUDA tensors of the current device, asynchronous on `stream` (default: torch's
+        current stream).  cov / stddev / info may be preallocated.  Returns (cov or None, stddev, info) tensors."""
+        import torch
+        dt = np.dtype({torch.float64: np.float64, torch.float32: np.float32}[x.dtype])
+        sfx, real, S, R, *_ = _types(dt)
+        assert (settings is None or isinstance(settings, S)) and x.is_cuda and x.is_contiguous()
+        batch, n = x.shape
+        bound_stride = 0 if l.dim() == 1 else n
+        flags = MODEL_FD_JACOBIAN if fd_jacobian else 0
+        if y is not None:
+            m = y.shape[1] if m is None else m
+        if t is not None and t.dim() == 2:
+            flags |= MODEL_GRID_PER_PROBLEM
+        if aux is not None and aux.dim() == 2:
+            flags |= _abi.MODEL_AUX_PER_PROBLEM
+        assert m is not None, "m is required for models without samples"
+        if cov is None and want_cov:
+            cov = torch.empty((batch, n, n), dtype=x.dtype, device=x.device)
+        if stddev is None:
+            stddev = torch.empty((batch, n), dtype=x.dtype, device=x.device)
+        if info is None:
+            info = torch.empty(batch, dtype=torch.int32, device=x.device)
+        desc = ModelDesc(int(model), flags, _vp(t), _vp(y), _vp(aux), float(param))
+        if stream is None:
+            stream = torch.cuda.current_stream(x.device).cuda_stream
+        fn = getattr(self.lib, f"mir_b200_covariance_batched_dev_{sfx}")
+        rc = fn(C.byref(settings) if settings is not None else None, C.byref(desc), batch, m, n, _vp(x), _vp(l), _vp(u),
+                bound_stride, 0 if scaled else _abi.COV_UNSCALED, _vp(cov), _vp(stddev), _vp(info), C.c_void_p(stream))
+        self._check(rc)
+        return cov, stddev, info
 
     # -- user-defined device models (NVRTC) ---------------------------------------------------
     def compile_model(self, cuda_source: str) -> int:
