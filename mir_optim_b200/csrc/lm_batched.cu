@@ -19,7 +19,7 @@ namespace mirb200 {
 
 // Models that read samples need both arrays (t: m or batch*m abscissae, y: batch*m observations -- the lengths are the
 // caller's contract, stated in the header); only LINEAR2, ROSENBROCK and SQRTCIRCLE are data-free.
-bool model_needs_data(unsigned model)
+static bool model_needs_data(unsigned model)
 {
     return !(model == MIR_MODEL_LINEAR2 || model == MIR_MODEL_ROSENBROCK || model == MIR_MODEL_SQRTCIRCLE || model >= (unsigned)MIR_MODEL_USER_BASE);
 }
@@ -34,7 +34,8 @@ static bool specialised_shape(unsigned model, size_t n)
     default: return false;
     }
 }
-static int check_model_data(const mir_model_desc* model, size_t batch, size_t m)
+// the samples check of the batched fit and of the covariance (lm_cov.cu)
+int check_model_data(const mir_model_desc* model, size_t batch, size_t m)
 {
     if (batch && m && model_needs_data(model->model) && (!model->t || !model->y)) {
         set_error("mir_optim_b200: this model reads samples: model->t and model->y must not be NULL");

@@ -1,57 +1,16 @@
 // lm_cov.cu -- C ABI of the batched covariance entry points (mir_b200_covariance_batched_*): argument checks, staging of
-// host buffers, and the launch of lm_cov_cta_kernel (lm_cov.cuh) for the built-in models.
+// host buffers, and the launch of lm_cov_cta_kernel (lm_cov.cuh) for the built-in models, with the model table
+// (visit_cta_model) and the launch policy (launch_persistent) of the general batched LM kernel.
 #include "lm_cov.cuh"
 #include "runtime.cuh"
 
 namespace mirb200 {
 
-bool model_needs_data(unsigned model);   // lm_batched.cu
+int check_model_data(const mir_model_desc* model, size_t batch, size_t m);   // lm_batched.cu
 
 namespace {
 
-template <class M> struct CovTag { using type = M; };
-
-// the model ids the general batched kernel serves, by functor; MIR_B200_EUNSUPPORTED for the rest (user models excluded)
-template <class T, class F> int visit_cov_model(uint32_t id, F&& f)
-{
-    switch (id) {
-    case MIR_MODEL_EXPDECAY2: return f(CovTag<CtaFromLarge<LModelExpDecay2<T>, T>>{});
-    case MIR_MODEL_EXPTAU3:   return f(CovTag<CtaFromLarge<LModelExpTau3<T>, T>>{});
-    case MIR_MODEL_EXPDECAY3: return f(CovTag<CtaFromLarge<LModelExpDecay3<T>, T>>{});
-    case MIR_MODEL_GAUSS4:    return f(CovTag<CtaFromLarge<LModelGauss4<T>, T>>{});
-    case MIR_MODEL_SUMEXP:    return f(CovTag<CtaFromLarge<LModelSumExp<T>, T>>{});
-    case MIR_MODEL_GAUSSMIX:  return f(CovTag<CtaFromLarge<LModelGaussMix<T>, T>>{});
-    case MIR_MODEL_SPLINE:    return f(CovTag<CtaSpline<T>>{});
-    default:
-        set_error("mir_optim_b200: model id not available for the covariance (it has no run-time-n functor)");
-        return MIR_B200_EUNSUPPORTED;
-    }
-}
-
-template <class Model, class T, bool FD>
-int launch_cov_fd(T jacEps, CovArgs ca, cudaStream_t stream)
-{
-    auto kern = lm_cov_cta_kernel<Model, T, FD>;
-    const size_t smem = cov_smem_bytes<T>((int)ca.n, Model::prep_elems((int)ca.n));
-    if (smem > kCovSmemLimit) { set_error("mir_optim_b200: n too large for the shared memory of the covariance kernel"); return MIR_B200_EUNSUPPORTED; }
-    MIRB200_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int blocksPerSM = 0;
-    MIRB200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocksPerSM, kern, CTA_NT, smem));
-    if (blocksPerSM < 1) blocksPerSM = 1;
-    if (blocksPerSM > 8) blocksPerSM = 8;
-    unsigned long long grid = (unsigned long long)sm_count() * blocksPerSM;
-    if (ca.batch < grid) grid = ca.batch;
-    ca.scratch_stride = (unsigned long long)ca.m * ca.n + ca.m + 2;
-    grid = cta_cap_grid(grid, ca.scratch_stride * sizeof(T));
-    T* scratch = nullptr;
-    MIRB200_CUDA(cudaMallocAsync((void**)&scratch, sizeof(T) * ca.scratch_stride * grid, stream));
-    ca.scratch = scratch;
-    kern<<<(unsigned)grid, CTA_NT, smem, stream>>>(jacEps, ca);
-    count_launch();
-    const int rc = check_cuda(cudaGetLastError(), "lm_cov_cta_kernel launch");
-    cudaFreeAsync(scratch, stream);
-    return rc;
-}
+constexpr const char* kNoCovModel = "mir_optim_b200: model id not available for the covariance (it has no run-time-n functor)";
 
 // argument checks shared by both forms (batch may be 0; data pointers are checked by the caller when batch > 0)
 template <class T>
@@ -63,8 +22,7 @@ int cov_check(const mir_model_desc* model, size_t m, size_t n, const void* cov, 
     if (n > 128) { set_error("mir_optim_b200: the covariance supports n <= 128"); return MIR_B200_EUNSUPPORTED; }
     if (m >= 0x7fffffffull) { set_error("mir_optim_b200: m too large"); return MIR_B200_EUNSUPPORTED; }
     if (model->model >= (uint32_t)MIR_MODEL_USER_BASE) return MIR_B200_OK;      // checked when the model is loaded
-    if (model->model == MIR_MODEL_SPLINE && !model->aux) { set_error("mir_optim_b200: MIR_MODEL_SPLINE needs the knots in model->aux"); return MIR_B200_EINVAL; }
-    return visit_cov_model<T>(model->model, [&](auto tag) {
+    return visit_cta_model<T>(*model, kNoCovModel, [&](auto tag) {
         using M = typename decltype(tag)::type;
         if (!M::valid((int)n, (int)m)) { set_error("mir_optim_b200: (m, n) not valid for this model"); return (int)MIR_B200_EINVAL; }
         return (int)MIR_B200_OK;
@@ -72,13 +30,11 @@ int cov_check(const mir_model_desc* model, size_t m, size_t n, const void* cov, 
 }
 
 template <class T>
-int cov_check_data(const mir_model_desc* model, const T* x, const T* l, const T* u, size_t n, size_t bound_stride, const int32_t* info)
+int cov_check_data(const mir_model_desc* model, size_t batch, size_t m, const T* x, const T* l, const T* u, size_t n, size_t bound_stride,
+                   const int32_t* info)
 {
     if (!x || !l || !u || !info) { set_error("mir_optim_b200: null argument"); return MIR_B200_EINVAL; }
-    if (model_needs_data(model->model) && (!model->t || !model->y)) {
-        set_error("mir_optim_b200: this model reads samples: model->t and model->y must not be NULL");
-        return MIR_B200_EINVAL;
-    }
+    if (int rc = check_model_data(model, batch, m)) return rc;
     if (bound_stride != 0 && bound_stride < n) { set_error("mir_optim_b200: bound_stride must be 0 or >= n"); return MIR_B200_EINVAL; }
     return MIR_B200_OK;
 }
@@ -91,7 +47,7 @@ int covariance_dev(const typename Num<T>::Settings* settings, const mir_model_de
     clear_error();
     if (int rc = cov_check<T>(model, m, n, cov, stddev)) return rc;
     if (batch == 0) return MIR_B200_OK;
-    if (int rc = cov_check_data<T>(model, x, l, u, n, bound_stride, info)) return rc;
+    if (int rc = cov_check_data<T>(model, batch, m, x, l, u, n, bound_stride, info)) return rc;
     if (batch >= 0xffffffffull) { set_error("mir_optim_b200: at most 2^32 - 2 problems per launch"); return MIR_B200_EINVAL; }
     if (int rc = require_device(-1)) return rc;
     typename Num<T>::Settings defaults;
@@ -119,7 +75,7 @@ int covariance_host(const typename Num<T>::Settings* settings, const mir_model_d
 {
     clear_error();
     if (int rc = cov_check<T>(model, m, n, cov, stddev)) return rc;
-    if (batch) { if (int rc = cov_check_data<T>(model, x, l, u, n, bound_stride, info)) return rc; }
+    if (batch) { if (int rc = cov_check_data<T>(model, batch, m, x, l, u, n, bound_stride, info)) return rc; }
     if (int rc = require_device(device)) return rc;
     if (batch == 0) return MIR_B200_OK;
 
@@ -181,11 +137,11 @@ template <class T>
 int launch_cov_model(const mir_model_desc& model, T jacEps, CovArgs ca, cudaStream_t stream)
 {
     if (model.model >= (uint32_t)MIR_MODEL_USER_BASE) return launch_user_cov<T>(model, jacEps, ca, stream);
-    const bool fd = (model.flags & MIR_MODEL_FD_JACOBIAN) != 0;
-    return visit_cov_model<T>(model.model, [&](auto tag) {
+    return visit_cta_model<T>(model, kNoCovModel, [&](auto tag) {
         using M = typename decltype(tag)::type;
-        if (fd || !M::kAnalytic) return launch_cov_fd<M, T, true>(jacEps, ca, stream);
-        return launch_cov_fd<M, T, false>(jacEps, ca, stream);
+        const bool fd = (model.flags & MIR_MODEL_FD_JACOBIAN) || !M::kAnalytic;
+        const RuntimeKernel kern{fd ? (const void*)lm_cov_cta_kernel<M, T, true> : (const void*)lm_cov_cta_kernel<M, T, false>, "lm_cov_cta_kernel launch"};
+        return launch_cov<T>(kern, jacEps, ca, M::prep_elems((int)ca.n), stream);
     });
 }
 template int launch_cov_model<double>(const mir_model_desc&, double, CovArgs, cudaStream_t);

@@ -4,9 +4,9 @@
 // include/mir_optim_b200.h next to mir_b200_covariance_batched_{d,s}.
 //
 // Layout.  Persistent CTAs of CTA_NT threads pull problems from an atomic counter.  Residuals and J (row-major m x n, the
-// fit's layout) go to a per-CTA global scratch; rows are dealt to the threads round-robin, and J is evaluated exactly
-// like the fresh-Jacobian step of lm_cta_kernel (analytic rows, or the reference's central difference with the bound
-// clamp of least_squares.d:1030-1047), over the free columns only.  A = J_F^T J_F is built in double, one thread per
+// fit's layout) go to a per-CTA global scratch; rows are dealt to the threads round-robin, and J is evaluated by the
+// fresh-Jacobian step of lm_cta_kernel (analytic rows, or cta_fd_column: the reference's central difference with the
+// bound clamp of least_squares.d:1030-1047), over the free columns only.  A = J_F^T J_F is built in double, one thread per
 // packed entry over the rows in row order; ||r||^2 is a cta_sum_all of per-thread partial sums in row order.  So every
 // bit of a problem's output depends on its own inputs only.  The scaled block, its Cholesky factor L, L^-1 and S^-1
 // live in shared memory as packed lower triangles (n <= 128: at most 2 x 66 KB).
@@ -35,15 +35,6 @@ struct CovArgs {
 };
 
 template <class T> __device__ __forceinline__ bool cov_finite(T v) { return t_abs(v) < Num<T>::inf(); }
-
-// row index i >= j of the packed lower-triangular entry e (tri(i, j) == e)
-__device__ __forceinline__ void cov_untri(int e, int& i, int& j)
-{
-    i = (int)((sqrtf(8.0f * (float)e + 1.0f) - 1.0f) * 0.5f);
-    while ((i + 1) * (i + 2) / 2 <= e) ++i;
-    while (i * (i + 1) / 2 > e) --i;
-    j = e - i * (i + 1) / 2;
-}
 
 template <class Model, class T, bool FD>
 __global__ void __launch_bounds__(CTA_NT)
@@ -79,12 +70,7 @@ lm_cov_cta_kernel(const T jacEps, const CovArgs ca)
         const unsigned long long prob = s_idx;
         if (prob >= ca.batch) break;
 
-        CtaProblem<T> pb;
-        pb.m = m; pb.n = n;
-        pb.t = ca.t ? static_cast<const T*>(ca.t) + ((ca.flags & MIR_MODEL_GRID_PER_PROBLEM) ? prob * m : 0) : nullptr;
-        pb.y = ca.y ? static_cast<const T*>(ca.y) + prob * m : nullptr;
-        pb.aux = ca.aux ? static_cast<const T*>(ca.aux) + ((ca.flags & MIR_MODEL_AUX_PER_PROBLEM) ? prob * n : 0) : nullptr;
-        pb.param = (T)ca.param;
+        const CtaProblem<T> pb = cta_problem<T>(ca.t, ca.y, ca.aux, ca.param, ca.flags, m, n, prob);
         bool bad = false;
         for (int i = tid; i < n; i += NT) {
             const T v = static_cast<const T*>(ca.x)[prob * n + i];
@@ -126,30 +112,7 @@ lm_cov_cta_kernel(const T jacEps, const CovArgs ca)
                 if constexpr (!useFD) {
                     for (int r = tid; r < m; r += NT) Model::jacobian_row(pb, x, prep, r, J + (size_t)r * n);
                 } else {
-                    for (int k = 0; k < nf; ++k) {
-                        const int j = fidx[k];
-                        const T xmh = t_max(x[j] - jacEps, lo[j]);                                       // LS:1030-1033
-                        const T xph = t_min(x[j] + jacEps, up[j]);
-                        const T twh = xph - xmh;
-                        if (twh != (T)0) {
-                            const T rt = rcp_ni(twh);
-                            __syncthreads();
-                            for (int i = tid; i < n; i += NT) pp[i] = (i == j) ? xph : x[i];
-                            __syncthreads();
-                            Model::prepare(pb, pp, prep);
-                            for (int r = tid; r < m; r += NT) J[(size_t)r * n + j] = Model::residual(pb, pp, prep, r);
-                            __syncthreads();
-                            if (tid == 0) pp[j] = xmh;
-                            __syncthreads();
-                            Model::prepare(pb, pp, prep);
-                            for (int r = tid; r < m; r += NT) {
-                                const T fm = Model::residual(pb, pp, prep, r);
-                                J[(size_t)r * n + j] = (J[(size_t)r * n + j] - fm) * rt;                 // LS:1040-1042
-                            }
-                        } else {
-                            for (int r = tid; r < m; r += NT) J[(size_t)r * n + j] = (T)0;               // LS:1045-1047
-                        }
-                    }
+                    for (int k = 0; k < nf; ++k) cta_fd_column<Model, T>(pb, x, lo, up, pp, prep, J, fidx[k], jacEps);
                 }
                 for (int r = tid; r < m; r += NT)
                     for (int k = 0; k < nf; ++k) bad = bad || !cov_finite(J[(size_t)r * n + fidx[k]]);
@@ -162,7 +125,7 @@ lm_cov_cta_kernel(const T jacEps, const CovArgs ca)
                 const int NPF = nf * (nf + 1) / 2;
                 // A = J_F^T J_F: one thread per entry, rows in order
                 for (int e = tid; e < NPF; e += NT) {
-                    int i, j; cov_untri(e, i, j);
+                    int i, j; cta_untri(e, i, j);
                     const T* Ji = J + fidx[i];
                     const T* Jj = J + fidx[j];
                     double acc = 0.0;
@@ -173,7 +136,7 @@ lm_cov_cta_kernel(const T jacEps, const CovArgs ca)
                 // S = D^-1/2 A D^-1/2; a zero diagonal gives a zero row and column, so its pivot stops the factorisation
                 for (int i = tid; i < nf; i += NT) { const double d = A[tri(i, i)]; sc[i] = d > 0.0 ? 1.0 / sqrt(d) : 0.0; }
                 __syncthreads();
-                for (int e = tid; e < NPF; e += NT) { int i, j; cov_untri(e, i, j); A[e] = (A[e] * sc[i]) * sc[j]; }
+                for (int e = tid; e < NPF; e += NT) { int i, j; cta_untri(e, i, j); A[e] = (A[e] * sc[i]) * sc[j]; }
                 __syncthreads();
                 // S = L L^T, column by column (LAPACK ?potf2, lower)
                 int fail = -1;
@@ -187,7 +150,7 @@ lm_cov_cta_kernel(const T jacEps, const CovArgs ca)
                     __syncthreads();
                     const int tr = nf - j - 1;
                     for (int e = tid; e < tr * (tr + 1) / 2; e += NT) {      // trailing update, each entry once per column
-                        int i, k; cov_untri(e, i, k);
+                        int i, k; cta_untri(e, i, k);
                         i += j + 1; k += j + 1;
                         A[tri(i, k)] = fma(-A[tri(i, j)], A[tri(k, j)], A[tri(i, k)]);
                     }
@@ -208,7 +171,7 @@ lm_cov_cta_kernel(const T jacEps, const CovArgs ca)
                     __syncthreads();
                     // S^-1 = W^T W (?lauum), lower triangle, into A
                     for (int e = tid; e < NPF; e += NT) {
-                        int i, j; cov_untri(e, i, j);
+                        int i, j; cta_untri(e, i, j);
                         double acc = 0.0;
                         for (int k = i; k < nf; ++k) acc = fma(W[tri(k, i)], W[tri(k, j)], acc);
                         A[e] = acc;
@@ -245,16 +208,20 @@ lm_cov_cta_kernel(const T jacEps, const CovArgs ca)
 }
 
 #ifndef __CUDACC_RTC__
-// dynamic shared memory of lm_cov_cta_kernel for n parameters and a model with `prepElems` prepared values
-template <class T> size_t cov_smem_bytes(int n, int prepElems)
+// lm_cov_cta_kernel (`kern`: built in or compiled at run time) over ca.batch problems, for a model with `prepElems`
+// prepared values
+template <class T, class K> int launch_cov(const K& kern, T jacEps, CovArgs ca, int prepElems, cudaStream_t stream)
 {
-    const size_t np = (size_t)n * (n + 1) / 2;
-    return sizeof(double) * (2 * np + n + 8) + sizeof(T) * (4 * (size_t)n + prepElems) + sizeof(int) * 2 * (size_t)n + 16;
+    const size_t n = ca.n, np = n * (n + 1) / 2;
+    const size_t smem = sizeof(double) * (2 * np + n + 8) + sizeof(T) * (4 * n + prepElems) + sizeof(int) * 2 * n + 16;
+    ca.scratch_stride = (unsigned long long)ca.m * ca.n + ca.m + 2;
+    void* params[] = {&jacEps, &ca};
+    return launch_persistent<T>(kern, smem, "mir_optim_b200: n too large for the shared memory of the covariance kernel", ca.batch,
+                                ca.scratch_stride, ca.scratch, params, stream);
 }
-constexpr size_t kCovSmemLimit = 220 * 1024;
 
 // covariance of the built-in models (lm_cov.cu) and of models compiled at run time (lm_nvrtc.cu).  `ca` is complete
-// except for scratch / scratch_stride, which the launchers fill; the caller has checked the arguments.
+// except for scratch / scratch_stride, which launch_cov fills; the caller has checked the arguments.
 template <class T>
 int launch_cov_model(const mir_model_desc& model, T jacEps, CovArgs ca, cudaStream_t stream);
 template <class T>

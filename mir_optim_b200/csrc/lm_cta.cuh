@@ -240,6 +240,63 @@ template <class U, class T> struct CtaUser {
     }
 };
 
+// ---- pieces shared by lm_cta_kernel and lm_cov_cta_kernel (lm_cov.cuh) ----------------------------------------------------
+// problem `prob` of a batch: t (m or batch*m, MIR_MODEL_GRID_PER_PROBLEM), y (batch*m), aux (n or batch*n,
+// MIR_MODEL_AUX_PER_PROBLEM); null arrays stay null
+template <class T>
+__device__ __forceinline__ CtaProblem<T> cta_problem(const void* t, const void* y, const void* aux, double param, unsigned flags,
+                                                     int m, int n, unsigned long long prob)
+{
+    CtaProblem<T> pb;
+    pb.m = m; pb.n = n;
+    pb.t = t ? static_cast<const T*>(t) + ((flags & MIR_MODEL_GRID_PER_PROBLEM) ? prob * m : 0) : nullptr;
+    pb.y = y ? static_cast<const T*>(y) + prob * m : nullptr;
+    pb.aux = aux ? static_cast<const T*>(aux) + ((flags & MIR_MODEL_AUX_PER_PROBLEM) ? prob * n : 0) : nullptr;
+    pb.param = (T)param;
+    return pb;
+}
+
+// Column j of the central-difference Jacobian at x into J (m x n row-major), the step clamped to the bounds, or a zero
+// column where the clamped step is empty (LS:1030-1047).  pp (n values) and prep are shared scratch.  Returns whether the
+// model was evaluated (twice).
+template <class Model, class T>
+__device__ __forceinline__ bool cta_fd_column(const CtaProblem<T>& pb, const T* x, const T* lo, const T* up, T* pp, T* prep,
+                                              T* J, int j, T eps)
+{
+    const int tid = threadIdx.x, n = pb.n, m = pb.m;
+    const T xmh = t_max(x[j] - eps, lo[j]);                                                         // LS:1030-1033
+    const T xph = t_min(x[j] + eps, up[j]);
+    const T twh = xph - xmh;
+    if (twh != (T)0) {
+        const T rt = rcp_ni(twh);
+        __syncthreads();
+        for (int i = tid; i < n; i += CTA_NT) pp[i] = (i == j) ? xph : x[i];
+        __syncthreads();
+        Model::prepare(pb, pp, prep);
+        for (int r = tid; r < m; r += CTA_NT) J[(size_t)r * n + j] = Model::residual(pb, pp, prep, r);   // f(x + h e_j), parked in its column
+        __syncthreads();
+        if (tid == 0) pp[j] = xmh;
+        __syncthreads();
+        Model::prepare(pb, pp, prep);
+        for (int r = tid; r < m; r += CTA_NT) {
+            const T fm = Model::residual(pb, pp, prep, r);
+            J[(size_t)r * n + j] = (J[(size_t)r * n + j] - fm) * rt;                                // LS:1040-1042
+        }
+        return true;
+    }
+    for (int r = tid; r < m; r += CTA_NT) J[(size_t)r * n + j] = (T)0;                              // LS:1045-1047
+    return false;
+}
+
+// (i, j), i >= j, of the packed lower-triangular entry e (tri(i, j) == e)
+__device__ __forceinline__ void cta_untri(int e, int& i, int& j)
+{
+    i = (int)((sqrtf(8.0f * (float)e + 1.0f) - 1.0f) * 0.5f);
+    while ((i + 1) * (i + 2) / 2 <= e) ++i;
+    while (i * (i + 1) / 2 > e) --i;
+    j = e - i * (i + 1) / 2;
+}
+
 template <class Model, class T, bool FD>
 __global__ void __launch_bounds__(CTA_NT)
 lm_cta_kernel(const typename Num<T>::Settings st, const CtaBatchArgs ca)
@@ -304,12 +361,7 @@ lm_cta_kernel(const typename Num<T>::Settings st, const CtaBatchArgs ca)
             }
             continue;
         }
-        CtaProblem<T> pb;
-        pb.m = m; pb.n = n;
-        pb.t = args.t ? static_cast<const T*>(args.t) + ((args.flags & MIR_MODEL_GRID_PER_PROBLEM) ? prob * m : 0) : nullptr;
-        pb.y = args.y ? static_cast<const T*>(args.y) + prob * m : nullptr;
-        pb.aux = ca.aux ? static_cast<const T*>(ca.aux) + ((args.flags & MIR_MODEL_AUX_PER_PROBLEM) ? prob * n : 0) : nullptr;
-        pb.param = (T)ca.param;
+        CtaProblem<T> pb = cta_problem<T>(args.t, args.y, ca.aux, ca.param, args.flags, m, n, prob);
         if (stageM && pb.y != nullptr && (reinterpret_cast<uintptr_t>(pb.y) & 15) == 0 && (pb.t == nullptr || (reinterpret_cast<uintptr_t>(pb.t) & 15) == 0)) {
             const bool perGrid = (args.flags & MIR_MODEL_GRID_PER_PROBLEM) != 0;
             const bool needT = pb.t != nullptr && (perGrid || !tStaged);
@@ -429,30 +481,8 @@ lm_cta_kernel(const typename Num<T>::Settings st, const CtaBatchArgs ca)
                         for (int r = tid; r < m; r += NT) Model::jacobian_row(pb, x, prepA, r, J + (size_t)r * n);
                     } else {                                                                        // LS:1018-1049
                         ret.fCalls += (unsigned)n;                                                  // (counts tasks, LS:1049)
-                        for (int j = 0; j < n; ++j) {
-                            const T xmh = t_max(x[j] - st.jacobianEpsilon, lo[j]);                  // LS:1030-1033
-                            const T xph = t_min(x[j] + st.jacobianEpsilon, up[j]);
-                            const T twh = xph - xmh;
-                            if (twh != (T)0) {
-                                const T rt = rcp_ni(twh);
-                                __syncthreads();
-                                for (int i = tid; i < n; i += NT) pp[i] = (i == j) ? xph : x[i];
-                                __syncthreads();
-                                Model::prepare(pb, pp, prepA);
-                                for (int r = tid; r < m; r += NT) J[(size_t)r * n + j] = Model::residual(pb, pp, prepA, r);   // f(x + h e_j), parked in its column
-                                __syncthreads();
-                                if (tid == 0) pp[j] = xmh;
-                                __syncthreads();
-                                Model::prepare(pb, pp, prepA);
-                                for (int r = tid; r < m; r += NT) {
-                                    const T fm = Model::residual(pb, pp, prepA, r);
-                                    J[(size_t)r * n + j] = (J[(size_t)r * n + j] - fm) * rt;        // LS:1040-1042
-                                }
-                                sEvals += 2;
-                            } else {
-                                for (int r = tid; r < m; r += NT) J[(size_t)r * n + j] = (T)0;      // LS:1045-1047
-                            }
-                        }
+                        for (int j = 0; j < n; ++j)
+                            if (cta_fd_column<Model, T>(pb, x, lo, up, pp, prepA, J, j, st.jacobianEpsilon)) sEvals += 2;
                     }
                 }
                 __syncthreads();
@@ -460,10 +490,7 @@ lm_cta_kernel(const typename Num<T>::Settings st, const CtaBatchArgs ca)
                 const int NP = n * (n + 1) / 2;
                 for (int e = tid; e < NP + n; e += NT) {
                     if (e < NP) {
-                        int i = (int)((sqrtf(8.0f * (float)e + 1.0f) - 1.0f) * 0.5f);
-                        while ((i + 1) * (i + 2) / 2 <= e) ++i;
-                        while (i * (i + 1) / 2 > e) --i;
-                        const int j = e - i * (i + 1) / 2;
+                        int i, j; cta_untri(e, i, j);
                         T acc = (T)0;
                         for (int r = 0; r < m; ++r) acc = fma(J[(size_t)r * n + i], J[(size_t)r * n + j], acc);
                         JJ[(size_t)i * n + j] = acc;
@@ -586,19 +613,6 @@ lm_cta_kernel(const typename Num<T>::Settings st, const CtaBatchArgs ca)
 
 // ---- host side -----------------------------------------------------------------------------------------------------------
 #ifndef __CUDACC_RTC__
-template <class T> size_t cta_smem_bytes(int n, int prepElems)
-{
-    return sizeof(T) * ((size_t)10 * n + 8 + prepElems + 1) + CtaQPScratch<T>::bytes(n) + 16;
-}
-// Room for the samples of one problem (t and y, m values each) behind everything else?  m even keeps the TMA copies at
-// 16-byte granularity; the budget leaves at least two CTAs per SM for the small shapes this kernel usually sees.
-template <class T> unsigned cta_stage_m(size_t smemBase, unsigned m)
-{
-    const size_t need = 2 * (size_t)m * sizeof(T) + 32;
-    const bool ok = m > 0 && (m * sizeof(T)) % 16 == 0 && need <= 48 * 1024 && smemBase + need <= 200 * 1024;
-    return ok ? m : 0u;
-}
-
 // The per-CTA scratch (J, J^T J, two residual vectors) is sized by m n: keep the resident wave within a few GB, fewer CTAs
 // if need be (they are persistent and pull problems from a queue, so any grid size solves the batch).
 inline unsigned long long cta_cap_grid(unsigned long long grid, unsigned long long bytesPerCta)
@@ -609,41 +623,73 @@ inline unsigned long long cta_cap_grid(unsigned long long grid, unsigned long lo
     return grid;
 }
 
-template <class Model, class T, bool FD>
-int launch_cta_fd(const typename Num<T>::Settings& st, const SmallBatchArgs& args, size_t n, const mir_model_desc& model, cudaStream_t stream)
+// a kernel of this library, for launch_persistent (runtime API); `what` names the launch in its error
+struct RuntimeKernel {
+    const void* fn; const char* what;
+    int set_smem(size_t smem) const { return check_cuda(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem), "cudaFuncSetAttribute"); }
+    int occupancy(int* blocks, size_t smem) const { return check_cuda(cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks, fn, CTA_NT, smem), "cudaOccupancyMaxActiveBlocksPerMultiprocessor"); }
+    int launch(unsigned grid, size_t smem, cudaStream_t s, void** params) const
+    {
+        cudaLaunchKernel(fn, dim3(grid), dim3(CTA_NT), params, smem, s);
+        return check_cuda(cudaGetLastError(), what);
+    }
+};
+
+// Launch policy of the persistent-CTA kernels (lm_cta_kernel, lm_cov_cta_kernel; built in or compiled at run time): up to
+// 8 resident CTAs per SM, no more CTAs than problems, and `stride` elements of T of global scratch per CTA, freed in stream
+// order behind the kernel; its address goes to `scratch`, a field of the argument struct `params` points to.  `kern` makes
+// the calls that differ between the runtime API (RuntimeKernel) and the driver API (lm_nvrtc.cu): set_smem, occupancy
+// and launch, each returning MIR_B200_OK or an error code with the error set.
+template <class T, class K>
+int launch_persistent(const K& kern, size_t smem, const char* tooBig, unsigned long long batch, unsigned long long stride,
+                      void*& scratch, void** params, cudaStream_t stream)
 {
-    if (n > 128) { set_error("mir_optim_b200: the batched path supports n <= 128"); return MIR_B200_EUNSUPPORTED; }
-    if (!Model::valid((int)n, (int)args.m)) { set_error("mir_optim_b200: (m, n) not valid for this model"); return MIR_B200_EINVAL; }
-    auto kern = lm_cta_kernel<Model, T, FD>;
-    size_t smem = cta_smem_bytes<T>((int)n, Model::prep_elems((int)n));
-    const unsigned stageM = cta_stage_m<T>(smem, args.m);
-    smem += stageM ? 2 * (size_t)stageM * sizeof(T) + 32 : 0;
-    if (smem > 220 * 1024) { set_error("mir_optim_b200: n too large for the shared memory of the general batched kernel"); return MIR_B200_EUNSUPPORTED; }
-    MIRB200_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    if (smem > 220 * 1024) { set_error(tooBig); return MIR_B200_EUNSUPPORTED; }
+    if (int rc = kern.set_smem(smem)) return rc;
     int blocksPerSM = 0;
-    MIRB200_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocksPerSM, kern, CTA_NT, smem));
+    if (int rc = kern.occupancy(&blocksPerSM, smem)) return rc;
     if (blocksPerSM < 1) blocksPerSM = 1;
     if (blocksPerSM > 8) blocksPerSM = 8;
     unsigned long long grid = (unsigned long long)sm_count() * blocksPerSM;
-    if (args.batch < grid) grid = args.batch ? args.batch : 1;
-    CtaBatchArgs ca;
-    ca.b = args; ca.aux = model.aux; ca.param = model.param; ca.n = (unsigned)n; ca.stage_m = stageM;
-    ca.scratch_stride = (unsigned long long)args.m * n + (unsigned long long)n * n + 2ull * args.m + 4;
-    grid = cta_cap_grid(grid, ca.scratch_stride * sizeof(T));
-    T* scratch = nullptr;
-    MIRB200_CUDA(cudaMallocAsync((void**)&scratch, sizeof(T) * ca.scratch_stride * grid, stream));
-    ca.scratch = scratch;
-    kern<<<(unsigned)grid, CTA_NT, smem, stream>>>(st, ca);
+    if (batch < grid) grid = batch ? batch : 1;
+    grid = cta_cap_grid(grid, stride * sizeof(T));
+    T* buf = nullptr;
+    MIRB200_CUDA(cudaMallocAsync((void**)&buf, sizeof(T) * stride * grid, stream));
+    scratch = buf;
+    const int rc = kern.launch((unsigned)grid, smem, stream, params);
     count_launch();
-    const int rc = check_cuda(cudaGetLastError(), "lm_cta_kernel launch");
-    cudaFreeAsync(scratch, stream);
+    cudaFreeAsync(buf, stream);
     return rc;
 }
-template <class Model, class T>
-int launch_cta(const typename Num<T>::Settings& st, const SmallBatchArgs& args, size_t n, const mir_model_desc& model, cudaStream_t stream)
+
+// lm_cta_kernel (`kern`: built in or compiled at run time) over a batch.  One problem's samples (t and y, m values each) are
+// staged in shared memory behind everything else where there is room: m even keeps the TMA copies at 16-byte
+// granularity; the budget leaves at least two CTAs per SM for the small shapes this kernel usually sees.
+template <class T, class K>
+int launch_cta_fit(const K& kern, const typename Num<T>::Settings& st, const SmallBatchArgs& args, const mir_model_desc& model,
+                   size_t n, int prepElems, cudaStream_t stream)
 {
-    if ((args.flags & MIR_MODEL_FD_JACOBIAN) || !Model::kAnalytic) return launch_cta_fd<Model, T, true>(st, args, n, model, stream);
-    return launch_cta_fd<Model, T, false>(st, args, n, model, stream);
+    const size_t smem = sizeof(T) * (10 * n + 8 + prepElems + 1) + CtaQPScratch<T>::bytes((int)n) + 16;
+    const size_t stage = 2 * (size_t)args.m * sizeof(T) + 32;
+    const bool staged = args.m > 0 && (args.m * sizeof(T)) % 16 == 0 && stage <= 48 * 1024 && smem + stage <= 200 * 1024;
+    CtaBatchArgs ca;
+    ca.b = args; ca.aux = model.aux; ca.param = model.param; ca.n = (unsigned)n; ca.stage_m = staged ? args.m : 0u;
+    ca.scratch_stride = (unsigned long long)args.m * n + (unsigned long long)n * n + 2ull * args.m + 4;
+    void* params[] = {(void*)&st, &ca};
+    return launch_persistent<T>(kern, staged ? smem + stage : smem, "mir_optim_b200: n too large for the shared memory of the general batched kernel",
+                                args.batch, ca.scratch_stride, ca.scratch, params, stream);
+}
+
+// The built-in models of the persistent-CTA kernels: f(ModelTag<M>{}) with the lm_cta model M of model.model; EINVAL for a
+// spline without its knots, EUNSUPPORTED with the error `unknown` for an id without a model.
+template <class T, class F> int visit_cta_model(const mir_model_desc& model, const char* unknown, F&& f)
+{
+    if (model.model == MIR_MODEL_SPLINE) {
+        if (!model.aux) { set_error("mir_optim_b200: MIR_MODEL_SPLINE needs the knots in model->aux"); return MIR_B200_EINVAL; }
+        return f(ModelTag<CtaSpline<T>>{});
+    }
+    return visit_large_model<T>(model.model, [&](auto tag) { return f(ModelTag<CtaFromLarge<typename decltype(tag)::type, T>>{}); },
+                                [&] { set_error(unknown); return (int)MIR_B200_EUNSUPPORTED; });
 }
 
 // general batched path by model id; MIR_B200_EUNSUPPORTED if the model has no run-time-n functor

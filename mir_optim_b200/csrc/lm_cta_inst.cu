@@ -8,20 +8,14 @@ template <class T>
 int launch_cta_model(const mir_model_desc& model, size_t n, const typename Num<T>::Settings& st, const SmallBatchArgs& args, cudaStream_t stream)
 {
     if (model.model >= (uint32_t)MIR_MODEL_USER_BASE) return launch_user_model<T>(model, n, st, args, stream);
-    switch (model.model) {
-    case MIR_MODEL_EXPDECAY2: return launch_cta<CtaFromLarge<LModelExpDecay2<T>, T>, T>(st, args, n, model, stream);
-    case MIR_MODEL_EXPTAU3:   return launch_cta<CtaFromLarge<LModelExpTau3<T>, T>, T>(st, args, n, model, stream);
-    case MIR_MODEL_EXPDECAY3: return launch_cta<CtaFromLarge<LModelExpDecay3<T>, T>, T>(st, args, n, model, stream);
-    case MIR_MODEL_GAUSS4:    return launch_cta<CtaFromLarge<LModelGauss4<T>, T>, T>(st, args, n, model, stream);
-    case MIR_MODEL_SUMEXP:    return launch_cta<CtaFromLarge<LModelSumExp<T>, T>, T>(st, args, n, model, stream);
-    case MIR_MODEL_GAUSSMIX:  return launch_cta<CtaFromLarge<LModelGaussMix<T>, T>, T>(st, args, n, model, stream);
-    case MIR_MODEL_SPLINE:
-        if (!model.aux) { set_error("mir_optim_b200: MIR_MODEL_SPLINE needs the knots in model->aux"); return MIR_B200_EINVAL; }
-        return launch_cta<CtaSpline<T>, T>(st, args, n, model, stream);
-    default:
-        set_error("mir_optim_b200: model id not available in the batched path");
-        return MIR_B200_EUNSUPPORTED;
-    }
+    return visit_cta_model<T>(model, "mir_optim_b200: model id not available in the batched path", [&](auto tag) {
+        using M = typename decltype(tag)::type;
+        if (n > 128) { set_error("mir_optim_b200: the batched path supports n <= 128"); return (int)MIR_B200_EUNSUPPORTED; }
+        if (!M::valid((int)n, (int)args.m)) { set_error("mir_optim_b200: (m, n) not valid for this model"); return (int)MIR_B200_EINVAL; }
+        const bool fd = (args.flags & MIR_MODEL_FD_JACOBIAN) || !M::kAnalytic;
+        const RuntimeKernel kern{fd ? (const void*)lm_cta_kernel<M, T, true> : (const void*)lm_cta_kernel<M, T, false>, "lm_cta_kernel launch"};
+        return launch_cta_fit<T>(kern, st, args, model, n, M::prep_elems((int)n), stream);
+    });
 }
 template int launch_cta_model<double>(const mir_model_desc&, size_t, const Num<double>::Settings&, const SmallBatchArgs&, cudaStream_t);
 template int launch_cta_model<float>(const mir_model_desc&, size_t, const Num<float>::Settings&, const SmallBatchArgs&, cudaStream_t);

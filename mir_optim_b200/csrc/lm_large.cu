@@ -109,15 +109,8 @@ template <class Model, class T> LargeKernels<T> kernels_of()
 }
 template <class T> bool large_model_kernels(unsigned model, LargeKernels<T>& k)
 {
-    switch (model) {
-        case MIR_MODEL_GAUSSMIX:  k = kernels_of<LModelGaussMix<T>, T>(); return true;
-        case MIR_MODEL_SUMEXP:    k = kernels_of<LModelSumExp<T>, T>(); return true;
-        case MIR_MODEL_EXPDECAY3: k = kernels_of<LModelExpDecay3<T>, T>(); return true;
-        case MIR_MODEL_EXPDECAY2: k = kernels_of<LModelExpDecay2<T>, T>(); return true;
-        case MIR_MODEL_EXPTAU3:   k = kernels_of<LModelExpTau3<T>, T>(); return true;
-        case MIR_MODEL_GAUSS4:    k = kernels_of<LModelGauss4<T>, T>(); return true;
-        default: return false;
-    }
+    return visit_large_model<T>(model, [&](auto tag) { k = kernels_of<typename decltype(tag)::type, T>(); return true; },
+                                [] { return false; });
 }
 
 // argument validation, least_squares.d:930-943 (first failure wins).  Returns 0 when valid.

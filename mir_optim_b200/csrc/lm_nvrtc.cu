@@ -3,8 +3,9 @@
 // compiles `lm_cta_kernel<CtaUser<UserModel<T>, T>, T, FD>` (the general batched LM kernel, lm_cta.cuh, whose sources
 // are embedded in the library by embed_headers.py) with NVRTC for sm_100a, loads the cubin with the driver API and
 // caches the functions.  The covariance kernel (`lm_cov_cta_kernel`, lm_cov.cuh) is a separate program, compiled at
-// the first covariance call per precision, so registration does no extra work for it.  libnvrtc and libcuda are bound
-// with dlopen: the library has no link-time dependency on them.
+// the first covariance call per precision, so registration does no extra work for it.  Both launch with the policy of
+// the built-in kernels (launch_persistent, lm_cta.cuh), through the driver API.  libnvrtc and libcuda are bound with
+// dlopen: the library has no link-time dependency on them.
 #include <dlfcn.h>
 
 #include <cstring>
@@ -170,6 +171,18 @@ int get_compiled(uint32_t id, bool isFloat, Program prog, Compiled** out)
     return MIR_B200_OK;
 }
 
+// a kernel compiled at run time, for launch_persistent (lm_cta.cuh; driver API); `what` names the launch in its error
+struct DriverKernel {
+    void* fn; const char* what;
+    static int rc(int cr, const char* call) { return cr ? cu_fail(call, cr) : MIR_B200_OK; }
+    int set_smem(size_t smem) const { return rc(rtc().cuFuncSetAttribute(fn, 8 /* CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES */, (int)smem), "cuFuncSetAttribute"); }
+    int occupancy(int* blocks, size_t smem) const { return rc(rtc().cuOccupancy(blocks, fn, CTA_NT, smem), "cuOccupancyMaxActiveBlocksPerMultiprocessor"); }
+    int launch(unsigned grid, size_t smem, cudaStream_t s, void** params) const
+    {
+        return rc(rtc().cuLaunchKernel(fn, grid, 1, 1, CTA_NT, 1, 1, (unsigned)smem, s, params, nullptr), what);
+    }
+};
+
 }  // namespace
 
 template <class T>
@@ -177,37 +190,9 @@ int launch_user_model(const mir_model_desc& model, size_t n, const typename Num<
 {
     if (n > 128) { set_error("mir_optim_b200: the batched path supports n <= 128"); return MIR_B200_EUNSUPPORTED; }
     Compiled* c = nullptr;
-    int rc = get_compiled(model.model, sizeof(T) == 4, kProgLM, &c);
-    if (rc) return rc;
-    Rtc& r = rtc();
+    if (int rc = get_compiled(model.model, sizeof(T) == 4, kProgLM, &c)) return rc;
     void* fn = c->fn[(args.flags & MIR_MODEL_FD_JACOBIAN) ? 1 : 0];      // (a model without jacobian() runs finite differences either way)
-    size_t smem = cta_smem_bytes<T>((int)n, 1);
-    const unsigned stageM = cta_stage_m<T>(smem, args.m);
-    smem += stageM ? 2 * (size_t)stageM * sizeof(T) + 32 : 0;
-    if (smem > 220 * 1024) { set_error("mir_optim_b200: n too large for the shared memory of the general batched kernel"); return MIR_B200_EUNSUPPORTED; }
-    int cr = r.cuFuncSetAttribute(fn, 8 /* CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES */, (int)smem);
-    if (cr) return cu_fail("cuFuncSetAttribute", cr);
-    int blocksPerSM = 0;
-    cr = r.cuOccupancy(&blocksPerSM, fn, CTA_NT, smem);
-    if (cr) return cu_fail("cuOccupancyMaxActiveBlocksPerMultiprocessor", cr);
-    if (blocksPerSM < 1) blocksPerSM = 1;
-    if (blocksPerSM > 8) blocksPerSM = 8;
-    unsigned long long grid = (unsigned long long)sm_count() * blocksPerSM;
-    if (args.batch < grid) grid = args.batch ? args.batch : 1;
-    CtaBatchArgs ca;
-    ca.b = args; ca.aux = model.aux; ca.param = model.param; ca.n = (unsigned)n; ca.stage_m = stageM;
-    ca.scratch_stride = (unsigned long long)args.m * n + (unsigned long long)n * n + 2ull * args.m + 4;
-    grid = cta_cap_grid(grid, ca.scratch_stride * sizeof(T));
-    T* scratch = nullptr;
-    MIRB200_CUDA(cudaMallocAsync((void**)&scratch, sizeof(T) * ca.scratch_stride * grid, stream));
-    ca.scratch = scratch;
-    typename Num<T>::Settings stc = st;
-    void* params[] = {&stc, &ca};
-    cr = r.cuLaunchKernel(fn, (unsigned)grid, 1, 1, CTA_NT, 1, 1, (unsigned)smem, stream, params, nullptr);
-    count_launch();
-    cudaFreeAsync(scratch, stream);
-    if (cr) return cu_fail("cuLaunchKernel (user model)", cr);
-    return MIR_B200_OK;
+    return launch_cta_fit<T>(DriverKernel{fn, "cuLaunchKernel (user model)"}, st, args, model, n, 1, stream);
 }
 template int launch_user_model<double>(const mir_model_desc&, size_t, const Num<double>::Settings&, const SmallBatchArgs&, cudaStream_t);
 template int launch_user_model<float>(const mir_model_desc&, size_t, const Num<float>::Settings&, const SmallBatchArgs&, cudaStream_t);
@@ -216,32 +201,9 @@ template <class T>
 int launch_user_cov(const mir_model_desc& model, T jacEps, CovArgs ca, cudaStream_t stream)
 {
     Compiled* c = nullptr;
-    int rc = get_compiled(model.model, sizeof(T) == 4, kProgCov, &c);
-    if (rc) return rc;
-    Rtc& r = rtc();
+    if (int rc = get_compiled(model.model, sizeof(T) == 4, kProgCov, &c)) return rc;
     void* fn = c->fn[(model.flags & MIR_MODEL_FD_JACOBIAN) ? 1 : 0];      // (a model without jacobian() runs finite differences either way)
-    const size_t smem = cov_smem_bytes<T>((int)ca.n, 1);
-    if (smem > kCovSmemLimit) { set_error("mir_optim_b200: n too large for the shared memory of the covariance kernel"); return MIR_B200_EUNSUPPORTED; }
-    int cr = r.cuFuncSetAttribute(fn, 8 /* CU_FUNC_ATTRIBUTE_MAX_DYNAMIC_SHARED_SIZE_BYTES */, (int)smem);
-    if (cr) return cu_fail("cuFuncSetAttribute", cr);
-    int blocksPerSM = 0;
-    cr = r.cuOccupancy(&blocksPerSM, fn, CTA_NT, smem);
-    if (cr) return cu_fail("cuOccupancyMaxActiveBlocksPerMultiprocessor", cr);
-    if (blocksPerSM < 1) blocksPerSM = 1;
-    if (blocksPerSM > 8) blocksPerSM = 8;
-    unsigned long long grid = (unsigned long long)sm_count() * blocksPerSM;
-    if (ca.batch < grid) grid = ca.batch;
-    ca.scratch_stride = (unsigned long long)ca.m * ca.n + ca.m + 2;
-    grid = cta_cap_grid(grid, ca.scratch_stride * sizeof(T));
-    T* scratch = nullptr;
-    MIRB200_CUDA(cudaMallocAsync((void**)&scratch, sizeof(T) * ca.scratch_stride * grid, stream));
-    ca.scratch = scratch;
-    void* params[] = {&jacEps, &ca};
-    cr = r.cuLaunchKernel(fn, (unsigned)grid, 1, 1, CTA_NT, 1, 1, (unsigned)smem, stream, params, nullptr);
-    count_launch();
-    cudaFreeAsync(scratch, stream);
-    if (cr) return cu_fail("cuLaunchKernel (user model covariance)", cr);
-    return MIR_B200_OK;
+    return launch_cov<T>(DriverKernel{fn, "cuLaunchKernel (user model covariance)"}, jacEps, ca, 1, stream);
 }
 template int launch_user_cov<double>(const mir_model_desc&, double, CovArgs, cudaStream_t);
 template int launch_user_cov<float>(const mir_model_desc&, float, CovArgs, cudaStream_t);

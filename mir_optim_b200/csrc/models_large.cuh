@@ -132,4 +132,22 @@ template <class T> struct LModelGauss4 {
     }
 };
 
+#ifndef __CUDACC_RTC__
+template <class M> struct ModelTag { using type = M; };
+
+// The functor of a model id: f(ModelTag<L>{}) for the ids above, otherwise() for every other id.
+template <class T, class F, class G> auto visit_large_model(unsigned id, F&& f, G&& otherwise)
+{
+    switch (id) {
+    case MIR_MODEL_EXPDECAY2: return f(ModelTag<LModelExpDecay2<T>>{});
+    case MIR_MODEL_EXPTAU3:   return f(ModelTag<LModelExpTau3<T>>{});
+    case MIR_MODEL_EXPDECAY3: return f(ModelTag<LModelExpDecay3<T>>{});
+    case MIR_MODEL_GAUSS4:    return f(ModelTag<LModelGauss4<T>>{});
+    case MIR_MODEL_SUMEXP:    return f(ModelTag<LModelSumExp<T>>{});
+    case MIR_MODEL_GAUSSMIX:  return f(ModelTag<LModelGaussMix<T>>{});
+    default:                  return otherwise();
+    }
+}
+#endif
+
 }  // namespace mirb200

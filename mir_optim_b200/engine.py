@@ -37,6 +37,23 @@ def _vp(a):
     return C.c_void_p(a.data_ptr())      # torch tensor
 
 
+def _model_desc(model, x, t, y, m, aux, param, fd_jacobian):
+    """(m, ModelDesc) of a batched call on x (batch, n): the model id and constants (aux, param), its samples t and y (or m
+    for a model without samples) and the flags they imply.  numpy inputs are converted to x's dtype, and the desc holds
+    the converted arrays; torch tensors are passed as they are."""
+    if isinstance(x, np.ndarray):
+        t, y, aux = (None if a is None else np.ascontiguousarray(a, dtype=x.dtype) for a in (t, y, aux))
+        assert y is None or y.shape[0] == x.shape[0]
+    if y is not None and m is None:
+        m = y.shape[1]
+    assert m is not None, "m is required for models without samples"
+    flags = ((MODEL_FD_JACOBIAN if fd_jacobian else 0) | (MODEL_GRID_PER_PROBLEM if t is not None and t.ndim == 2 else 0)
+             | (_abi.MODEL_AUX_PER_PROBLEM if aux is not None and aux.ndim == 2 else 0))
+    desc = ModelDesc(int(model), flags, _vp(t), _vp(y), _vp(aux), float(param))
+    desc.arrays = (t, y, aux)
+    return m, desc
+
+
 class Engine(ReferenceAPI):
     def __init__(self, lib):
         super().__init__(lib)
@@ -68,23 +85,11 @@ class Engine(ReferenceAPI):
         batch, n = x.shape
         l = np.ascontiguousarray(l, dtype=x.dtype); u = np.ascontiguousarray(u, dtype=x.dtype)
         bound_stride = 0 if l.ndim == 1 else n
-        flags = (MODEL_FD_JACOBIAN if fd_jacobian else 0) | (0 if tail_shortcut else MODEL_NO_TAIL_SHORTCUT)
-        if y is not None:
-            y = np.ascontiguousarray(y, dtype=x.dtype); assert y.shape[0] == batch
-            m = y.shape[1] if m is None else m
-        if t is not None:
-            t = np.ascontiguousarray(t, dtype=x.dtype)
-            if t.ndim == 2:
-                flags |= MODEL_GRID_PER_PROBLEM
-        assert m is not None, "m is required for data-free models"
-        if aux is not None:
-            aux = np.ascontiguousarray(aux, dtype=x.dtype)
-            if aux.ndim == 2:
-                flags |= _abi.MODEL_AUX_PER_PROBLEM
+        m, desc = _model_desc(model, x, t, y, m, aux, param, fd_jacobian)
+        desc.flags |= 0 if tail_shortcut else MODEL_NO_TAIL_SHORTCUT
         if warm_start:
             assert results is not None, "warm_start reads results['lambda'] of a previous call"
-            flags |= _abi.MODEL_WARM_START
-        desc = ModelDesc(int(model), flags, _vp(t), _vp(y), _vp(aux), float(param))
+            desc.flags |= _abi.MODEL_WARM_START
         if results is None:
             results = np.empty(batch, dtype=RESULT_DTYPES[x.dtype])
         assert results.dtype == RESULT_DTYPES[x.dtype] and results.shape == (batch,) and results.flags.c_contiguous
@@ -109,19 +114,13 @@ class Engine(ReferenceAPI):
         assert isinstance(settings, S) and x.is_cuda and x.is_contiguous()
         batch, n = x.shape
         bound_stride = 0 if l.dim() == 1 else n
-        flags = (MODEL_FD_JACOBIAN if fd_jacobian else 0) | (0 if tail_shortcut else MODEL_NO_TAIL_SHORTCUT)
-        if y is not None:
-            m = y.shape[1] if m is None else m
-        if t is not None and t.dim() == 2:
-            flags |= MODEL_GRID_PER_PROBLEM
-        if aux is not None and aux.dim() == 2:
-            flags |= _abi.MODEL_AUX_PER_PROBLEM
+        m, desc = _model_desc(model, x, t, y, m, aux, param, fd_jacobian)
+        desc.flags |= 0 if tail_shortcut else MODEL_NO_TAIL_SHORTCUT
         if warm_start:
             assert results is not None, "warm_start reads the lambda of a previous call's results"
-            flags |= _abi.MODEL_WARM_START
+            desc.flags |= _abi.MODEL_WARM_START
         if results is None:
             results = torch.empty(batch * RESULT_DTYPES[dt].itemsize, dtype=torch.uint8, device=x.device)
-        desc = ModelDesc(int(model), flags, _vp(t), _vp(y), _vp(aux), float(param))
         if stream is None:
             stream = torch.cuda.current_stream(x.device).cuda_stream
         fn = getattr(self.lib, f"mir_optimize_least_squares_batched_dev_{sfx}")
@@ -147,20 +146,7 @@ class Engine(ReferenceAPI):
         batch, n = x.shape
         l = np.ascontiguousarray(l, dtype=x.dtype); u = np.ascontiguousarray(u, dtype=x.dtype)
         bound_stride = 0 if l.ndim == 1 else n
-        flags = MODEL_FD_JACOBIAN if fd_jacobian else 0
-        if y is not None:
-            y = np.ascontiguousarray(y, dtype=x.dtype); assert y.shape[0] == batch
-            m = y.shape[1] if m is None else m
-        if t is not None:
-            t = np.ascontiguousarray(t, dtype=x.dtype)
-            if t.ndim == 2:
-                flags |= MODEL_GRID_PER_PROBLEM
-        assert m is not None, "m is required for models without samples"
-        if aux is not None:
-            aux = np.ascontiguousarray(aux, dtype=x.dtype)
-            if aux.ndim == 2:
-                flags |= _abi.MODEL_AUX_PER_PROBLEM
-        desc = ModelDesc(int(model), flags, _vp(t), _vp(y), _vp(aux), float(param))
+        m, desc = _model_desc(model, x, t, y, m, aux, param, fd_jacobian)
         cov = np.empty((batch, n, n), dtype=x.dtype) if want_cov else None
         stddev = np.empty((batch, n), dtype=x.dtype)
         info = np.empty(batch, dtype=np.int32)
@@ -181,21 +167,13 @@ class Engine(ReferenceAPI):
         assert (settings is None or isinstance(settings, S)) and x.is_cuda and x.is_contiguous()
         batch, n = x.shape
         bound_stride = 0 if l.dim() == 1 else n
-        flags = MODEL_FD_JACOBIAN if fd_jacobian else 0
-        if y is not None:
-            m = y.shape[1] if m is None else m
-        if t is not None and t.dim() == 2:
-            flags |= MODEL_GRID_PER_PROBLEM
-        if aux is not None and aux.dim() == 2:
-            flags |= _abi.MODEL_AUX_PER_PROBLEM
-        assert m is not None, "m is required for models without samples"
+        m, desc = _model_desc(model, x, t, y, m, aux, param, fd_jacobian)
         if cov is None and want_cov:
             cov = torch.empty((batch, n, n), dtype=x.dtype, device=x.device)
         if stddev is None:
             stddev = torch.empty((batch, n), dtype=x.dtype, device=x.device)
         if info is None:
             info = torch.empty(batch, dtype=torch.int32, device=x.device)
-        desc = ModelDesc(int(model), flags, _vp(t), _vp(y), _vp(aux), float(param))
         if stream is None:
             stream = torch.cuda.current_stream(x.device).cuda_stream
         fn = getattr(self.lib, f"mir_b200_covariance_batched_dev_{sfx}")

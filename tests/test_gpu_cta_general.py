@@ -116,6 +116,29 @@ def test_largest_and_smallest_n(eng, oracle_lib):
     assert np.array_equal(rg["status"], ro["status"]) and np.array_equal(rg["fCalls"], ro["fCalls"]) and np.max(rel_err(xg, xo)) < 1e-11
 
 
+@pytest.mark.parametrize("dtype", [np.float64, np.float32])
+@pytest.mark.parametrize("fd", [False, True])
+def test_argument_errors_of_the_general_path(eng, dtype, fd):
+    """What the fit returns for shapes and models the general kernel cannot run: 3 (MIR_B200_EUNSUPPORTED) for n > 128 and
+    for an id without a run-time-n functor, 2 (MIR_B200_EINVAL) for a spline without knots, an (m, n) the model does not
+    accept and an unknown user model."""
+    from mir_optim_b200 import B200Error
+    m = 32
+
+    def code(model, n, data=True):
+        x = np.ones((2, n), dtype); l = np.full(n, -np.inf, dtype); u = np.full(n, np.inf, dtype)
+        t = np.linspace(0.0, 1.0, m, dtype=dtype) if data else None
+        y = np.zeros((2, m), dtype) if data else None
+        with pytest.raises(B200Error) as e:
+            eng.optimize_batched(eng.settings(dtype), model, x, l, u, t=t, y=y, m=m, fd_jacobian=fd)
+        return e.value.code
+    assert code(ModelId.GAUSSMIX, 129) == 3
+    assert code(ModelId.SPLINE, 4) == 2
+    assert code(ModelId.GAUSS4, 5) == 2
+    assert code(ModelId.LINEAR2, 3, data=False) == 3
+    assert code(0x1000 + 99999, 4, data=False) == 2
+
+
 @pytest.mark.parametrize("n", [2, 3, 4])
 def test_fit_spline_few_knots(eng, oracle_lib, n):
     """Two knots (a line), three (the parabola of the not-a-knot condition) and four (the first general case)."""
