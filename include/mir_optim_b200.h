@@ -486,6 +486,16 @@ int mir_b200_posvx_batched_d(int variant, size_t batch, size_t n, const double* 
 int mir_b200_posvx_batched_s(int variant, size_t batch, size_t n, const float* A, const float* b, float* x,
                              int32_t* info, int32_t* equed, int device);
 
+/* Diagnostics: the device math under every residual functor and the mux kernel's Cholesky, on its own, for unit tests
+ * against the host restatement oracle/repro_math.h (bit for bit) and a high-precision reference.  y[i] = f(x[i]) for
+ * i < n.  variant 0: exp_repro_tp (early returns; the large-problem evaluators and user models); 1: exp_repro (out of
+ * line); 2: exp_repro_inl; 3 / 4: exp_repro_many<K>, K = 4 / 16, each thread taking K consecutive inputs; 5 / 6:
+ * exp_repro_many_conv<K>, K = 4 / 16, each warp taking 32*K consecutive inputs (its fast path runs when all of them have
+ * |x| < 700, |x| < 80 in float; past the end of x the warp is padded with 0); 7: mux_sqrt_rcp, sqrt(x) to y and
+ * 1/sqrt(x) to y2 (y2 is ignored by the other variants).  Host pointers, synchronous. */
+int mir_b200_math_hook_d(int variant, size_t n, const double* x, double* y, double* y2, int device);
+int mir_b200_math_hook_s(int variant, size_t n, const float* x, float* y, float* y2, int device);
+
 /* NCCL bootstrap helpers so that a host runtime without NCCL bindings (ctypes, D) can build the
  * communicator: rank 0 calls get_unique_id (128 bytes), shares it by any means, all call init. */
 int  mir_b200_nccl_unique_id(void* id128);

@@ -142,6 +142,7 @@ B200_SYMBOLS = [
     "mir_solve_box_qp_batched_dev_d", "mir_solve_box_qp_batched_dev_s",
     "mir_optimize_least_squares_sharded_d", "mir_b200_syrk_lower_dev_d",
     "mir_b200_posvx_batched_d", "mir_b200_posvx_batched_s",
+    "mir_b200_math_hook_d", "mir_b200_math_hook_s",
     "mir_b200_nccl_unique_id", "mir_b200_nccl_comm_init", "mir_b200_nccl_comm_destroy",
     "mir_fit_spline_d", "mir_fit_spline_s", "mir_fit_spline_batched_d", "mir_fit_spline_batched_s",
     "mir_b200_model_compile", "mir_b200_model_release",
@@ -205,6 +206,8 @@ def bind_b200_abi(lib):
     for sfx in ("d", "s"):
         fn = getattr(lib, f"mir_b200_posvx_batched_{sfx}")
         fn.argtypes = [C.c_int, C.c_size_t, C.c_size_t, vp, vp, vp, vp, vp, C.c_int]; fn.restype = C.c_int
+        fn = getattr(lib, f"mir_b200_math_hook_{sfx}")
+        fn.argtypes = [C.c_int, C.c_size_t, vp, vp, vp, C.c_int]; fn.restype = C.c_int
     for sfx, S, R, real in (("d", LeastSquaresSettingsD, LeastSquaresResultD, C.c_double), ("s", LeastSquaresSettingsS, LeastSquaresResultS, C.c_float)):
         fn = getattr(lib, f"mir_fit_spline_{sfx}")
         fn.argtypes = [C.POINTER(S), C.c_size_t, vp, vp, C.c_size_t, vp, vp, vp, real, vp, C.POINTER(R)]; fn.restype = C.c_int

@@ -274,6 +274,18 @@ class Engine(ReferenceAPI):
         self._check(getattr(self.lib, f"mir_b200_posvx_batched_{sfx}")(variant, batch, n, _vp(A), _vp(b), _vp(x), _vp(info), _vp(equed), device))
         return x, info, equed
 
+    def math_hook(self, x: np.ndarray, variant: int, device: int = -1):
+        """Diagnostics: one device form of the reproducible exp (variants 0-6) or the mux Cholesky pivot step (variant 7)
+        applied elementwise to x (1-d, float64 or float32).  Returns y, or (sqrt(x), 1/sqrt(x)) for variant 7.  The
+        variants are listed in the header."""
+        sfx = _types(x.dtype)[0]
+        x = np.ascontiguousarray(x)
+        assert x.ndim == 1
+        y = np.empty_like(x)
+        y2 = np.empty_like(x) if variant == 7 else None
+        self._check(getattr(self.lib, f"mir_b200_math_hook_{sfx}")(variant, x.size, _vp(x), _vp(y), _vp(y2), device))
+        return (y, y2) if variant == 7 else y
+
     # -- one problem through the reference's own entry point, residual model on the device ------
     def optimize_device_model(self, settings, model: ModelId, x: np.ndarray, l: np.ndarray, u: np.ndarray,
                               t: np.ndarray | None = None, y: np.ndarray | None = None, m: int | None = None,

@@ -313,6 +313,18 @@ void oracle_model_g_d(void* c, size_t m, size_t n, const double* x, double* J) {
 void oracle_model_f_s(void* c, size_t m, size_t n, const float* x, float* y)   { model_f<float>(c, m, n, x, y); }
 void oracle_model_g_s(void* c, size_t m, size_t n, const float* x, float* J)   { model_g<float>(c, m, n, x, J); }
 
+/* The restated exp alone (unit tests: against decimal, and every device form of it bit for bit): y[i] = exp_repro(x[i]). */
+void oracle_exp_repro_d(size_t n, const double* x, double* y)
+{
+#pragma omp parallel for schedule(static) if (n >= 65536)
+    for (long long i = 0; i < (long long)n; ++i) y[i] = exp_repro(x[i]);
+}
+void oracle_exp_repro_s(size_t n, const float* x, float* y)
+{
+#pragma omp parallel for schedule(static) if (n >= 65536)
+    for (long long i = 0; i < (long long)n; ++i) y[i] = exp_repro(x[i]);
+}
+
 /* The restated spline alone (unit tests: against scipy's not-a-knot CubicSpline): values and first derivatives at t[0..nt). */
 void oracle_spline_eval_d(size_t n, const double* knots, const double* values, size_t nt, const double* t, double* out_v, double* out_d)
 {
