@@ -251,10 +251,12 @@ enum {
     MIR_MODEL_NO_TAIL_SHORTCUT = 4u,  /* verification only: execute every pass of the lambda-overflow tail
                                          instead of fast-forwarding it (results are identical, DESIGN.md 4.3) */
     MIR_MODEL_AUX_PER_PROBLEM  = 8u,  /* aux has batch*n entries instead of n shared ones                   */
-    MIR_MODEL_WARM_START       = 16u  /* batched entries: results[b].lambda on entry (> 0, finite) is the initial
+    MIR_MODEL_WARM_START       = 16u, /* batched entries: results[b].lambda on entry (> 0, finite) is the initial
                                          damping instead of 0 (LS:966); the reference documents Result.lambda as
                                          the initial trust-region value (LS:141-142) but never reads it back.
                                          Chain it with the x of a previous call to continue a fit.            */
+    MIR_MODEL_WEIGHTED         = 32u  /* per-observation weights in model->w (an extension; the reference has none):
+                                         every row's residual and Jacobian row are scaled by w_i, see mir_model_desc */
 };
 
 typedef struct mir_model_desc {
@@ -264,7 +266,25 @@ typedef struct mir_model_desc {
     const void* y;       /* observations, T[batch*m]; NULL for data-free models             */
     const void* aux;     /* model constants, T[n] (shared) or T[batch*n]: the knots of MIR_MODEL_SPLINE; else NULL */
     double      param;   /* model constant: the smoothing weight lambda of MIR_MODEL_SPLINE; else 0  */
-} mir_model_desc;
+    const void* w;       /* observation weights, T[batch*m], row-aligned with y; used only with MIR_MODEL_WEIGHTED */
+} mir_model_desc;                              /* 48 bytes (40 before w was added: the library copies the whole
+                                                  struct, so binaries built against the older header must be rebuilt) */
+
+/*
+ * Weighted least squares (MIR_MODEL_WEIGHTED).  For every row i < m of a problem the solver sees
+ *     r~_i = w_i * r_i(p)        (rounded once in T)
+ *     J~_ij = w_i * J_ij         (analytic Jacobian, each entry rounded once); the finite-difference Jacobian is the
+ *                                reference's central difference (LS:1016-1050, with the bound clamp) taken of r~
+ * and everything downstream -- the LM loop, Result.residual = sum r~_i^2 (chi^2 with w = 1/sigma), the g-test, J^T J, the
+ * covariance -- is exactly the reference run with f = w (.) r.  w follows y: host pointer in the host forms, device
+ * pointer in the _dev_ forms.  Values are the caller's contract, like y: w_i = 0 removes row i (pad short problems of a
+ * ragged batch to a common m with zero weights; the padded rows' residuals must still be finite, since 0 * inf is NaN),
+ * and a non-finite weight acts like a non-finite observation.
+ * Honoured by mir_optimize_least_squares_batched_{d,s} / _dev_{d,s} and mir_b200_covariance_batched_{d,s} / _dev_{d,s}
+ * (with any of the other flags); weighted fits always run the general batched kernel (lm_cta.cuh).  MIR_B200_EINVAL
+ * for w == NULL (batch > 0, m > 0); MIR_B200_EUNSUPPORTED for the data-free models LINEAR2, ROSENBROCK and SQRTCIRCLE
+ * and from mir_optimize_least_squares_sharded_d.  The legacy entry points in device-model mode return numericError.
+ */
 
 /*
  * User-defined residual models on the device (the reference takes arbitrary f / g, LS:78-80; SURVEY 8f-2).  `source`
@@ -358,19 +378,22 @@ int mir_optimize_least_squares_batched_dev_s(
  *   matrix     double).
  *   Inverse    S = D^-1/2 A D^-1/2 with D = diag(A); the Cholesky factor of S is inverted (LAPACK ?potrf + ?potri
  *              semantics) and unscaled.  A zero diagonal entry of A, or a pivot <= 0 or NaN, stops the factorisation.
- *   Scale      s^2 = ||r||^2 / (m - n_F); with MIR_COV_UNSCALED (residuals already divided by sigma; scipy's
- *              absolute_sigma=True) s^2 = 1.
+ *   Scale      s^2 = ||r||^2 / (m - n_F); with MIR_COV_UNSCALED s^2 = 1.  With MIR_MODEL_WEIGHTED, r and J are the
+ *              weighted r~ and J~, and m counts only the rows with w_i != 0 (m_w), so a problem padded with zero
+ *              weights has the covariance of the unpadded one.  With w = 1/sigma, MIR_COV_UNSCALED is scipy's
+ *              curve_fit(sigma=..., absolute_sigma=True) and the scaled form is absolute_sigma=False.
  *   Outputs    cov = s^2 A^-1 on F x F; rows and columns of fixed parameters are exactly 0.  Both triangles are written
  *              and are exactly symmetric (the lower triangle is computed and mirrored).  stddev_i = sqrt(cov_ii).
  *              Everything is computed in double and rounded once to T.
  *   info[b]    0   OK, including n_F = 0 (cov all zeros)
  *              k>0 the factorisation broke down at the pivot of parameter k-1 (1-based, original numbering); free block NaN
- *              -1  m <= n_F and scaled; free block +inf, as in scipy
+ *              -1  m <= n_F (m_w <= n_F when weighted) and scaled; free block +inf, as in scipy
  *              -2  a residual, a Jacobian entry or an x_i is not finite; free block NaN
  *              (checked in the order -2, -1, k).
  *
  * Model data as in the batched LM entries: t shared or MIR_MODEL_GRID_PER_PROBLEM, y, aux shared or
- * MIR_MODEL_AUX_PER_PROBLEM, param, l / u shared (bound_stride == 0) or T[batch*bound_stride], MIR_MODEL_FD_JACOBIAN;
+ * MIR_MODEL_AUX_PER_PROBLEM, param, w with MIR_MODEL_WEIGHTED, l / u shared (bound_stride == 0) or T[batch*bound_stride],
+ * MIR_MODEL_FD_JACOBIAN;
  * MIR_MODEL_WARM_START and MIR_MODEL_NO_TAIL_SHORTCUT are ignored.  settings may be NULL (defaults); only
  * jacobianEpsilon is read.  User models (mir_b200_model_compile) are compiled for the covariance at their first
  * covariance call per precision.

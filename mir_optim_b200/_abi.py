@@ -54,6 +54,7 @@ MODEL_GRID_PER_PROBLEM = 2
 MODEL_NO_TAIL_SHORTCUT = 4
 MODEL_AUX_PER_PROBLEM = 8
 MODEL_WARM_START = 16
+MODEL_WEIGHTED = 32
 COV_UNSCALED = 1
 
 
@@ -103,7 +104,7 @@ class LSTask(C.Structure):
 
 class ModelDesc(C.Structure):
     _fields_ = [("model", C.c_uint32), ("flags", C.c_uint32), ("t", C.c_void_p), ("y", C.c_void_p),
-                ("aux", C.c_void_p), ("param", C.c_double)]
+                ("aux", C.c_void_p), ("param", C.c_double), ("w", C.c_void_p)]
 
 
 class BatchStats(C.Structure):

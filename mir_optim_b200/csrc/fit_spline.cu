@@ -30,7 +30,7 @@ static int fit_spline(const typename Num<T>::Settings* settings, size_t batch, s
     if (batch == 0) return MIR_B200_OK;
     const bool per = (flags & MIR_MODEL_GRID_PER_PROBLEM) != 0;
     const size_t m = points + (lambda == (T)0 ? 1 : 0);
-    mir_model_desc d;
+    mir_model_desc d{};
     d.model = MIR_MODEL_SPLINE;
     d.flags = MIR_MODEL_FD_JACOBIAN | (flags & (MIR_MODEL_GRID_PER_PROBLEM | MIR_MODEL_AUX_PER_PROBLEM | MIR_MODEL_NO_TAIL_SHORTCUT));
     d.aux = knots; d.param = (double)lambda;

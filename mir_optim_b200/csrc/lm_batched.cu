@@ -19,9 +19,13 @@ namespace mirb200 {
 
 // Models that read samples need both arrays (t: m or batch*m abscissae, y: batch*m observations -- the lengths are the
 // caller's contract, stated in the header); only LINEAR2, ROSENBROCK and SQRTCIRCLE are data-free.
+static bool model_data_free(unsigned model)
+{
+    return model == MIR_MODEL_LINEAR2 || model == MIR_MODEL_ROSENBROCK || model == MIR_MODEL_SQRTCIRCLE;
+}
 static bool model_needs_data(unsigned model)
 {
-    return !(model == MIR_MODEL_LINEAR2 || model == MIR_MODEL_ROSENBROCK || model == MIR_MODEL_SQRTCIRCLE || model >= (unsigned)MIR_MODEL_USER_BASE);
+    return !(model_data_free(model) || model >= (unsigned)MIR_MODEL_USER_BASE);
 }
 // Shapes the specialised kernels (lm_tpp / lm_mux / lm_small) instantiate; everything else goes to the general kernel.
 static bool specialised_shape(unsigned model, size_t n)
@@ -34,12 +38,19 @@ static bool specialised_shape(unsigned model, size_t n)
     default: return false;
     }
 }
-// the samples check of the batched fit and of the covariance (lm_cov.cu)
+// the samples and weights check of the batched fit and of the covariance (lm_cov.cu)
 int check_model_data(const mir_model_desc* model, size_t batch, size_t m)
 {
     if (batch && m && model_needs_data(model->model) && (!model->t || !model->y)) {
         set_error("mir_optim_b200: this model reads samples: model->t and model->y must not be NULL");
         return MIR_B200_EINVAL;
+    }
+    if (model->flags & MIR_MODEL_WEIGHTED) {
+        if (model_data_free(model->model)) {
+            set_error("mir_optim_b200: MIR_MODEL_WEIGHTED needs a model with observation rows (not LINEAR2, ROSENBROCK or SQRTCIRCLE)");
+            return MIR_B200_EUNSUPPORTED;
+        }
+        if (batch && m && !model->w) { set_error("mir_optim_b200: MIR_MODEL_WEIGHTED: model->w must not be NULL"); return MIR_B200_EINVAL; }
     }
     return MIR_B200_OK;
 }
@@ -68,7 +79,8 @@ static int batched_dev(const typename Num<T>::Settings* settings, const mir_mode
     a.counter = counter; a.ready = ready; a.spin_limit = spinLimit; a.stats = stats; a.batch = batch; a.m = (unsigned)m;
     a.bound_stride = (unsigned)bound_stride; a.flags = model->flags;
     static const bool forceGeneral = [] { const char* e = std::getenv("MIRB200_BATCH_KERNEL"); return e && !std::strcmp(e, "cta"); }();   // tests / experiments
-    if (specialised_shape(model->model, n) && !forceGeneral) {
+    // weights are an adapter of the general kernel's models (CtaWeighted): the specialised kernels never see them
+    if (specialised_shape(model->model, n) && !forceGeneral && !(model->flags & MIR_MODEL_WEIGHTED)) {
         rc = launch_small_model<T>(model->model, n, *settings, a, stream);
         // a shape the specialised kernels do not cover after all (m beyond their rows-per-lane instantiations): general kernel
         if (rc == MIR_B200_EUNSUPPORTED && model_needs_data(model->model) && batch > 1) { clear_error(); rc = launch_cta_model<T>(*model, n, *settings, a, stream); }
@@ -109,6 +121,7 @@ static int batched_host(const typename Num<T>::Settings* settings, const mir_mod
     const bool per = (model->flags & MIR_MODEL_GRID_PER_PROBLEM) != 0;
     const size_t tBytes = model->t ? sizeof(T) * (per ? batch * m : m) : 0;
     const size_t yBytes = model->y ? sizeof(T) * batch * m : 0;
+    const size_t wBytes = (model->flags & MIR_MODEL_WEIGHTED) ? sizeof(T) * batch * m : 0;
     const size_t xBytes = sizeof(T) * batch * n;
     const size_t bBytes = sizeof(T) * (bound_stride ? batch * bound_stride : n);
     const size_t rBytes = sizeof(Result) * batch;
@@ -154,7 +167,8 @@ static int batched_host(const typename Num<T>::Settings* settings, const mir_mod
     *h_flag = 0;
 
     auto align = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    const size_t total = align(tBytes) + align(yBytes) + align(xBytes) + 2 * align(bBytes) + align(rBytes) + align(sizeof(mir_batch_stats)) + align(aBytes) + 256;
+    const size_t total = align(tBytes) + align(yBytes) + align(xBytes) + 2 * align(bBytes) + align(rBytes) + align(sizeof(mir_batch_stats)) + align(aBytes) + 256
+                         + align(wBytes);
     char* base = nullptr;
     cudaError_t e = cudaMallocAsync((void**)&base, total, cs);
     if (e != cudaSuccess) { cleanup(); return check_cuda(e, "cudaMallocAsync(batch buffers)"); }
@@ -167,7 +181,8 @@ static int batched_host(const typename Num<T>::Settings* settings, const mir_mod
     Result* dr = (Result*)p; p += align(rBytes);
     mir_batch_stats* ds = (mir_batch_stats*)p; p += align(sizeof(mir_batch_stats));
     T* da = (T*)p; p += align(aBytes);
-    unsigned int* d_ready = (unsigned int*)p;                     // {watermark, time-out flag}
+    unsigned int* d_ready = (unsigned int*)p; p += 256;           // {watermark, time-out flag}
+    T* dw = (T*)p;
 
     // shared inputs, counters and the watermark (0 = nothing staged) on the compute stream; the copy stream starts behind them
     if (tBytes && !per) CK(cudaMemcpyAsync(dt, model->t, tBytes, cudaMemcpyHostToDevice, cs), "H2D t");
@@ -186,6 +201,7 @@ static int batched_host(const typename Num<T>::Settings* settings, const mir_mod
         const size_t nb = (lo + chunk <= batch) ? chunk : batch - lo;
         if (tBytes && per) CK(cudaMemcpyAsync(dt + lo * m, static_cast<const T*>(model->t) + lo * m, sizeof(T) * nb * m, cudaMemcpyHostToDevice, ps), "H2D t");
         if (yBytes) CK(cudaMemcpyAsync(dy + lo * m, static_cast<const T*>(model->y) + lo * m, sizeof(T) * nb * m, cudaMemcpyHostToDevice, ps), "H2D y");
+        if (wBytes) CK(cudaMemcpyAsync(dw + lo * m, static_cast<const T*>(model->w) + lo * m, sizeof(T) * nb * m, cudaMemcpyHostToDevice, ps), "H2D w");
         CK(cudaMemcpyAsync(dx + lo * n, x + lo * n, sizeof(T) * nb * n, cudaMemcpyHostToDevice, ps), "H2D x");
         if (model->flags & MIR_MODEL_WARM_START) CK(cudaMemcpyAsync(dr + lo, results + lo, sizeof(Result) * nb, cudaMemcpyHostToDevice, ps), "H2D results (warm start)");
         if (bound_stride) {
@@ -200,7 +216,7 @@ static int batched_host(const typename Num<T>::Settings* settings, const mir_mod
     }
     auto launch = [&](const unsigned int* ready) {
         mir_model_desc dm = *model;
-        dm.t = tBytes ? dt : nullptr; dm.y = yBytes ? dy : nullptr; dm.aux = aBytes ? da : nullptr;
+        dm.t = tBytes ? dt : nullptr; dm.y = yBytes ? dy : nullptr; dm.aux = aBytes ? da : nullptr; dm.w = wBytes ? dw : nullptr;
         if (rc == MIR_B200_OK) rc = batched_dev<T>(settings, &dm, batch, m, n, dx, dl, du, bound_stride, dr, stats ? ds : nullptr, cs, ready, spinLimit);
     };
     if (staged) {

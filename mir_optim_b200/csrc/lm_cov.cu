@@ -6,6 +6,9 @@
 
 namespace mirb200 {
 
+extern template int launch_cov_builtin<double, true>(const mir_model_desc&, double, CovArgs, const char*, cudaStream_t);
+extern template int launch_cov_builtin<float, true>(const mir_model_desc&, float, CovArgs, const char*, cudaStream_t);
+
 int check_model_data(const mir_model_desc* model, size_t batch, size_t m);   // lm_batched.cu
 
 namespace {
@@ -63,6 +66,7 @@ int covariance_dev(const typename Num<T>::Settings* settings, const mir_model_de
     ca.cov = cov; ca.stddev = stddev; ca.info = info; ca.counter = counter; ca.scratch = nullptr; ca.scratch_stride = 0;
     ca.batch = batch; ca.m = (unsigned)m; ca.n = (unsigned)n; ca.bound_stride = (unsigned)bound_stride;
     ca.flags = model->flags; ca.unscaled = (covFlags & MIR_COV_UNSCALED) ? 1u : 0u;
+    ca.w = (model->flags & MIR_MODEL_WEIGHTED) ? model->w : nullptr;
     const int rc = launch_cov_model<T>(*model, settings->jacobianEpsilon, ca, stream);
     cudaFreeAsync(counter, stream);
     return rc;
@@ -82,6 +86,7 @@ int covariance_host(const typename Num<T>::Settings* settings, const mir_model_d
     const bool per = (model->flags & MIR_MODEL_GRID_PER_PROBLEM) != 0;
     const size_t tBytes = model->t ? sizeof(T) * (per ? batch * m : m) : 0;
     const size_t yBytes = model->y ? sizeof(T) * batch * m : 0;
+    const size_t wBytes = (model->flags & MIR_MODEL_WEIGHTED) ? sizeof(T) * batch * m : 0;
     const size_t aBytes = model->aux ? sizeof(T) * ((model->flags & MIR_MODEL_AUX_PER_PROBLEM) ? batch * n : n) : 0;
     const size_t xBytes = sizeof(T) * batch * n;
     const size_t bBytes = sizeof(T) * (bound_stride ? batch * bound_stride : n);
@@ -89,7 +94,7 @@ int covariance_host(const typename Num<T>::Settings* settings, const mir_model_d
     const size_t sBytes = stddev ? sizeof(T) * batch * n : 0;
     const size_t iBytes = sizeof(int32_t) * batch;
     auto align = [](size_t v) { return (v + 255) & ~(size_t)255; };
-    const size_t total = align(tBytes) + align(yBytes) + align(aBytes) + align(xBytes) + 2 * align(bBytes) + align(cBytes) + align(sBytes) + align(iBytes);
+    const size_t total = align(tBytes) + align(yBytes) + align(wBytes) + align(aBytes) + align(xBytes) + 2 * align(bBytes) + align(cBytes) + align(sBytes) + align(iBytes);
 
     cudaStream_t s = nullptr;
     MIRB200_CUDA(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
@@ -101,6 +106,7 @@ int covariance_host(const typename Num<T>::Settings* settings, const mir_model_d
         char* p = base;
         T* dt = (T*)p; p += align(tBytes);
         T* dy = (T*)p; p += align(yBytes);
+        T* dw = (T*)p; p += align(wBytes);
         T* da = (T*)p; p += align(aBytes);
         T* dx = (T*)p; p += align(xBytes);
         T* dl = (T*)p; p += align(bBytes);
@@ -110,12 +116,13 @@ int covariance_host(const typename Num<T>::Settings* settings, const mir_model_d
         int32_t* di = (int32_t*)p;
         if (tBytes) CK(cudaMemcpyAsync(dt, model->t, tBytes, cudaMemcpyHostToDevice, s), "H2D t");
         if (yBytes) CK(cudaMemcpyAsync(dy, model->y, yBytes, cudaMemcpyHostToDevice, s), "H2D y");
+        if (wBytes) CK(cudaMemcpyAsync(dw, model->w, wBytes, cudaMemcpyHostToDevice, s), "H2D w");
         if (aBytes) CK(cudaMemcpyAsync(da, model->aux, aBytes, cudaMemcpyHostToDevice, s), "H2D aux");
         CK(cudaMemcpyAsync(dx, x, xBytes, cudaMemcpyHostToDevice, s), "H2D x");
         CK(cudaMemcpyAsync(dl, l, bBytes, cudaMemcpyHostToDevice, s), "H2D l");
         CK(cudaMemcpyAsync(du, u, bBytes, cudaMemcpyHostToDevice, s), "H2D u");
         mir_model_desc dm = *model;
-        dm.t = tBytes ? dt : nullptr; dm.y = yBytes ? dy : nullptr; dm.aux = aBytes ? da : nullptr;
+        dm.t = tBytes ? dt : nullptr; dm.y = yBytes ? dy : nullptr; dm.aux = aBytes ? da : nullptr; dm.w = wBytes ? dw : nullptr;
         if (rc == MIR_B200_OK)
             rc = covariance_dev<T>(settings, &dm, batch, m, n, dx, dl, du, bound_stride, covFlags, cov ? dc : nullptr, stddev ? ds : nullptr, di, s);
         if (rc == MIR_B200_OK) {
@@ -137,12 +144,8 @@ template <class T>
 int launch_cov_model(const mir_model_desc& model, T jacEps, CovArgs ca, cudaStream_t stream)
 {
     if (model.model >= (uint32_t)MIR_MODEL_USER_BASE) return launch_user_cov<T>(model, jacEps, ca, stream);
-    return visit_cta_model<T>(model, kNoCovModel, [&](auto tag) {
-        using M = typename decltype(tag)::type;
-        const bool fd = (model.flags & MIR_MODEL_FD_JACOBIAN) || !M::kAnalytic;
-        const RuntimeKernel kern{fd ? (const void*)lm_cov_cta_kernel<M, T, true> : (const void*)lm_cov_cta_kernel<M, T, false>, "lm_cov_cta_kernel launch"};
-        return launch_cov<T>(kern, jacEps, ca, M::prep_elems((int)ca.n), stream);
-    });
+    if (model.flags & MIR_MODEL_WEIGHTED) return launch_cov_builtin<T, true>(model, jacEps, ca, kNoCovModel, stream);
+    return launch_cov_builtin<T, false>(model, jacEps, ca, kNoCovModel, stream);
 }
 template int launch_cov_model<double>(const mir_model_desc&, double, CovArgs, cudaStream_t);
 template int launch_cov_model<float>(const mir_model_desc&, float, CovArgs, cudaStream_t);

@@ -44,6 +44,7 @@ template <class T> struct CtaProblem {
     const T* y;      // observations of this problem (m values) or null
     const T* aux;    // model constants of this problem (n values) or null
     T param;
+    const T* w;      // observation weights of this problem (m values) with MIR_MODEL_WEIGHTED, else null
 };
 
 struct CtaBatchArgs {
@@ -54,6 +55,7 @@ struct CtaBatchArgs {
     unsigned long long scratch_stride;   // elements per CTA
     unsigned n;
     unsigned stage_m;       // != 0: shared memory holds room for the problem's samples (t, y: 2 * stage_m values) staged by TMA
+    const void* w;          // T[batch*m] observation weights (MIR_MODEL_WEIGHTED) or null
 };
 
 // ---- TMA bulk copy + mbarrier (as in syrk_dmma.cuh) ------------------------------------------------------------------------
@@ -240,12 +242,34 @@ template <class U, class T> struct CtaUser {
     }
 };
 
+// ---- weighted least squares (MIR_MODEL_WEIGHTED): the model M with every row scaled by its weight, r~_i = w_i r_i and
+// J~_ij = w_i J_ij, each rounded once; a finite-difference Jacobian (cta_fd_column) differentiates r~ itself.  The weights
+// are read from global memory (pb.w), where the problem's rows stay in L1/L2.
+template <class M, class T> struct CtaWeighted {
+    static constexpr bool kAnalytic = M::kAnalytic;
+    __host__ __device__ static bool valid(int n, int m) { return M::valid(n, m); }
+    __host__ __device__ static int prep_elems(int n) { return M::prep_elems(n); }
+    __device__ static void prepare(const CtaProblem<T>& pb, const T* p, T* prep) { M::prepare(pb, p, prep); }
+    __device__ static T residual(const CtaProblem<T>& pb, const T* p, const T* prep, int row)
+    {
+        return mul_rn(pb.w[row], M::residual(pb, p, prep, row));
+    }
+    __device__ static void jacobian_row(const CtaProblem<T>& pb, const T* p, const T* prep, int row, T* Jrow)
+    {
+        M::jacobian_row(pb, p, prep, row, Jrow);
+        const T w = pb.w[row];
+        for (int k = 0; k < pb.n; ++k) Jrow[k] = mul_rn(w, Jrow[k]);
+    }
+};
+template <class M> struct CtaIsWeighted { static constexpr bool value = false; };
+template <class M, class T> struct CtaIsWeighted<CtaWeighted<M, T>> { static constexpr bool value = true; };
+
 // ---- pieces shared by lm_cta_kernel and lm_cov_cta_kernel (lm_cov.cuh) ----------------------------------------------------
 // problem `prob` of a batch: t (m or batch*m, MIR_MODEL_GRID_PER_PROBLEM), y (batch*m), aux (n or batch*n,
-// MIR_MODEL_AUX_PER_PROBLEM); null arrays stay null
+// MIR_MODEL_AUX_PER_PROBLEM), w (batch*m, read with MIR_MODEL_WEIGHTED only); null arrays stay null
 template <class T>
 __device__ __forceinline__ CtaProblem<T> cta_problem(const void* t, const void* y, const void* aux, double param, unsigned flags,
-                                                     int m, int n, unsigned long long prob)
+                                                     int m, int n, unsigned long long prob, const void* w)
 {
     CtaProblem<T> pb;
     pb.m = m; pb.n = n;
@@ -253,6 +277,7 @@ __device__ __forceinline__ CtaProblem<T> cta_problem(const void* t, const void* 
     pb.y = y ? static_cast<const T*>(y) + prob * m : nullptr;
     pb.aux = aux ? static_cast<const T*>(aux) + ((flags & MIR_MODEL_AUX_PER_PROBLEM) ? prob * n : 0) : nullptr;
     pb.param = (T)param;
+    pb.w = (w && (flags & MIR_MODEL_WEIGHTED)) ? static_cast<const T*>(w) + prob * m : nullptr;
     return pb;
 }
 
@@ -361,7 +386,7 @@ lm_cta_kernel(const typename Num<T>::Settings st, const CtaBatchArgs ca)
             }
             continue;
         }
-        CtaProblem<T> pb = cta_problem<T>(args.t, args.y, ca.aux, ca.param, args.flags, m, n, prob);
+        CtaProblem<T> pb = cta_problem<T>(args.t, args.y, ca.aux, ca.param, args.flags, m, n, prob, ca.w);
         if (stageM && pb.y != nullptr && (reinterpret_cast<uintptr_t>(pb.y) & 15) == 0 && (pb.t == nullptr || (reinterpret_cast<uintptr_t>(pb.t) & 15) == 0)) {
             const bool perGrid = (args.flags & MIR_MODEL_GRID_PER_PROBLEM) != 0;
             const bool needT = pb.t != nullptr && (perGrid || !tStaged);
@@ -674,6 +699,7 @@ int launch_cta_fit(const K& kern, const typename Num<T>::Settings& st, const Sma
     const bool staged = args.m > 0 && (args.m * sizeof(T)) % 16 == 0 && stage <= 48 * 1024 && smem + stage <= 200 * 1024;
     CtaBatchArgs ca;
     ca.b = args; ca.aux = model.aux; ca.param = model.param; ca.n = (unsigned)n; ca.stage_m = staged ? args.m : 0u;
+    ca.w = (model.flags & MIR_MODEL_WEIGHTED) ? model.w : nullptr;
     ca.scratch_stride = (unsigned long long)args.m * n + (unsigned long long)n * n + 2ull * args.m + 4;
     void* params[] = {(void*)&st, &ca};
     return launch_persistent<T>(kern, staged ? smem + stage : smem, "mir_optim_b200: n too large for the shared memory of the general batched kernel",
@@ -690,6 +716,22 @@ template <class T, class F> int visit_cta_model(const mir_model_desc& model, con
     }
     return visit_large_model<T>(model.model, [&](auto tag) { return f(ModelTag<CtaFromLarge<typename decltype(tag)::type, T>>{}); },
                                 [&] { set_error(unknown); return (int)MIR_B200_EUNSUPPORTED; });
+}
+
+// The built-in models on lm_cta_kernel, as they are (W = false) or behind CtaWeighted (W = true; lm_cta_w_inst.cu)
+template <class T, bool W>
+int launch_cta_builtin(const mir_model_desc& model, size_t n, const typename Num<T>::Settings& st, const SmallBatchArgs& args, cudaStream_t stream)
+{
+    return visit_cta_model<T>(model, "mir_optim_b200: model id not available in the batched path", [&](auto tag) {
+        using M = typename decltype(tag)::type;
+        if (n > 128) { set_error("mir_optim_b200: the batched path supports n <= 128"); return (int)MIR_B200_EUNSUPPORTED; }
+        if (!M::valid((int)n, (int)args.m)) { set_error("mir_optim_b200: (m, n) not valid for this model"); return (int)MIR_B200_EINVAL; }
+        const bool fd = (args.flags & MIR_MODEL_FD_JACOBIAN) || !M::kAnalytic;
+        const void* fn;
+        if constexpr (W) fn = fd ? (const void*)lm_cta_kernel<CtaWeighted<M, T>, T, true> : (const void*)lm_cta_kernel<CtaWeighted<M, T>, T, false>;
+        else fn = fd ? (const void*)lm_cta_kernel<M, T, true> : (const void*)lm_cta_kernel<M, T, false>;
+        return launch_cta_fit<T>(RuntimeKernel{fn, "lm_cta_kernel launch"}, st, args, model, n, M::prep_elems((int)n), stream);
+    });
 }
 
 // general batched path by model id; MIR_B200_EUNSUPPORTED if the model has no run-time-n functor

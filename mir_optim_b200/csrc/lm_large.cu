@@ -440,6 +440,11 @@ static typename Num<T>::Result legacy_entry(const typename Num<T>::Settings* set
         const mir_model_desc* desc = static_cast<const mir_model_desc*>(fContext);
         if (!desc) { set_error("mir_optim_b200: device-model mode needs fContext = mir_model_desc*"); return ret; }
         if (g && (void*)g != Sentinels<T>::g()) { set_error("mir_optim_b200: device-model mode takes g = NULL (finite differences) or mir_b200_device_model_jac_*"); return ret; }
+        // (the flags are masked below: without this check a weighted desc would run unweighted)
+        if (desc->flags & MIR_MODEL_WEIGHTED) {
+            set_error("mir_optim_b200: MIR_MODEL_WEIGHTED is supported by the batched and covariance entry points, not by device-model mode");
+            return ret;
+        }
         mir_model_desc d = *desc;
         d.flags = (d.flags & (uint32_t)MIR_MODEL_NO_TAIL_SHORTCUT) | (g ? 0u : (uint32_t)MIR_MODEL_FD_JACOBIAN);
         // small shapes, fitSpline's residual and models compiled at run time: the batched kernels with a batch of one;
@@ -523,6 +528,7 @@ int mir_optimize_least_squares_sharded_d(const mir_least_squares_settings_d* set
     clear_error();
     if (!settings || !model || !x || !l || !u || !result) { set_error("mir_optim_b200: null argument"); return MIR_B200_EINVAL; }
     if (m_local && (!model->t || !model->y)) { set_error("mir_optim_b200: sharded solve needs device pointers model->t / model->y"); return MIR_B200_EINVAL; }
+    if (model->flags & MIR_MODEL_WEIGHTED) { set_error("mir_optim_b200: the sharded solve does not support MIR_MODEL_WEIGHTED"); return MIR_B200_EUNSUPPORTED; }
     return large_solve<double>(*settings, model->model, model->flags, (long long)m_local, n,
                                (const double*)model->t, (const double*)model->y, nullptr, x, l, u, nccl_comm, (cudaStream_t)cuda_stream,
                                result, stats);

@@ -3,7 +3,9 @@
 // compiles `lm_cta_kernel<CtaUser<UserModel<T>, T>, T, FD>` (the general batched LM kernel, lm_cta.cuh, whose sources
 // are embedded in the library by embed_headers.py) with NVRTC for sm_100a, loads the cubin with the driver API and
 // caches the functions.  The covariance kernel (`lm_cov_cta_kernel`, lm_cov.cuh) is a separate program, compiled at
-// the first covariance call per precision, so registration does no extra work for it.  Both launch with the policy of
+// the first covariance call per precision, so registration does no extra work for it; so are the weighted forms of both
+// (`lm_cta_kernel<CtaWeighted<CtaUser<...>>>`, `lm_cov_cta_weighted_kernel<CtaWeighted<CtaUser<...>>>`, MIR_MODEL_WEIGHTED), compiled
+// at the first weighted call.  All launch with the policy of
 // the built-in kernels (launch_persistent, lm_cta.cuh), through the driver API.  libnvrtc and libcuda are bound with
 // dlopen: the library has no link-time dependency on them.
 #include <dlfcn.h>
@@ -83,14 +85,15 @@ Rtc& rtc()
 }
 
 struct Compiled { void* module = nullptr; void* fn[2] = {nullptr, nullptr}; };   // fn[FD]
-// the two programs compiled per user model: the LM kernel (at registration for double) and the covariance kernel (lazily)
-enum Program { kProgLM = 0, kProgCov = 1 };
+// the programs compiled per user model: the LM kernel (at registration for double), the covariance kernel and the
+// weighted forms of both (lazily)
+enum Program { kProgLM = 0, kProgCov = 1, kProgLMW = 2, kProgCovW = 3, kProgCount = 4 };
 struct UserModelEntry {
     std::string source;
     std::mutex mu;                                  // compilation / loading of THIS model (others are not held up)
-    // key = (device ordinal * 2 + (float ? 1 : 0)) * 2 + program: a module belongs to one context
+    // key = (device ordinal * 2 + (float ? 1 : 0)) * kProgCount + program: a module belongs to one context
     std::map<int, std::unique_ptr<Compiled>> loaded;
-    std::vector<char> cubin[2][2]; std::string names[2][2][2];   // [program][precision], kept for other devices
+    std::vector<char> cubin[kProgCount][2]; std::string names[kProgCount][2][2];   // [program][precision], kept for other devices
 };
 std::mutex g_mu;
 std::map<uint32_t, std::shared_ptr<UserModelEntry>> g_models;
@@ -102,11 +105,14 @@ int compile_source(const std::string& user, bool isFloat, Program which, std::ve
     Rtc& r = rtc();
     if (!r.ok) { set_error("mir_optim_b200: run-time compilation unavailable: " + r.why); return MIR_B200_EUNSUPPORTED; }
     const char* T = isFloat ? "float" : "double";
-    const std::string header = which == kProgLM ? "lm_cta.cuh" : "lm_cov.cuh";
-    const std::string kernel = which == kProgLM ? "mirb200::lm_cta_kernel" : "mirb200::lm_cov_cta_kernel";
+    const bool lm = which == kProgLM || which == kProgLMW, weighted = which == kProgLMW || which == kProgCovW;
+    const std::string header = lm ? "lm_cta.cuh" : "lm_cov.cuh";
+    const std::string kernel = lm ? "mirb200::lm_cta_kernel" : weighted ? "mirb200::lm_cov_cta_weighted_kernel" : "mirb200::lm_cov_cta_kernel";
     std::string src = "#include \"" + header + "\"\n#line 1 \"user_model.cu\"\n" + user + "\n";
-    const std::string e0 = kernel + "<mirb200::CtaUser<UserModel<" + T + ">, " + T + ">, " + T + ", false>";
-    const std::string e1 = kernel + "<mirb200::CtaUser<UserModel<" + T + ">, " + T + ">, " + T + ", true>";
+    std::string model = std::string("mirb200::CtaUser<UserModel<") + T + ">, " + T + ">";
+    if (weighted) model = "mirb200::CtaWeighted<" + model + ", " + T + ">";
+    const std::string e0 = kernel + "<" + model + ", " + T + ", false>";
+    const std::string e1 = kernel + "<" + model + ", " + T + ", true>";
     nvrtcProgram prog = nullptr;
     int rc = r.createProgram(&prog, src.c_str(), "mir_user_model.cu", kEmbeddedCount, kEmbeddedSources, kEmbeddedNames);
     if (rc) { set_error(std::string("mir_optim_b200: nvrtcCreateProgram: ") + (r.getErrorString ? r.getErrorString(rc) : "?")); return MIR_B200_ECUDA; }
@@ -152,7 +158,7 @@ int get_compiled(uint32_t id, bool isFloat, Program prog, Compiled** out)
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) dev = 0;
     std::lock_guard<std::mutex> g(e->mu);
-    std::unique_ptr<Compiled>& c = e->loaded[(dev * 2 + (isFloat ? 1 : 0)) * 2 + prog];
+    std::unique_ptr<Compiled>& c = e->loaded[(dev * 2 + (isFloat ? 1 : 0)) * kProgCount + prog];
     if (!c) {
         const int pi = isFloat ? 1 : 0;
         if (e->cubin[prog][pi].empty()) { const int rc = compile_source(e->source, isFloat, prog, e->cubin[prog][pi], e->names[prog][pi]); if (rc) return rc; }
@@ -190,7 +196,7 @@ int launch_user_model(const mir_model_desc& model, size_t n, const typename Num<
 {
     if (n > 128) { set_error("mir_optim_b200: the batched path supports n <= 128"); return MIR_B200_EUNSUPPORTED; }
     Compiled* c = nullptr;
-    if (int rc = get_compiled(model.model, sizeof(T) == 4, kProgLM, &c)) return rc;
+    if (int rc = get_compiled(model.model, sizeof(T) == 4, (model.flags & MIR_MODEL_WEIGHTED) ? kProgLMW : kProgLM, &c)) return rc;
     void* fn = c->fn[(args.flags & MIR_MODEL_FD_JACOBIAN) ? 1 : 0];      // (a model without jacobian() runs finite differences either way)
     return launch_cta_fit<T>(DriverKernel{fn, "cuLaunchKernel (user model)"}, st, args, model, n, 1, stream);
 }
@@ -201,7 +207,7 @@ template <class T>
 int launch_user_cov(const mir_model_desc& model, T jacEps, CovArgs ca, cudaStream_t stream)
 {
     Compiled* c = nullptr;
-    if (int rc = get_compiled(model.model, sizeof(T) == 4, kProgCov, &c)) return rc;
+    if (int rc = get_compiled(model.model, sizeof(T) == 4, (model.flags & MIR_MODEL_WEIGHTED) ? kProgCovW : kProgCov, &c)) return rc;
     void* fn = c->fn[(model.flags & MIR_MODEL_FD_JACOBIAN) ? 1 : 0];      // (a model without jacobian() runs finite differences either way)
     return launch_cov<T>(DriverKernel{fn, "cuLaunchKernel (user model covariance)"}, jacEps, ca, 1, stream);
 }
@@ -238,7 +244,7 @@ int mir_b200_model_release(uint32_t model_id)
     int cur = 0; cudaGetDevice(&cur);
     for (auto& kv : it->second->loaded) {
         if (!kv.second || !kv.second->module || !rtc().cuModuleUnload) continue;
-        if (cudaSetDevice(kv.first / 4) == cudaSuccess) { cudaDeviceSynchronize(); rtc().cuModuleUnload(kv.second->module); }
+        if (cudaSetDevice(kv.first / (2 * kProgCount)) == cudaSuccess) { cudaDeviceSynchronize(); rtc().cuModuleUnload(kv.second->module); }
     }
     cudaSetDevice(cur);
     g_models.erase(it);

@@ -37,20 +37,22 @@ def _vp(a):
     return C.c_void_p(a.data_ptr())      # torch tensor
 
 
-def _model_desc(model, x, t, y, m, aux, param, fd_jacobian):
+def _model_desc(model, x, t, y, m, aux, param, fd_jacobian, w=None):
     """(m, ModelDesc) of a batched call on x (batch, n): the model id and constants (aux, param), its samples t and y (or m
-    for a model without samples) and the flags they imply.  numpy inputs are converted to x's dtype, and the desc holds
-    the converted arrays; torch tensors are passed as they are."""
+    for a model without samples), the observation weights w (batch, m) if given, and the flags they imply.  numpy inputs
+    are converted to x's dtype, and the desc holds the converted arrays; torch tensors are passed as they are."""
     if isinstance(x, np.ndarray):
-        t, y, aux = (None if a is None else np.ascontiguousarray(a, dtype=x.dtype) for a in (t, y, aux))
+        t, y, aux, w = (None if a is None else np.ascontiguousarray(a, dtype=x.dtype) for a in (t, y, aux, w))
         assert y is None or y.shape[0] == x.shape[0]
     if y is not None and m is None:
         m = y.shape[1]
     assert m is not None, "m is required for models without samples"
+    if w is not None:
+        assert tuple(w.shape) == ((x.shape[0], m) if y is None else tuple(y.shape)), "w must have the shape (batch, m) of y"
     flags = ((MODEL_FD_JACOBIAN if fd_jacobian else 0) | (MODEL_GRID_PER_PROBLEM if t is not None and t.ndim == 2 else 0)
-             | (_abi.MODEL_AUX_PER_PROBLEM if aux is not None and aux.ndim == 2 else 0))
-    desc = ModelDesc(int(model), flags, _vp(t), _vp(y), _vp(aux), float(param))
-    desc.arrays = (t, y, aux)
+             | (_abi.MODEL_AUX_PER_PROBLEM if aux is not None and aux.ndim == 2 else 0) | (_abi.MODEL_WEIGHTED if w is not None else 0))
+    desc = ModelDesc(int(model), flags, _vp(t), _vp(y), _vp(aux), float(param), _vp(w))
+    desc.arrays = (t, y, aux, w)
     return m, desc
 
 
@@ -75,17 +77,19 @@ class Engine(ReferenceAPI):
                          t: np.ndarray | None = None, y: np.ndarray | None = None, m: int | None = None,
                          fd_jacobian: bool = False, want_stats: bool = False, device: int = -1, tail_shortcut: bool = True,
                          results: np.ndarray | None = None, aux: np.ndarray | None = None, param: float = 0.0,
-                         warm_start: bool = False):
+                         warm_start: bool = False, w: np.ndarray | None = None):
         """Solve ``batch`` independent problems; x (batch, n) is updated in place.
         l/u: shape (n,) shared, or (batch, n).  Returns (results structured array, stats dict | None).
-        results: optional preallocated structured array (e.g. a view of pinned memory) to receive the Result PODs."""
+        results: optional preallocated structured array (e.g. a view of pinned memory) to receive the Result PODs.
+        w: optional observation weights (batch, m): row i's residual and Jacobian row are scaled by w_i (1/sigma_i for
+        a chi^2 fit; 0 removes the row)."""
         sfx, real, S, R, *_ = _types(x.dtype)
         assert isinstance(settings, S)
         assert x.ndim == 2 and x.flags.c_contiguous
         batch, n = x.shape
         l = np.ascontiguousarray(l, dtype=x.dtype); u = np.ascontiguousarray(u, dtype=x.dtype)
         bound_stride = 0 if l.ndim == 1 else n
-        m, desc = _model_desc(model, x, t, y, m, aux, param, fd_jacobian)
+        m, desc = _model_desc(model, x, t, y, m, aux, param, fd_jacobian, w)
         desc.flags |= 0 if tail_shortcut else MODEL_NO_TAIL_SHORTCUT
         if warm_start:
             assert results is not None, "warm_start reads results['lambda'] of a previous call"
@@ -103,18 +107,19 @@ class Engine(ReferenceAPI):
     # -- batched LM, device-resident torch tensors ----------------------------------------
     def optimize_batched_device(self, settings, model: ModelId, x, l, u, t=None, y=None, m: int | None = None,
                                 fd_jacobian: bool = False, results=None, stats=None, stream=None, tail_shortcut: bool = True,
-                                aux=None, param: float = 0.0, warm_start: bool = False):
+                                aux=None, param: float = 0.0, warm_start: bool = False, w=None):
         """All tensors are CUDA tensors on the current device; asynchronous on `stream` (default:
         torch's current stream).  `results` : uint8 tensor (batch * sizeof(Result)); `stats`: int64[8] tensor.
         aux: (n,) shared or (batch, n) model constants (the knots of ModelId.SPLINE); param: the model constant;
-        warm_start: results holds a previous call's Result PODs and their lambda is the initial damping."""
+        warm_start: results holds a previous call's Result PODs and their lambda is the initial damping;
+        w: observation weights (batch, m), as in :meth:`optimize_batched`."""
         import torch
         dt = np.dtype({torch.float64: np.float64, torch.float32: np.float32}[x.dtype])
         sfx, real, S, R, *_ = _types(dt)
         assert isinstance(settings, S) and x.is_cuda and x.is_contiguous()
         batch, n = x.shape
         bound_stride = 0 if l.dim() == 1 else n
-        m, desc = _model_desc(model, x, t, y, m, aux, param, fd_jacobian)
+        m, desc = _model_desc(model, x, t, y, m, aux, param, fd_jacobian, w)
         desc.flags |= 0 if tail_shortcut else MODEL_NO_TAIL_SHORTCUT
         if warm_start:
             assert results is not None, "warm_start reads the lambda of a previous call's results"
@@ -133,10 +138,11 @@ class Engine(ReferenceAPI):
     def covariance_batched(self, settings, model: ModelId, x: np.ndarray, l: np.ndarray, u: np.ndarray,
                            t: np.ndarray | None = None, y: np.ndarray | None = None, m: int | None = None,
                            fd_jacobian: bool = False, aux: np.ndarray | None = None, param: float = 0.0,
-                           scaled: bool = True, want_cov: bool = True, device: int = -1):
+                           scaled: bool = True, want_cov: bool = True, device: int = -1, w: np.ndarray | None = None):
         """Covariance and standard errors of the parameters x (batch, n) -- normally a fit's output -- with the model data
-        of :meth:`optimize_batched`.  settings may be None (only jacobianEpsilon is read).  scaled=False: residuals are
-        already divided by sigma (s^2 = 1, scipy's absolute_sigma=True).  Returns (cov (batch, n, n) or None,
+        of :meth:`optimize_batched`, weights w included.  settings may be None (only jacobianEpsilon is read).
+        scaled=False: s^2 = 1; with w = 1/sigma that is scipy's absolute_sigma=True, and scaled=True (s^2 from the weighted
+        residuals over the rows with w != 0) is absolute_sigma=False.  Returns (cov (batch, n, n) or None,
         stddev (batch, n), info int32[batch]); info: 0 OK, k > 0 breakdown at parameter k-1, -1 m <= number of free
         parameters, -2 non-finite values (see mir_b200_covariance_batched_d in the header)."""
         x = np.ascontiguousarray(x)
@@ -146,7 +152,7 @@ class Engine(ReferenceAPI):
         batch, n = x.shape
         l = np.ascontiguousarray(l, dtype=x.dtype); u = np.ascontiguousarray(u, dtype=x.dtype)
         bound_stride = 0 if l.ndim == 1 else n
-        m, desc = _model_desc(model, x, t, y, m, aux, param, fd_jacobian)
+        m, desc = _model_desc(model, x, t, y, m, aux, param, fd_jacobian, w)
         cov = np.empty((batch, n, n), dtype=x.dtype) if want_cov else None
         stddev = np.empty((batch, n), dtype=x.dtype)
         info = np.empty(batch, dtype=np.int32)
@@ -158,7 +164,7 @@ class Engine(ReferenceAPI):
 
     def covariance_batched_device(self, settings, model: ModelId, x, l, u, t=None, y=None, m: int | None = None,
                                   fd_jacobian: bool = False, aux=None, param: float = 0.0, scaled: bool = True,
-                                  want_cov: bool = True, cov=None, stddev=None, info=None, stream=None):
+                                  want_cov: bool = True, cov=None, stddev=None, info=None, stream=None, w=None):
         """:meth:`covariance_batched` on CUDA tensors of the current device, asynchronous on `stream` (default: torch's
         current stream).  cov / stddev / info may be preallocated.  Returns (cov or None, stddev, info) tensors."""
         import torch
@@ -167,7 +173,7 @@ class Engine(ReferenceAPI):
         assert (settings is None or isinstance(settings, S)) and x.is_cuda and x.is_contiguous()
         batch, n = x.shape
         bound_stride = 0 if l.dim() == 1 else n
-        m, desc = _model_desc(model, x, t, y, m, aux, param, fd_jacobian)
+        m, desc = _model_desc(model, x, t, y, m, aux, param, fd_jacobian, w)
         if cov is None and want_cov:
             cov = torch.empty((batch, n, n), dtype=x.dtype, device=x.device)
         if stddev is None:
