@@ -423,6 +423,63 @@ int mir_b200_covariance_batched_dev_s(const mir_least_squares_settings_s* settin
     unsigned cov_flags, float* cov, float* stddev, int32_t* info, void* cuda_stream);
 
 /*
+ * Batched model prediction at new abscissae and its delta-method standard error (lmfit's eval_uncertainty) from a
+ * covariance, normally mir_b200_covariance_batched_*'s output at a fit's x.  The reference has none; this is an
+ * extension.  For problem b, with t*_0 .. t*_{k-1} the evaluation abscissae:
+ *
+ *   Inputs     model->t holds t*: T[k] shared, or T[batch*k] with MIR_MODEL_GRID_PER_PROBLEM.  aux, param,
+ *              MIR_MODEL_AUX_PER_PROBLEM and MIR_MODEL_FD_JACOBIAN mean what they mean in the fit.  model->y and model->w
+ *              are not read, and MIR_MODEL_WEIGHTED, MIR_MODEL_WARM_START and MIR_MODEL_NO_TAIL_SHORTCUT are ignored: a
+ *              prediction is of f, weights describe observations, and the cov passed in already carries the weighting.
+ *   Value      value[b*k+i] = f(t*_i; x_b): the model's residual of row i with y_i = 0, so it has the bits the fit's
+ *              functor computes.  MIR_MODEL_SPLINE is evaluated with m = k + 1 and param = 0: rows 0..k-1 are
+ *              spline(t*_i), and the trailing smoothing row is computed and discarded.  User models see m = k (and
+ *              y = 0), so a user model whose residual depends on `row` or `m` gets what it computes for those.
+ *   Free set   F = { a : l_a < x_a < u_a }, exactly as in the covariance.  Rows and columns of cov outside F are never read.
+ *   Gradient   g_a = d f(t*_i) / d p_a for a in F: the analytic Jacobian row, or the reference's central difference with
+ *              settings->jacobianEpsilon and the bound clamp (LS:1030-1047), as in the covariance.
+ *   Quadratic  q is computed in double, each step an fma, in this order:
+ *   form           q = 0
+ *                  for a in F (ascending):  acc = 0
+ *                                           for c in F (ascending): acc = fma(C(a,c), g_c, acc)
+ *                                           q = fma(g_a, acc, q)
+ *              with C(a,c) = cov[b*n*n + max(a,c)*n + min(a,c)]: only the lower triangle is read, in the layout
+ *              mir_b200_covariance_batched_* writes.  g and C are converted from T to double.
+ *   Output     se[b*k+i] = sqrt(q), rounded once to T; 0 when n_F = 0.  Non-finite inputs propagate through IEEE
+ *              arithmetic.  There is no info array: the caller already holds the covariance's info.
+ *
+ * Usage: a confidence band of the fitted curve is value -/+ t_q * se with t_q a quantile of Student's t with m - n_F
+ * degrees of freedom (as lmfit's eval_uncertainty(sigma=...)); a prediction band for a new observation adds the
+ * caller's observation variance to se^2 first: sqrt(se^2 + sigma_obs^2).
+ *
+ *   x        T[batch*n];  l, u  T[n] shared (bound_stride == 0) or T[batch*bound_stride]
+ *   cov      T[batch*n*n]; must be non-NULL when se is requested, not read otherwise
+ *   value    T[batch*k] or NULL;  se  T[batch*k] or NULL (not both NULL)
+ * settings may be NULL (defaults); only jacobianEpsilon is read.  User models (mir_b200_model_compile) are compiled for
+ * the prediction at their first prediction call per precision.
+ * Returns MIR_B200_EINVAL for a NULL model, x, l or u, value and se both NULL, se without cov, n == 0 or k == 0, a data
+ * model with NULL t, a spline with no knots (aux), bound_stride neither 0 nor >= n, an n the model rejects, or an
+ * unknown user id; MIR_B200_EUNSUPPORTED for n > 128, k >= 2^31 - 1 and for LINEAR2, ROSENBROCK and SQRTCIRCLE.  The
+ * checks run in the covariance's order.  batch == 0 does nothing.  A problem's output bits depend only on its own inputs
+ * (not on the batch size, its position or the run).
+ * Host-pointer form: stages the inputs to `device` (-1 = current), runs, copies value / se back.  Device form: every
+ * pointer (model->t, model->aux, x, l, u, cov, value, se) is a device pointer on the current device; asynchronous on
+ * `cuda_stream`.
+ */
+int mir_b200_predict_batched_d(const mir_least_squares_settings_d* settings, const mir_model_desc* model,
+    size_t batch, size_t k, size_t n, const double* x, const double* l, const double* u, size_t bound_stride,
+    const double* cov, double* value, double* se, int device);
+int mir_b200_predict_batched_s(const mir_least_squares_settings_s* settings, const mir_model_desc* model,
+    size_t batch, size_t k, size_t n, const float* x, const float* l, const float* u, size_t bound_stride,
+    const float* cov, float* value, float* se, int device);
+int mir_b200_predict_batched_dev_d(const mir_least_squares_settings_d* settings, const mir_model_desc* model,
+    size_t batch, size_t k, size_t n, const double* x, const double* l, const double* u, size_t bound_stride,
+    const double* cov, double* value, double* se, void* cuda_stream);
+int mir_b200_predict_batched_dev_s(const mir_least_squares_settings_s* settings, const mir_model_desc* model,
+    size_t batch, size_t k, size_t n, const float* x, const float* l, const float* u, size_t bound_stride,
+    const float* cov, float* value, float* se, void* cuda_stream);
+
+/*
  * fitSpline (fit_splie.d:26-85): least-squares fit of a C2 cubic spline (mir.interpolate.spline with the default
  * SplineConfiguration: not-a-knot ends) with FIXED knots x[n] to `points` data points; the unknowns are the spline
  * values at the knots, bounded by l[n] <= spline(x) <= u[n]; lambda >= 0 weighs the smoothing term

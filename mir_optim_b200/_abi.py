@@ -149,6 +149,8 @@ B200_SYMBOLS = [
     "mir_b200_model_compile", "mir_b200_model_release",
     "mir_b200_covariance_batched_d", "mir_b200_covariance_batched_s",
     "mir_b200_covariance_batched_dev_d", "mir_b200_covariance_batched_dev_s",
+    "mir_b200_predict_batched_d", "mir_b200_predict_batched_s",
+    "mir_b200_predict_batched_dev_d", "mir_b200_predict_batched_dev_s",
 ]
 
 
@@ -197,6 +199,10 @@ def bind_b200_abi(lib):
             fn = getattr(lib, f"mir_b200_covariance_batched{dev}_{sfx}")
             fn.argtypes = [C.POINTER(S), C.POINTER(ModelDesc), C.c_size_t, C.c_size_t, C.c_size_t,
                            vp, vp, vp, C.c_size_t, C.c_uint, vp, vp, vp, vp if dev else C.c_int]
+            fn.restype = C.c_int
+            fn = getattr(lib, f"mir_b200_predict_batched{dev}_{sfx}")
+            fn.argtypes = [C.POINTER(S), C.POINTER(ModelDesc), C.c_size_t, C.c_size_t, C.c_size_t,
+                           vp, vp, vp, C.c_size_t, vp, vp, vp, vp if dev else C.c_int]
             fn.restype = C.c_int
     fn = lib.mir_optimize_least_squares_sharded_d
     fn.argtypes = [C.POINTER(LeastSquaresSettingsD), C.POINTER(ModelDesc), C.c_size_t, C.c_size_t, vp, vp, vp,

@@ -263,6 +263,10 @@ template <class M, class T> struct CtaWeighted {
 };
 template <class M> struct CtaIsWeighted { static constexpr bool value = false; };
 template <class M, class T> struct CtaIsWeighted<CtaWeighted<M, T>> { static constexpr bool value = true; };
+// models whose last residual row is not an observation row: the spline's smoothing row (row m-1).  The prediction kernel
+// (lm_pred.cuh) evaluates such a model at k abscissae with m = k + 1 and discards that row.
+template <class M> struct CtaTrailingRow { static constexpr bool value = false; };
+template <class T> struct CtaTrailingRow<CtaSpline<T>> { static constexpr bool value = true; };
 
 // ---- pieces shared by lm_cta_kernel and lm_cov_cta_kernel (lm_cov.cuh) ----------------------------------------------------
 // problem `prob` of a batch: t (m or batch*m, MIR_MODEL_GRID_PER_PROBLEM), y (batch*m), aux (n or batch*n,

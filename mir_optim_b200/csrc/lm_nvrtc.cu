@@ -5,7 +5,8 @@
 // caches the functions.  The covariance kernel (`lm_cov_cta_kernel`, lm_cov.cuh) is a separate program, compiled at
 // the first covariance call per precision, so registration does no extra work for it; so are the weighted forms of both
 // (`lm_cta_kernel<CtaWeighted<CtaUser<...>>>`, `lm_cov_cta_weighted_kernel<CtaWeighted<CtaUser<...>>>`, MIR_MODEL_WEIGHTED), compiled
-// at the first weighted call.  All launch with the policy of
+// at the first weighted call, and the prediction kernel (`lm_pred_cta_kernel`, lm_pred.cuh), compiled at the first
+// prediction call.  All launch with the policy of
 // the built-in kernels (launch_persistent, lm_cta.cuh), through the driver API.  libnvrtc and libcuda are bound with
 // dlopen: the library has no link-time dependency on them.
 #include <dlfcn.h>
@@ -18,6 +19,7 @@
 #include <vector>
 
 #include "lm_cov.cuh"
+#include "lm_pred.cuh"
 #include "runtime.cuh"
 
 namespace mirb200 {
@@ -85,9 +87,9 @@ Rtc& rtc()
 }
 
 struct Compiled { void* module = nullptr; void* fn[2] = {nullptr, nullptr}; };   // fn[FD]
-// the programs compiled per user model: the LM kernel (at registration for double), the covariance kernel and the
-// weighted forms of both (lazily)
-enum Program { kProgLM = 0, kProgCov = 1, kProgLMW = 2, kProgCovW = 3, kProgCount = 4 };
+// the programs compiled per user model: the LM kernel (at registration for double), the covariance kernel, the
+// weighted forms of both and the prediction kernel (lazily)
+enum Program { kProgLM = 0, kProgCov = 1, kProgLMW = 2, kProgCovW = 3, kProgPred = 4, kProgCount = 5 };
 struct UserModelEntry {
     std::string source;
     std::mutex mu;                                  // compilation / loading of THIS model (others are not held up)
@@ -106,8 +108,10 @@ int compile_source(const std::string& user, bool isFloat, Program which, std::ve
     if (!r.ok) { set_error("mir_optim_b200: run-time compilation unavailable: " + r.why); return MIR_B200_EUNSUPPORTED; }
     const char* T = isFloat ? "float" : "double";
     const bool lm = which == kProgLM || which == kProgLMW, weighted = which == kProgLMW || which == kProgCovW;
-    const std::string header = lm ? "lm_cta.cuh" : "lm_cov.cuh";
-    const std::string kernel = lm ? "mirb200::lm_cta_kernel" : weighted ? "mirb200::lm_cov_cta_weighted_kernel" : "mirb200::lm_cov_cta_kernel";
+    const bool pred = which == kProgPred;
+    const std::string header = lm ? "lm_cta.cuh" : pred ? "lm_pred.cuh" : "lm_cov.cuh";
+    const std::string kernel = lm ? "mirb200::lm_cta_kernel" : pred ? "mirb200::lm_pred_cta_kernel"
+                             : weighted ? "mirb200::lm_cov_cta_weighted_kernel" : "mirb200::lm_cov_cta_kernel";
     std::string src = "#include \"" + header + "\"\n#line 1 \"user_model.cu\"\n" + user + "\n";
     std::string model = std::string("mirb200::CtaUser<UserModel<") + T + ">, " + T + ">";
     if (weighted) model = "mirb200::CtaWeighted<" + model + ", " + T + ">";
@@ -213,6 +217,17 @@ int launch_user_cov(const mir_model_desc& model, T jacEps, CovArgs ca, cudaStrea
 }
 template int launch_user_cov<double>(const mir_model_desc&, double, CovArgs, cudaStream_t);
 template int launch_user_cov<float>(const mir_model_desc&, float, CovArgs, cudaStream_t);
+
+template <class T>
+int launch_user_pred(const mir_model_desc& model, T jacEps, PredArgs pa, cudaStream_t stream)
+{
+    Compiled* c = nullptr;
+    if (int rc = get_compiled(model.model, sizeof(T) == 4, kProgPred, &c)) return rc;
+    void* fn = c->fn[(model.flags & MIR_MODEL_FD_JACOBIAN) ? 1 : 0];      // (a model without jacobian() runs finite differences either way)
+    return launch_pred<T>(DriverKernel{fn, "cuLaunchKernel (user model prediction)"}, jacEps, pa, 1, stream);
+}
+template int launch_user_pred<double>(const mir_model_desc&, double, PredArgs, cudaStream_t);
+template int launch_user_pred<float>(const mir_model_desc&, float, PredArgs, cudaStream_t);
 
 }  // namespace mirb200
 

@@ -188,6 +188,63 @@ class Engine(ReferenceAPI):
         self._check(rc)
         return cov, stddev, info
 
+    # -- model prediction and its standard error at new abscissae ---------------------------------
+    def predict_batched(self, settings, model: ModelId, x: np.ndarray, l: np.ndarray, u: np.ndarray,
+                        t: np.ndarray | None = None, k: int | None = None, cov: np.ndarray | None = None,
+                        fd_jacobian: bool = False, aux: np.ndarray | None = None, param: float = 0.0,
+                        want_value: bool = True, device: int = -1):
+        """The model at the parameters x (batch, n) -- normally a fit's output -- evaluated at the abscissae t ((k,) shared
+        or (batch, k)), and with cov (batch, n, n) -- normally covariance_batched's output -- the delta-method standard
+        error se = sqrt(g^T C g) of each value, g = df/dp on the free parameters (lmfit's eval_uncertainty).  k is needed
+        only for a model without abscissae.  settings may be None (only jacobianEpsilon is read).  Returns
+        (value (batch, k) or None, se (batch, k) or None); see mir_b200_predict_batched_d in the header."""
+        x = np.ascontiguousarray(x)
+        sfx, real, S, R, *_ = _types(x.dtype)
+        assert settings is None or isinstance(settings, S)
+        assert x.ndim == 2
+        batch, n = x.shape
+        l = np.ascontiguousarray(l, dtype=x.dtype); u = np.ascontiguousarray(u, dtype=x.dtype)
+        bound_stride = 0 if l.ndim == 1 else n
+        if t is not None and k is None:
+            k = np.shape(t)[-1]
+        k, desc = _model_desc(model, x, t, None, k, aux, param, fd_jacobian)
+        if cov is not None:
+            cov = np.ascontiguousarray(cov, dtype=x.dtype)
+            assert cov.shape == (batch, n, n)
+        value = np.empty((batch, k), dtype=x.dtype) if want_value else None
+        se = np.empty((batch, k), dtype=x.dtype) if cov is not None else None
+        fn = getattr(self.lib, f"mir_b200_predict_batched_{sfx}")
+        rc = fn(C.byref(settings) if settings is not None else None, C.byref(desc), batch, k, n, _vp(x), _vp(l), _vp(u),
+                bound_stride, _vp(cov), _vp(value), _vp(se), device)
+        self._check(rc)
+        return value, se
+
+    def predict_batched_device(self, settings, model: ModelId, x, l, u, t=None, k: int | None = None, cov=None,
+                               fd_jacobian: bool = False, aux=None, param: float = 0.0, want_value: bool = True,
+                               value=None, se=None, stream=None):
+        """:meth:`predict_batched` on CUDA tensors of the current device, asynchronous on `stream` (default: torch's
+        current stream).  value / se (batch, k) may be preallocated.  Returns (value or None, se or None) tensors."""
+        import torch
+        dt = np.dtype({torch.float64: np.float64, torch.float32: np.float32}[x.dtype])
+        sfx, real, S, R, *_ = _types(dt)
+        assert (settings is None or isinstance(settings, S)) and x.is_cuda and x.is_contiguous()
+        batch, n = x.shape
+        bound_stride = 0 if l.dim() == 1 else n
+        if t is not None and k is None:
+            k = t.shape[-1]
+        k, desc = _model_desc(model, x, t, None, k, aux, param, fd_jacobian)
+        if value is None and want_value:
+            value = torch.empty((batch, k), dtype=x.dtype, device=x.device)
+        if se is None and cov is not None:
+            se = torch.empty((batch, k), dtype=x.dtype, device=x.device)
+        if stream is None:
+            stream = torch.cuda.current_stream(x.device).cuda_stream
+        fn = getattr(self.lib, f"mir_b200_predict_batched_dev_{sfx}")
+        rc = fn(C.byref(settings) if settings is not None else None, C.byref(desc), batch, k, n, _vp(x), _vp(l), _vp(u),
+                bound_stride, _vp(cov), _vp(value), _vp(se), C.c_void_p(stream))
+        self._check(rc)
+        return value, se
+
     # -- user-defined device models (NVRTC) ---------------------------------------------------
     def compile_model(self, cuda_source: str) -> int:
         """Registers a residual model written in CUDA C++ (``template <class REAL> struct UserModel {...}``, see
