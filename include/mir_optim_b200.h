@@ -255,8 +255,12 @@ enum {
                                          damping instead of 0 (LS:966); the reference documents Result.lambda as
                                          the initial trust-region value (LS:141-142) but never reads it back.
                                          Chain it with the x of a previous call to continue a fit.            */
-    MIR_MODEL_WEIGHTED         = 32u  /* per-observation weights in model->w (an extension; the reference has none):
+    MIR_MODEL_WEIGHTED         = 32u, /* per-observation weights in model->w (an extension; the reference has none):
                                          every row's residual and Jacobian row are scaled by w_i, see mir_model_desc */
+    MIR_MODEL_LOSS_SOFT_L1     = 64u, /* robust loss rho(z) = 2 (sqrt(1 + z) - 1) (scipy's least_squares(loss=
+                                         'soft_l1')); an extension, see "Robust losses" below                     */
+    MIR_MODEL_LOSS_HUBER       = 128u /* robust loss rho(z) = z (z <= 1), 2 sqrt(z) - 1 (z > 1) (loss='huber');
+                                         at most one of the two loss flags                                       */
 };
 
 typedef struct mir_model_desc {
@@ -284,6 +288,41 @@ typedef struct mir_model_desc {
  * (with any of the other flags); weighted fits always run the general batched kernel (lm_cta.cuh).  MIR_B200_EINVAL
  * for w == NULL (batch > 0, m > 0); MIR_B200_EUNSUPPORTED for the data-free models LINEAR2, ROSENBROCK and SQRTCIRCLE
  * and from mir_optimize_least_squares_sharded_d.  The legacy entry points in device-model mode return numericError.
+ */
+
+/*
+ * Robust losses (MIR_MODEL_LOSS_SOFT_L1, MIR_MODEL_LOSS_HUBER; an extension, the reference has none).  Outlier-resistant
+ * fitting as scipy's least_squares(loss=...), minimising sum_i rho(u_i^2) with u_i = w_i r_i (MIR_MODEL_WEIGHTED) or
+ * u_i = r_i.  There is no separate scale: the weights are the scale, so least_squares(loss=L, f_scale=C) is w_i = 1/C and
+ * curve_fit(sigma=s, loss=L) is w = 1/s; each problem (each row) can have its own.  With z = u^2:
+ *     soft_l1   rho(z) = 2 (sqrt(1 + z) - 1)
+ *     huber     rho(z) = z for z <= 1, 2 sqrt(z) - 1 otherwise
+ * The solver sees the square-root form, row by row: the residual f~_i = sign(u_i) sqrt(rho(u_i^2)), so sum f~_i^2 =
+ * sum rho(u_i^2), and the Jacobian row J~_i = g(u_i) (w_i J_i) with g = d f~ / du = rho'(u^2) |u| / sqrt(rho(u^2)).  A
+ * finite-difference Jacobian is the reference's central difference (LS:1016-1050, with the bound clamp) taken of f~.
+ * Everything downstream is the reference run with f = f~:
+ *   Result.residual = sum rho(u_i^2): 2 * scipy's cost with f_scale = 1, and 2 cost / C^2 with w = 1/C in place of
+ *                     f_scale = C; maxGoodResidual is compared with that sum.
+ *   g-test            J~^T f~ = sum rho'(u^2) u grad(u), the gradient of sum rho / 2.
+ *   solutions         the stationary points of scipy's robust objective.  The iterates differ from scipy's (which runs TRF
+ *                     with a Triggs-corrected Jacobian), so compare at the solution.
+ * Each operation below is rounded once in T (no contraction), with a = |u|, and f~ = -F for u < 0, else F:
+ *   huber,   a <= 1:  f~ = u, g = 1 (the row is bit for bit the squared-loss row)
+ *   huber,   a > 1:   v = a - 0.5;  F = 2 * sqrt(0.5 * v);  g = 1 / F
+ *   soft_l1, a <= 1:  s = sqrt(1 + a * a);  r = sqrt(0.5 * (s + 1));  F = a / r (f~ = u / r);  g = r / s
+ *   soft_l1, a > 1:   q = 1 / a;  c = sqrt(1 + q * q);  r = sqrt(0.5 * (c + q));  b = sqrt(a);  F = b / r;  g = r / (b * c)
+ *   J~_ij = g * (w_i * J_ij) (w_i = 1 without MIR_MODEL_WEIGHTED)
+ * The a > 1 forms never square u and never divide into the subnormals (q only meets 1 and c), so for every finite u, in
+ * both precisions, f~ and g are finite and within 4 ulp of their exact values (the naive u sqrt(2 / (s + 1)) gives f~ = 0
+ * for a float |u| > 1.8e19, and such a trial point would be accepted).  A NaN or infinite u gives a NaN or infinite f~,
+ * which the reference's non-finite handling (LS:1117-1122) treats as for any residual.  f~^2 ~ 2|u| overflows in T only
+ * for |u| near the largest finite value.
+ * Honoured by mir_optimize_least_squares_batched_{d,s} / _dev_{d,s} with any of the other flags; robust fits always run
+ * the general batched kernel (lm_cta.cuh).  MIR_B200_EINVAL for both loss flags at once; MIR_B200_EUNSUPPORTED for
+ * LINEAR2, ROSENBROCK and SQRTCIRCLE, from mir_b200_covariance_batched_* (a covariance of a robust fit is not defined
+ * here: the squared-loss covariance at a robust solution would mislead) and from mir_optimize_least_squares_sharded_d.
+ * The legacy entry points in device-model mode return numericError.  mir_b200_predict_batched_* ignores the flags (a
+ * prediction is of f).  User models compile their robust program at the first robust fit per precision.
  */
 
 /*

@@ -55,6 +55,8 @@ MODEL_NO_TAIL_SHORTCUT = 4
 MODEL_AUX_PER_PROBLEM = 8
 MODEL_WARM_START = 16
 MODEL_WEIGHTED = 32
+MODEL_LOSS_SOFT_L1 = 64
+MODEL_LOSS_HUBER = 128
 COV_UNSCALED = 1
 
 

@@ -38,7 +38,7 @@ static bool specialised_shape(unsigned model, size_t n)
     default: return false;
     }
 }
-// the samples and weights check of the batched fit and of the covariance (lm_cov.cu)
+// the samples, weights and loss check of the batched fit and of the covariance (lm_cov.cu, which refuses the loss flags first)
 int check_model_data(const mir_model_desc* model, size_t batch, size_t m)
 {
     if (batch && m && model_needs_data(model->model) && (!model->t || !model->y)) {
@@ -51,6 +51,15 @@ int check_model_data(const mir_model_desc* model, size_t batch, size_t m)
             return MIR_B200_EUNSUPPORTED;
         }
         if (batch && m && !model->w) { set_error("mir_optim_b200: MIR_MODEL_WEIGHTED: model->w must not be NULL"); return MIR_B200_EINVAL; }
+    }
+    const unsigned loss = model->flags & (MIR_MODEL_LOSS_SOFT_L1 | MIR_MODEL_LOSS_HUBER);
+    if (loss == (MIR_MODEL_LOSS_SOFT_L1 | MIR_MODEL_LOSS_HUBER)) {
+        set_error("mir_optim_b200: MIR_MODEL_LOSS_SOFT_L1 and MIR_MODEL_LOSS_HUBER are mutually exclusive");
+        return MIR_B200_EINVAL;
+    }
+    if (loss && model_data_free(model->model)) {
+        set_error("mir_optim_b200: a robust loss (MIR_MODEL_LOSS_*) needs a model with observation rows (not LINEAR2, ROSENBROCK or SQRTCIRCLE)");
+        return MIR_B200_EUNSUPPORTED;
     }
     return MIR_B200_OK;
 }
@@ -79,8 +88,10 @@ static int batched_dev(const typename Num<T>::Settings* settings, const mir_mode
     a.counter = counter; a.ready = ready; a.spin_limit = spinLimit; a.stats = stats; a.batch = batch; a.m = (unsigned)m;
     a.bound_stride = (unsigned)bound_stride; a.flags = model->flags;
     static const bool forceGeneral = [] { const char* e = std::getenv("MIRB200_BATCH_KERNEL"); return e && !std::strcmp(e, "cta"); }();   // tests / experiments
-    // weights are an adapter of the general kernel's models (CtaWeighted): the specialised kernels never see them
-    if (specialised_shape(model->model, n) && !forceGeneral && !(model->flags & MIR_MODEL_WEIGHTED)) {
+    // weights and robust losses are adapters of the general kernel's models (CtaWeighted, CtaRobust): the specialised
+    // kernels never see them
+    const unsigned adapted = MIR_MODEL_WEIGHTED | MIR_MODEL_LOSS_SOFT_L1 | MIR_MODEL_LOSS_HUBER;
+    if (specialised_shape(model->model, n) && !forceGeneral && !(model->flags & adapted)) {
         rc = launch_small_model<T>(model->model, n, *settings, a, stream);
         // a shape the specialised kernels do not cover after all (m beyond their rows-per-lane instantiations): general kernel
         if (rc == MIR_B200_EUNSUPPORTED && model_needs_data(model->model) && batch > 1) { clear_error(); rc = launch_cta_model<T>(*model, n, *settings, a, stream); }

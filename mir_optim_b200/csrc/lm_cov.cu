@@ -20,6 +20,11 @@ template <class T>
 int cov_check(const mir_model_desc* model, size_t m, size_t n, const void* cov, const void* stddev)
 {
     if (!model) { set_error("mir_optim_b200: null model"); return MIR_B200_EINVAL; }
+    if (model->flags & (MIR_MODEL_LOSS_SOFT_L1 | MIR_MODEL_LOSS_HUBER)) {
+        set_error("mir_optim_b200: the covariance of a robust fit (MIR_MODEL_LOSS_*) is not defined by this library; "
+                  "the squared-loss covariance would not describe a robust solution");
+        return MIR_B200_EUNSUPPORTED;
+    }
     if (!cov && !stddev) { set_error("mir_optim_b200: cov and stddev are both NULL: nothing to compute"); return MIR_B200_EINVAL; }
     if (n == 0 || m == 0) { set_error("mir_optim_b200: m and n must be > 0"); return MIR_B200_EINVAL; }
     if (n > 128) { set_error("mir_optim_b200: the covariance supports n <= 128"); return MIR_B200_EUNSUPPORTED; }

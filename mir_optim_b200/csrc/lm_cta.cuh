@@ -45,6 +45,7 @@ template <class T> struct CtaProblem {
     const T* aux;    // model constants of this problem (n values) or null
     T param;
     const T* w;      // observation weights of this problem (m values) with MIR_MODEL_WEIGHTED, else null
+    unsigned loss;   // MIR_MODEL_LOSS_SOFT_L1 or MIR_MODEL_LOSS_HUBER (read by CtaRobust only), else 0
 };
 
 struct CtaBatchArgs {
@@ -263,6 +264,70 @@ template <class M, class T> struct CtaWeighted {
 };
 template <class M> struct CtaIsWeighted { static constexpr bool value = false; };
 template <class M, class T> struct CtaIsWeighted<CtaWeighted<M, T>> { static constexpr bool value = true; };
+
+// ---- robust losses (MIR_MODEL_LOSS_SOFT_L1 / MIR_MODEL_LOSS_HUBER): the square-root form of rho(u^2) for one row.  Returns
+// f~ = sign(u) sqrt(rho(u^2)) and sets g = d f~ / du, each operation rounded once in T, in exactly the order the header
+// states (a host restatement reproduces the bits).  With a = |u|:
+//   huber,   a <= 1:  f~ = u, g = 1
+//   huber,   a > 1:   v = a - 1/2;  F = 2 sqrt(v / 2) (= sqrt(2a - 1), the scalings exact: no overflow of 2a);  g = 1 / F
+//   soft_l1, a <= 1:  s = sqrt(1 + a a);  r = sqrt((s + 1) / 2);  f~ = u / r;  g = r / s
+//   soft_l1, a > 1:   q = 1 / a;  c = sqrt(1 + q q);  r = sqrt((c + q) / 2);  b = sqrt(a);  F = b / r;  g = r / (b c)
+//                     (s = a c: no u^2 to overflow, and nothing that can go subnormal but q, which only meets 1 and c)
+// and f~ = -F for u < 0, else F.  A NaN or infinite u takes the a > 1 branch and gives a NaN or infinite f~.
+template <class T> __device__ __forceinline__ T cta_robust_loss(unsigned loss, T u, T& g)
+{
+    const T a = t_abs(u);
+    if (a <= (T)1) {
+        if (loss & MIR_MODEL_LOSS_HUBER) { g = (T)1; return u; }
+        const T s = sqrt_ni(add_rn((T)1, mul_rn(a, a)));
+        const T r = sqrt_ni(mul_rn((T)0.5, add_rn(s, (T)1)));
+        g = div_ni(r, s);
+        return div_ni(u, r);
+    }
+    T F;
+    if (loss & MIR_MODEL_LOSS_HUBER) {
+        F = mul_rn((T)2, sqrt_ni(mul_rn((T)0.5, sub_rn(a, (T)0.5))));
+        g = rcp_ni(F);
+    } else {
+        const T q = rcp_ni(a);
+        const T c = sqrt_ni(add_rn((T)1, mul_rn(q, q)));
+        const T r = sqrt_ni(mul_rn((T)0.5, add_rn(c, q)));
+        const T b = sqrt_ni(a);
+        F = div_ni(b, r);
+        g = div_ni(r, mul_rn(b, c));
+    }
+    return (u < (T)0) ? -F : F;
+}
+
+// The model M (with its weights when pb.w is set, exactly as CtaWeighted) under a robust loss: u_i = w_i r_i (or r_i), and
+// the solver sees f~_i = cta_robust_loss(u_i) and J~_ij = g(u_i) (w_i J_ij) (two roundings; g = 1 leaves the row's bits
+// as they are).  sum f~_i^2 = sum rho(u_i^2), and J~^T f~ is the gradient of sum rho / 2.  The Jacobian step re-evaluates
+// the row's residual for u; a finite-difference Jacobian (cta_fd_column) differentiates f~ itself.  The loss is the
+// run-time pb.loss, uniform over a batch, so one instantiation per model serves both losses, weighted or not.
+template <class M, class T> struct CtaRobust {
+    static constexpr bool kAnalytic = M::kAnalytic;
+    __host__ __device__ static bool valid(int n, int m) { return M::valid(n, m); }
+    __host__ __device__ static int prep_elems(int n) { return M::prep_elems(n); }
+    __device__ static void prepare(const CtaProblem<T>& pb, const T* p, T* prep) { M::prepare(pb, p, prep); }
+    __device__ static T scaled(const CtaProblem<T>& pb, const T* p, const T* prep, int row)
+    {
+        const T r = M::residual(pb, p, prep, row);
+        return pb.w ? mul_rn(pb.w[row], r) : r;
+    }
+    __device__ static T residual(const CtaProblem<T>& pb, const T* p, const T* prep, int row)
+    {
+        T g;
+        return cta_robust_loss(pb.loss, scaled(pb, p, prep, row), g);
+    }
+    __device__ static void jacobian_row(const CtaProblem<T>& pb, const T* p, const T* prep, int row, T* Jrow)
+    {
+        T g;
+        cta_robust_loss(pb.loss, scaled(pb, p, prep, row), g);
+        M::jacobian_row(pb, p, prep, row, Jrow);
+        const T w = pb.w ? pb.w[row] : (T)1;
+        for (int k = 0; k < pb.n; ++k) Jrow[k] = mul_rn(g, mul_rn(w, Jrow[k]));
+    }
+};
 // models whose last residual row is not an observation row: the spline's smoothing row (row m-1).  The prediction kernel
 // (lm_pred.cuh) evaluates such a model at k abscissae with m = k + 1 and discards that row.
 template <class M> struct CtaTrailingRow { static constexpr bool value = false; };
@@ -270,7 +335,7 @@ template <class T> struct CtaTrailingRow<CtaSpline<T>> { static constexpr bool v
 
 // ---- pieces shared by lm_cta_kernel and lm_cov_cta_kernel (lm_cov.cuh) ----------------------------------------------------
 // problem `prob` of a batch: t (m or batch*m, MIR_MODEL_GRID_PER_PROBLEM), y (batch*m), aux (n or batch*n,
-// MIR_MODEL_AUX_PER_PROBLEM), w (batch*m, read with MIR_MODEL_WEIGHTED only); null arrays stay null
+// MIR_MODEL_AUX_PER_PROBLEM), w (batch*m, read with MIR_MODEL_WEIGHTED only); null arrays stay null; the loss flags
 template <class T>
 __device__ __forceinline__ CtaProblem<T> cta_problem(const void* t, const void* y, const void* aux, double param, unsigned flags,
                                                      int m, int n, unsigned long long prob, const void* w)
@@ -282,6 +347,7 @@ __device__ __forceinline__ CtaProblem<T> cta_problem(const void* t, const void* 
     pb.aux = aux ? static_cast<const T*>(aux) + ((flags & MIR_MODEL_AUX_PER_PROBLEM) ? prob * n : 0) : nullptr;
     pb.param = (T)param;
     pb.w = (w && (flags & MIR_MODEL_WEIGHTED)) ? static_cast<const T*>(w) + prob * m : nullptr;
+    pb.loss = flags & (MIR_MODEL_LOSS_SOFT_L1 | MIR_MODEL_LOSS_HUBER);
     return pb;
 }
 
@@ -722,8 +788,10 @@ template <class T, class F> int visit_cta_model(const mir_model_desc& model, con
                                 [&] { set_error(unknown); return (int)MIR_B200_EUNSUPPORTED; });
 }
 
-// The built-in models on lm_cta_kernel, as they are (W = false) or behind CtaWeighted (W = true; lm_cta_w_inst.cu)
-template <class T, bool W>
+// The built-in models on lm_cta_kernel: as they are (kCtaPlain), behind CtaWeighted (kCtaWeighted; lm_cta_w_inst.cu) or
+// behind CtaRobust (kCtaRobust, weighted or not; lm_cta_r_inst.cu)
+enum CtaAdapter { kCtaPlain, kCtaWeighted, kCtaRobust };
+template <class T, CtaAdapter A>
 int launch_cta_builtin(const mir_model_desc& model, size_t n, const typename Num<T>::Settings& st, const SmallBatchArgs& args, cudaStream_t stream)
 {
     return visit_cta_model<T>(model, "mir_optim_b200: model id not available in the batched path", [&](auto tag) {
@@ -732,7 +800,8 @@ int launch_cta_builtin(const mir_model_desc& model, size_t n, const typename Num
         if (!M::valid((int)n, (int)args.m)) { set_error("mir_optim_b200: (m, n) not valid for this model"); return (int)MIR_B200_EINVAL; }
         const bool fd = (args.flags & MIR_MODEL_FD_JACOBIAN) || !M::kAnalytic;
         const void* fn;
-        if constexpr (W) fn = fd ? (const void*)lm_cta_kernel<CtaWeighted<M, T>, T, true> : (const void*)lm_cta_kernel<CtaWeighted<M, T>, T, false>;
+        if constexpr (A == kCtaRobust) fn = fd ? (const void*)lm_cta_kernel<CtaRobust<M, T>, T, true> : (const void*)lm_cta_kernel<CtaRobust<M, T>, T, false>;
+        else if constexpr (A == kCtaWeighted) fn = fd ? (const void*)lm_cta_kernel<CtaWeighted<M, T>, T, true> : (const void*)lm_cta_kernel<CtaWeighted<M, T>, T, false>;
         else fn = fd ? (const void*)lm_cta_kernel<M, T, true> : (const void*)lm_cta_kernel<M, T, false>;
         return launch_cta_fit<T>(RuntimeKernel{fn, "lm_cta_kernel launch"}, st, args, model, n, M::prep_elems((int)n), stream);
     });

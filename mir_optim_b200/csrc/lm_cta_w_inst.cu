@@ -5,7 +5,7 @@
 
 namespace mirb200 {
 
-template int launch_cta_builtin<double, true>(const mir_model_desc&, size_t, const Num<double>::Settings&, const SmallBatchArgs&, cudaStream_t);
-template int launch_cta_builtin<float, true>(const mir_model_desc&, size_t, const Num<float>::Settings&, const SmallBatchArgs&, cudaStream_t);
+template int launch_cta_builtin<double, kCtaWeighted>(const mir_model_desc&, size_t, const Num<double>::Settings&, const SmallBatchArgs&, cudaStream_t);
+template int launch_cta_builtin<float, kCtaWeighted>(const mir_model_desc&, size_t, const Num<float>::Settings&, const SmallBatchArgs&, cudaStream_t);
 
 }  // namespace mirb200

@@ -5,8 +5,9 @@
 // caches the functions.  The covariance kernel (`lm_cov_cta_kernel`, lm_cov.cuh) is a separate program, compiled at
 // the first covariance call per precision, so registration does no extra work for it; so are the weighted forms of both
 // (`lm_cta_kernel<CtaWeighted<CtaUser<...>>>`, `lm_cov_cta_weighted_kernel<CtaWeighted<CtaUser<...>>>`, MIR_MODEL_WEIGHTED), compiled
-// at the first weighted call, and the prediction kernel (`lm_pred_cta_kernel`, lm_pred.cuh), compiled at the first
-// prediction call.  All launch with the policy of
+// at the first weighted call, the robust fit (`lm_cta_kernel<CtaRobust<CtaUser<...>>>`, MIR_MODEL_LOSS_*, weighted or
+// not), compiled at the first robust fit, and the prediction kernel (`lm_pred_cta_kernel`, lm_pred.cuh), compiled at the
+// first prediction call.  All launch with the policy of
 // the built-in kernels (launch_persistent, lm_cta.cuh), through the driver API.  libnvrtc and libcuda are bound with
 // dlopen: the library has no link-time dependency on them.
 #include <dlfcn.h>
@@ -88,8 +89,8 @@ Rtc& rtc()
 
 struct Compiled { void* module = nullptr; void* fn[2] = {nullptr, nullptr}; };   // fn[FD]
 // the programs compiled per user model: the LM kernel (at registration for double), the covariance kernel, the
-// weighted forms of both and the prediction kernel (lazily)
-enum Program { kProgLM = 0, kProgCov = 1, kProgLMW = 2, kProgCovW = 3, kProgPred = 4, kProgCount = 5 };
+// weighted forms of both, the prediction kernel and the robust LM kernel (lazily)
+enum Program { kProgLM = 0, kProgCov = 1, kProgLMW = 2, kProgCovW = 3, kProgPred = 4, kProgLMR = 5, kProgCount = 6 };
 struct UserModelEntry {
     std::string source;
     std::mutex mu;                                  // compilation / loading of THIS model (others are not held up)
@@ -107,7 +108,7 @@ int compile_source(const std::string& user, bool isFloat, Program which, std::ve
     Rtc& r = rtc();
     if (!r.ok) { set_error("mir_optim_b200: run-time compilation unavailable: " + r.why); return MIR_B200_EUNSUPPORTED; }
     const char* T = isFloat ? "float" : "double";
-    const bool lm = which == kProgLM || which == kProgLMW, weighted = which == kProgLMW || which == kProgCovW;
+    const bool lm = which == kProgLM || which == kProgLMW || which == kProgLMR, weighted = which == kProgLMW || which == kProgCovW;
     const bool pred = which == kProgPred;
     const std::string header = lm ? "lm_cta.cuh" : pred ? "lm_pred.cuh" : "lm_cov.cuh";
     const std::string kernel = lm ? "mirb200::lm_cta_kernel" : pred ? "mirb200::lm_pred_cta_kernel"
@@ -115,6 +116,7 @@ int compile_source(const std::string& user, bool isFloat, Program which, std::ve
     std::string src = "#include \"" + header + "\"\n#line 1 \"user_model.cu\"\n" + user + "\n";
     std::string model = std::string("mirb200::CtaUser<UserModel<") + T + ">, " + T + ">";
     if (weighted) model = "mirb200::CtaWeighted<" + model + ", " + T + ">";
+    if (which == kProgLMR) model = "mirb200::CtaRobust<" + model + ", " + T + ">";
     const std::string e0 = kernel + "<" + model + ", " + T + ", false>";
     const std::string e1 = kernel + "<" + model + ", " + T + ", true>";
     nvrtcProgram prog = nullptr;
@@ -200,7 +202,9 @@ int launch_user_model(const mir_model_desc& model, size_t n, const typename Num<
 {
     if (n > 128) { set_error("mir_optim_b200: the batched path supports n <= 128"); return MIR_B200_EUNSUPPORTED; }
     Compiled* c = nullptr;
-    if (int rc = get_compiled(model.model, sizeof(T) == 4, (model.flags & MIR_MODEL_WEIGHTED) ? kProgLMW : kProgLM, &c)) return rc;
+    const Program prog = (model.flags & (MIR_MODEL_LOSS_SOFT_L1 | MIR_MODEL_LOSS_HUBER)) ? kProgLMR   // (weights included)
+                       : (model.flags & MIR_MODEL_WEIGHTED) ? kProgLMW : kProgLM;
+    if (int rc = get_compiled(model.model, sizeof(T) == 4, prog, &c)) return rc;
     void* fn = c->fn[(args.flags & MIR_MODEL_FD_JACOBIAN) ? 1 : 0];      // (a model without jacobian() runs finite differences either way)
     return launch_cta_fit<T>(DriverKernel{fn, "cuLaunchKernel (user model)"}, st, args, model, n, 1, stream);
 }

@@ -56,6 +56,16 @@ def _model_desc(model, x, t, y, m, aux, param, fd_jacobian, w=None):
     return m, desc
 
 
+def _loss_flag(loss):
+    """The model flag of a robust loss name (scipy's least_squares names): 0 for "linear" (the squared loss)."""
+    flags = {"linear": 0, "soft_l1": _abi.MODEL_LOSS_SOFT_L1, "huber": _abi.MODEL_LOSS_HUBER}
+    if loss in flags:
+        return flags[loss]
+    if loss in ("cauchy", "arctan"):
+        raise ValueError(f"loss={loss!r} is not supported: the batched fits offer 'linear', 'soft_l1' and 'huber'")
+    raise ValueError(f"unknown loss {loss!r}: expected 'linear', 'soft_l1' or 'huber'")
+
+
 class Engine(ReferenceAPI):
     def __init__(self, lib):
         super().__init__(lib)
@@ -77,12 +87,15 @@ class Engine(ReferenceAPI):
                          t: np.ndarray | None = None, y: np.ndarray | None = None, m: int | None = None,
                          fd_jacobian: bool = False, want_stats: bool = False, device: int = -1, tail_shortcut: bool = True,
                          results: np.ndarray | None = None, aux: np.ndarray | None = None, param: float = 0.0,
-                         warm_start: bool = False, w: np.ndarray | None = None):
+                         warm_start: bool = False, w: np.ndarray | None = None, loss: str = "linear"):
         """Solve ``batch`` independent problems; x (batch, n) is updated in place.
         l/u: shape (n,) shared, or (batch, n).  Returns (results structured array, stats dict | None).
         results: optional preallocated structured array (e.g. a view of pinned memory) to receive the Result PODs.
         w: optional observation weights (batch, m): row i's residual and Jacobian row are scaled by w_i (1/sigma_i for
-        a chi^2 fit; 0 removes the row)."""
+        a chi^2 fit; 0 removes the row).
+        loss: "linear" (squared loss), "soft_l1" or "huber": scipy's robust losses of u = w r, so w = 1/f_scale sets the
+        scale (MIR_MODEL_LOSS_* in the header); results["residual"] is then sum rho(u^2)."""
+        loss_flag = _loss_flag(loss)
         sfx, real, S, R, *_ = _types(x.dtype)
         assert isinstance(settings, S)
         assert x.ndim == 2 and x.flags.c_contiguous
@@ -90,7 +103,7 @@ class Engine(ReferenceAPI):
         l = np.ascontiguousarray(l, dtype=x.dtype); u = np.ascontiguousarray(u, dtype=x.dtype)
         bound_stride = 0 if l.ndim == 1 else n
         m, desc = _model_desc(model, x, t, y, m, aux, param, fd_jacobian, w)
-        desc.flags |= 0 if tail_shortcut else MODEL_NO_TAIL_SHORTCUT
+        desc.flags |= (0 if tail_shortcut else MODEL_NO_TAIL_SHORTCUT) | loss_flag
         if warm_start:
             assert results is not None, "warm_start reads results['lambda'] of a previous call"
             desc.flags |= _abi.MODEL_WARM_START
@@ -107,12 +120,13 @@ class Engine(ReferenceAPI):
     # -- batched LM, device-resident torch tensors ----------------------------------------
     def optimize_batched_device(self, settings, model: ModelId, x, l, u, t=None, y=None, m: int | None = None,
                                 fd_jacobian: bool = False, results=None, stats=None, stream=None, tail_shortcut: bool = True,
-                                aux=None, param: float = 0.0, warm_start: bool = False, w=None):
+                                aux=None, param: float = 0.0, warm_start: bool = False, w=None, loss: str = "linear"):
         """All tensors are CUDA tensors on the current device; asynchronous on `stream` (default:
         torch's current stream).  `results` : uint8 tensor (batch * sizeof(Result)); `stats`: int64[8] tensor.
         aux: (n,) shared or (batch, n) model constants (the knots of ModelId.SPLINE); param: the model constant;
         warm_start: results holds a previous call's Result PODs and their lambda is the initial damping;
-        w: observation weights (batch, m), as in :meth:`optimize_batched`."""
+        w: observation weights (batch, m) and loss: the robust loss, as in :meth:`optimize_batched`."""
+        loss_flag = _loss_flag(loss)
         import torch
         dt = np.dtype({torch.float64: np.float64, torch.float32: np.float32}[x.dtype])
         sfx, real, S, R, *_ = _types(dt)
@@ -120,7 +134,7 @@ class Engine(ReferenceAPI):
         batch, n = x.shape
         bound_stride = 0 if l.dim() == 1 else n
         m, desc = _model_desc(model, x, t, y, m, aux, param, fd_jacobian, w)
-        desc.flags |= 0 if tail_shortcut else MODEL_NO_TAIL_SHORTCUT
+        desc.flags |= (0 if tail_shortcut else MODEL_NO_TAIL_SHORTCUT) | loss_flag
         if warm_start:
             assert results is not None, "warm_start reads the lambda of a previous call's results"
             desc.flags |= _abi.MODEL_WARM_START
